@@ -2,7 +2,7 @@
 """Benchmark of the hot path: matched frame-pairs/s at 1241x376 (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload flow|quad|mono|flow4k]
-                  [--bucket B] [--scaling weak|strong] [--sequences S] [--no-extra]
+                  [--bucket B] [--scaling weak|strong] [--sequences S] [--no-extra] [--dump-outputs DIR]
 
 A step = one new frame for every one of the S independent sequences of this rank (S frame pairs):
 Matcher::pushBack + matchFeatures [+ bucketFeatures + RANSAC/pose for `mono`], results back on the host.
@@ -16,6 +16,7 @@ The rank-0 line also carries the roofline of the fused filter+NMS kernel (timed 
 launch so that the input exceeds L2; primary leg = the configuration of the workload, i.e. Matcher defaults =
 half-resolution mode, second leg = half_resolution 0), the reference CPU path on this box's host cores (`cpu_baseline`),
 and, at N = 1, an `extra` object with short runs of the other configurations of BASELINE.json.
+--dump-outputs DIR writes what the last timed step delivered to the caller (see dump_outputs).
 """
 import argparse
 import ctypes as C
@@ -184,7 +185,24 @@ class Staged:
             self.tctx.host_free(self.pinned_r); self.tctx.device_free(self.dev_r)
 
 
-def timed_run(tctx, st, workload, S, threads, K, Wm, mp, where, local_rank, barrier, sample_clocks):
+def dump_outputs(out_dir, runner, S, mode, prefix):
+    """The results of the last step as a caller of the runner receives them: every sequence's final match list (one row per
+    match, the twelve fields of p_match in their order, as float64: exact for the float32 coordinates and int32 indices) and,
+    for odometry, its 4x4 motion.  Above 64 MB in all, every list keeps the same share of its rows, drawn with a fixed seed."""
+    lists = {'%smatches_seq%03d' % (prefix, s): runner.matches(s) for s in range(S)}
+    arrays = {k: np.stack([m[f] for f in m.dtype.names], 1).astype(np.float64) if len(m) else np.zeros((0, 12))
+              for k, m in lists.items()}
+    if mode == 1:
+        arrays.update({'%smotion_seq%03d' % (prefix, s): np.asarray(runner.motion(s), np.float64) for s in range(S)})
+    share = min(1.0, 64e6 / sum(a.nbytes for a in arrays.values()))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        if share < 1.0 and k.startswith(prefix + 'matches'):
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), int(len(a) * share), replace=False))]
+        np.save(os.path.join(out_dir, k + '.npy'), a)
+
+
+def timed_run(tctx, st, workload, S, threads, K, Wm, mp, where, local_rank, barrier, sample_clocks, dump=None):
     import host_py as Hh
     method = 2 if workload == 'quad' else 0
     mode = 1 if workload == 'mono' else 0
@@ -221,6 +239,8 @@ def timed_run(tctx, st, workload, S, threads, K, Wm, mp, where, local_rank, barr
     l1 = runner.launches(); b1 = runner.transfer_bytes()
     ro = runner.outlier_stats()
     stages = {kk: round(1e3 * v[0] / max(v[1], 1), 4) for kk, v in Hh.stage_times().items() if v[1]}
+    if dump:
+        dump_outputs(dump[0], runner, S, mode, dump[1])
     runner.close()
     return dict(ms=1e3 * secs, event_ms=ev_ms, launches=l1 - l0, h2d=(b1[0] - b0[0]) / K, d2h=(b1[1] - b0[1]) / K,
                 matches_per_pair=int(nm.sum()) / float(S * K), ok_frac=int(ok.sum()) / float(S * K), clocks=clocks, stages=stages, outliers=ro)
@@ -292,7 +312,8 @@ def run_ours(args, rank, world, local_rank):
             import torch.distributed as dist
             dist.barrier()
 
-    res_dev = timed_run(tctx, st, workload, S, threads, K, Wm, mp, 'dev', local_rank, barrier, rank == 0)
+    dump = (args.dump_outputs, 'rank%d_' % rank if world > 1 else '') if args.dump_outputs else None
+    res_dev = timed_run(tctx, st, workload, S, threads, K, Wm, mp, 'dev', local_rank, barrier, rank == 0, dump)
     res_e2e = timed_run(tctx, st, workload, S, threads, K, Wm, mp, 'pinned', local_rank, barrier, False)
     extra = {}
     roof = roof2 = None
@@ -364,6 +385,7 @@ def main():
     ap.add_argument('--no-extra', action='store_true', help='skip the single-Matcher / pageable / other-workload figures')
     ap.add_argument('--no-roofline', action='store_true')
     ap.add_argument('--dry-run', action='store_true', help='no GPU work: fake per-rank timings over gloo (tests of the N>1 plumbing)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the results of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
 

@@ -13,17 +13,11 @@ def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a B200 (run on the GPU box with -m gpu)')
 
 
-@pytest.fixture(scope='session')
-def ref():
-    """The unmodified reference CPU path (oracle/_ref/libvisoref.so) -- the checker, never the product."""
-    import pyref
-    return pyref.RefLib()
-
-
-@pytest.fixture(scope='session')
-def ref_nofma():
-    import pyref
-    return pyref.RefLib('nofma')
+@pytest.fixture
+def reference(request):
+    """Stored outputs of the unmodified reference CPU path for this test (oracle/refgold.py) -- the checker, never the product."""
+    import refgold
+    return refgold.Reference(request.node.path.stem, request.node.name)
 
 
 @pytest.fixture(scope='session')
