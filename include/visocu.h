@@ -193,6 +193,25 @@ int  visocu_ransac_F(visocu_ctx* ctx, int32_t n_jobs, const float* const* uv, co
                      double* F9, uint8_t* const* inlier_mask, int32_t* n_inliers, int32_t* best_iter,
                      int32_t* const* counts, double* const* F_all);
 
+/* ---- stereo odometry: VisualOdometryStereo::estimateMotion (viso_stereo.cpp:42-145) for n_jobs match lists at once ----
+ * matches[j]: N[j] >= 6 p_match records (u1p, v1p, u2p: previous stereo pair; u1c, v1c, u2c, v2c: current).  samples[j]:
+ * p->ransac_iters x 3 indices drawn by the host with the reference's generator (one getRandomSample(N, 3) per iteration).
+ * Per job: one thread per hypothesis runs Gauss-Newton from tr = 0 on the 12 rows of its sample (step 1, eps 1e-6, at most
+ * 22 updates; the 6x6 normal equations solved as Matrix::solve does, a failed solve drops the hypothesis); one thread per
+ * match scores every hypothesis (unweighted squared reprojection error of u1c, v1c, u2c, v2c < inlier_threshold^2); the
+ * earliest hypothesis with the strictly largest count (> 0) wins; one CTA refines on all its inliers (eps 1e-8, at most 102
+ * updates, a fixed reduction tree: a call is bit-identical from run to run).  Out per job: ok[j] (>= 6 inliers and the
+ * refinement converged), tr6 (rx, ry, rz, tx, ty, tz; valid if ok, else 0), inlier_mask (optional, N[j] bytes: the winning
+ * hypothesis' inliers), n_inliers (optional), best_iter (optional, -1 if no hypothesis had an inlier).  Optional, for
+ * parity tests: counts[j] (iters; -1 = that hypothesis' Gauss-Newton failed) and tr_all[j] (iters x 6).  N[j] < 6, a
+ * sample index outside [0, N[j]) or a null input gives VISOCU_EINVAL before anything is written.  One upload, three
+ * launches and one read-back per 128 jobs, on the context's current lane. */
+typedef struct { double f, cu, cv, base, inlier_threshold; int32_t ransac_iters, reweighting; } visocu_stereo_params;
+int  visocu_stereo_motion(visocu_ctx* ctx, int32_t n_jobs, const visocu_pmatch* const* matches, const int32_t* N,
+                          const int32_t* const* samples, const visocu_stereo_params* p, double* tr6, int32_t* ok,
+                          uint8_t* const* inlier_mask, int32_t* n_inliers, int32_t* best_iter,
+                          int32_t* const* counts, double* const* tr_all);
+
 /* ---- pose recovery helpers after RANSAC (SURVEY.md 8f rank 2) ----
  * visocu_triangulate: VisualOdometryMono::triangulateChieral (viso_mono.cpp:394-431) for up to four (R|t) candidates
  * at once.  uv: N x 4 floats (u1p,v1p,u1c,v1c) in pixels; P1: 3x4 projection of the previous camera, P2: n_sol 3x4

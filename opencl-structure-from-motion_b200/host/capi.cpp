@@ -153,16 +153,19 @@ struct StereoParamsC {        // flat mirror of VisualOdometryStereo::parameters
 };
 struct StereoAccess : public VisualOdometryStereo {
   explicit StereoAccess(VisualOdometryStereo::parameters p) : VisualOdometryStereo(p) {}
+  // what process() hands to the quad matching: the previous motion once there is a valid one
+  const Matrix* predictedMotion() const { return Tr_valid ? &Tr_delta : nullptr; }
 };
-}  // namespace
-VISOB_API void* visob_stereo_create(const StereoParamsC* p) {
+VisualOdometryStereo::parameters to_cpp(const StereoParamsC* p) {
   VisualOdometryStereo::parameters q;
   q.match = p->match;
   q.bucket.max_features = p->bucket_max_features; q.bucket.bucket_width = p->bucket_width; q.bucket.bucket_height = p->bucket_height;
   q.calib.f = p->f; q.calib.cu = p->cu; q.calib.cv = p->cv;
   q.base = p->base; q.ransac_iters = p->ransac_iters; q.inlier_threshold = p->inlier_threshold; q.reweighting = p->reweighting != 0;
-  return new StereoAccess(q);
+  return q;
 }
+}  // namespace
+VISOB_API void* visob_stereo_create(const StereoParamsC* p) { return new StereoAccess(to_cpp(p)); }
 VISOB_API void visob_stereo_destroy(void* v) { delete (StereoAccess*)v; }
 VISOB_API int visob_stereo_process(void* v, uint8_t* I1, uint8_t* I2, const int32_t* dims, int replace) {
   uint32_t d[3] = {(uint32_t)dims[0], (uint32_t)dims[1], (uint32_t)dims[2]};
@@ -181,6 +184,20 @@ VISOB_API int visob_stereo_get_inliers(void* v, int32_t* out, int cap) {
   std::vector<int32_t> in = ((StereoAccess*)v)->getInlierIndices();
   if (out) memcpy(out, in.data(), sizeof(int32_t) * (size_t)std::min((int)in.size(), cap));
   return (int)in.size();
+}
+VISOB_API int visob_stereo_get_samples(void* v, int32_t* out, int cap) {
+  const std::vector<int>& s = ((StereoAccess*)v)->lastSamples();
+  if (out) for (int i = 0; i < std::min((int)s.size(), cap); i++) out[i] = s[i];
+  return (int)s.size();
+}
+// the two halves of the batched estimate on a stand-alone object fed with matches (process(matches) split in two)
+VISOB_API int visob_stereo_batch_prepare(void* v, const void* matches, int n) {
+  std::vector<Matcher::p_match> pm((const Matcher::p_match*)matches, (const Matcher::p_match*)matches + n);
+  const visocu_pmatch* m = 0; int32_t N = 0; const int32_t* smp = 0;
+  return ((StereoAccess*)v)->batchPrepare(pm, &m, &N, &smp) ? 1 : 0;
+}
+VISOB_API int visob_stereo_batch_finish(void* v, const double* tr6, int ok, const uint8_t* mask) {
+  return ((StereoAccess*)v)->batchFinish(tr6, ok, mask) ? 1 : 0;
 }
 VISOB_API void visob_matcher_match_features_tr(void* m, int method, const double* tr16) {
   Matrix T(4, 4, tr16);
@@ -251,15 +268,18 @@ VISOB_API void visob_svd(const double* A, int m, int n, double* U, double* W, do
 // Sharded sequence runner.  S independent sequences live on one GPU; sequences are dealt round-robin to `threads` host
 // workers.  Matcher mode: every worker drives its sequences through ONE MatcherBatch (one context, one stream, every GPU
 // stage a single batched launch for all of the worker's sequences) and runs their host stages (outlier removal, priors,
-// bucketing) in between; the workers' streams overlap on the GPU.  Mono-odometry mode: one VisualOdometryMono per
-// sequence (each with its own stream).
+// bucketing) in between; the workers' streams overlap on the GPU.  Odometry modes: one VisualOdometryMono or
+// VisualOdometryStereo per sequence, running on its sequence of the worker's batch; the GPU stages of the motion estimate
+// are one batched call per worker.
 namespace {
 struct Runner {
-  int device, S, threads, mode, method;      // mode 0 = Matcher only, 1 = VisualOdometryMono::process
+  int device, S, threads, mode, method;      // mode 0 = Matcher only, 1 = VisualOdometryMono::process, 2 = VisualOdometryStereo::process
   int bucket_max; float bucket_w, bucket_h;
   MonoParamsC params;
-  std::vector<MatcherBatch*> batches;        // one per worker (mode 0)
+  StereoParamsC sparams;
+  std::vector<MatcherBatch*> batches;        // one per worker
   std::vector<MonoAccess*> monos;            // one per sequence (mode 1)
+  std::vector<StereoAccess*> stereos;        // one per sequence (mode 2)
   std::vector<int32_t> last_matches, last_ok;
   Matcher& matcher_of(int seq) { return batches[seq % threads]->sequence(seq / threads); }
 };
@@ -268,7 +288,36 @@ struct Runner {
 // mode normalisation, sample tables, ONE batched RANSAC call for all of the worker's sequences, pose
 void runner_post(Runner* r, int tid, int bucket, int32_t* n_matches_out, int32_t* ok_out) {
   MatcherBatch* b = r->batches[tid];
-  if (r->mode == 1) {
+  if (r->mode == 2) {
+    // bucketing and sample tables per sequence, then ONE device motion estimate for all of the worker's sequences
+    std::vector<int> ids;
+    std::vector<const visocu_pmatch*> ml;
+    std::vector<int32_t> N;
+    std::vector<const int32_t*> smp;
+    for (int s = tid; s < r->S; s += r->threads) {
+      const visocu_pmatch* m = 0; int32_t n = 0; const int32_t* sp = 0;
+      r->last_ok[s] = 0;
+      if (r->stereos[s]->batchPrepare(&m, &n, &sp)) { ids.push_back(s); ml.push_back(m); N.push_back(n); smp.push_back(sp); }
+      r->last_matches[s] = r->stereos[s]->getNumberOfMatches();
+    }
+    if (!ids.empty()) {
+      const int nj = (int)ids.size();
+      std::vector<double> tr(6 * (size_t)nj);
+      std::vector<int32_t> ok(nj);
+      std::vector<std::vector<uint8_t> > masks(nj);
+      std::vector<uint8_t*> mptr(nj);
+      for (int j = 0; j < nj; j++) { masks[j].resize(N[j]); mptr[j] = masks[j].data(); }
+      const StereoParamsC& q = r->sparams;
+      const visocu_stereo_params sp = {q.f, q.cu, q.cv, q.base, q.inlier_threshold, q.ransac_iters, q.reweighting};
+      visocu_ctx* ctx = b->context();
+      visocu_set_lane(ctx, 4);                     // odometry calls run on their own lane, matching stays on lane 0
+      const int rc = visocu_stereo_motion(ctx, nj, ml.data(), N.data(), smp.data(), &sp, tr.data(), ok.data(), mptr.data(), 0, 0, 0, 0);
+      if (rc != VISOCU_OK) std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
+      visocu_set_lane(ctx, 0);
+      if (rc == VISOCU_OK)
+        for (int j = 0; j < nj; j++) r->last_ok[ids[j]] = r->stereos[ids[j]]->batchFinish(&tr[6 * (size_t)j], ok[j], mptr[j]) ? 1 : 0;
+    }
+  } else if (r->mode == 1) {
     std::vector<int> ids;
     std::vector<const float*> uv;
     std::vector<int32_t> N;
@@ -354,7 +403,13 @@ void runner_advance(Runner* r, int tid, const uint8_t* const* imgs, const uint8_
     if (b->stepSubmit(i1.data(), d, on_device != 0)) b->stepCollect();
   } else {
     runner_push(r, tid, imgs, imgs2, dims, on_device);
-    b->matchFeatures(r->method);
+    if (r->mode == 2) {
+      std::vector<const Matrix*> pred;                 // quad matching with each sequence's motion, as process() does
+      for (int s = tid; s < r->S; s += r->threads) pred.push_back(r->stereos[s]->predictedMotion());
+      b->matchFeatures(r->method, pred.data());
+    } else {
+      b->matchFeatures(r->method);
+    }
   }
   runner_post(r, tid, bucket, n_matches_out, ok_out);
 }
@@ -367,17 +422,26 @@ template <class F> void run_workers(int threads, F work) {
 }
 }  // namespace
 
-VISOB_API void* visob_runner_create(int device, int n_sequences, int threads, int mode, int method, const MonoParamsC* p) {
+namespace {
+Runner* runner_new(int device, int n_sequences, int threads, int mode, int method, const Matcher::parameters& match) {
   Runner* r = new Runner();
   r->device = device; r->S = n_sequences; r->threads = std::max(1, std::min(threads, n_sequences)); r->mode = mode; r->method = method;
-  r->params = *p;
-  r->bucket_max = p->bucket_max_features; r->bucket_w = (float)p->bucket_width; r->bucket_h = (float)p->bucket_height;
   visob::set_device(device);
   for (int t = 0; t < r->threads; t++) {
     int n = 0;
     for (int s = t; s < n_sequences; s += r->threads) n++;
-    r->batches.push_back(new MatcherBatch(p->match, n));
+    r->batches.push_back(new MatcherBatch(match, n));
   }
+  r->last_matches.assign(n_sequences, 0);
+  r->last_ok.assign(n_sequences, 0);
+  return r;
+}
+}  // namespace
+
+VISOB_API void* visob_runner_create(int device, int n_sequences, int threads, int mode, int method, const MonoParamsC* p) {
+  Runner* r = runner_new(device, n_sequences, threads, mode, method, p->match);
+  r->params = *p;
+  r->bucket_max = p->bucket_max_features; r->bucket_w = (float)p->bucket_width; r->bucket_h = (float)p->bucket_height;
   if (mode == 1) {
     // one odometry object per sequence, running on its sequence of the worker's batch
     for (int s = 0; s < n_sequences; s++) {
@@ -386,13 +450,26 @@ VISOB_API void* visob_runner_create(int device, int n_sequences, int threads, in
       r->monos.push_back(vo);
     }
   }
-  r->last_matches.assign(n_sequences, 0);
-  r->last_ok.assign(n_sequences, 0);
+  return r;
+}
+// Stereo odometry (mode 2): one VisualOdometryStereo per sequence.  A step pushes the left and right images of every
+// sequence, runs quad matching with each sequence's previous motion where it has one, and per worker ONE
+// visocu_stereo_motion for the sequences with enough matches; steps are synchronous (imgs2 is required).
+VISOB_API void* visob_runner_create_stereo(int device, int n_sequences, int threads, const StereoParamsC* p) {
+  Runner* r = runner_new(device, n_sequences, threads, 2, 2, p->match);
+  r->sparams = *p;
+  r->bucket_max = p->bucket_max_features; r->bucket_w = (float)p->bucket_width; r->bucket_h = (float)p->bucket_height;
+  for (int s = 0; s < n_sequences; s++) {
+    StereoAccess* vo = new StereoAccess(to_cpp(p));
+    vo->adoptMatcher(&r->batches[s % r->threads]->sequence(s / r->threads));
+    r->stereos.push_back(vo);
+  }
   return r;
 }
 VISOB_API void visob_runner_destroy(void* h) {
   Runner* r = (Runner*)h;
   for (MonoAccess* m : r->monos) delete m;
+  for (StereoAccess* m : r->stereos) delete m;
   for (MatcherBatch* b : r->batches) delete b;
   delete r;
 }
@@ -451,13 +528,22 @@ VISOB_API int visob_runner_get_matches(void* h, int seq, void* out, int cap) {
   Runner* r = (Runner*)h;
   if (seq < 0 || seq >= r->S) return -1;
   if (r->mode == 1) return copy_matches(r->monos[seq]->usedMatches(), out, cap);
+  if (r->mode == 2) return copy_matches(r->stereos[seq]->usedMatches(), out, cap);
   return copy_matches(r->matcher_of(seq).matches(2), out, cap);
 }
 VISOB_API void visob_runner_get_motion(void* h, int seq, double* out16) {
   Runner* r = (Runner*)h;
-  if (r->mode != 1 || seq < 0 || seq >= r->S) return;
-  Matrix T = r->monos[seq]->getMotion();
+  if (r->mode == 0 || seq < 0 || seq >= r->S) return;
+  Matrix T = r->mode == 1 ? r->monos[seq]->getMotion() : r->stereos[seq]->getMotion();
   for (int i = 0; i < 4; i++) for (int j = 0; j < 4; j++) out16[4 * i + j] = T.val[i][j];
+}
+// inlier indices of the last motion estimate (odometry modes); -1 for mode 0 or a bad sequence
+VISOB_API int visob_runner_get_inliers(void* h, int seq, int32_t* out, int cap) {
+  Runner* r = (Runner*)h;
+  if (r->mode == 0 || seq < 0 || seq >= r->S) return -1;
+  std::vector<int32_t> in = r->mode == 1 ? r->monos[seq]->getInlierIndices() : r->stereos[seq]->getInlierIndices();
+  if (out) memcpy(out, in.data(), sizeof(int32_t) * (size_t)std::min((int)in.size(), cap));
+  return (int)in.size();
 }
 VISOB_API void visob_runner_transfer_bytes(void* h, uint64_t* h2d, uint64_t* d2h) {
   Runner* r = (Runner*)h;

@@ -593,7 +593,9 @@ bool MatcherBatch::matchPass(const vector<int32_t>& active, int pass, int32_t me
   vector<visocu_quad> quads(n);
   vector<visocu_pmatch*> outs(n);
   vector<const visocu_range*> rptr(n);
+  vector<const double*> tptr(n, 0);
   vector<int32_t> cap(n), cnt(n), done(n, 0);
+  bool any_tr = false;
   for (size_t k = 0; k < n; k++) {
     Matcher* m = seq[active[k]];
     vector<Matcher::p_match>& out = pass == 0 ? m->p_matched_1 : m->p_matched_2;
@@ -603,9 +605,10 @@ bool MatcherBatch::matchPass(const vector<int32_t>& active, int pass, int32_t me
     outs[k] = reinterpret_cast<visocu_pmatch*>(out.data());
     rptr[k] = reinterpret_cast<const visocu_range*>(m->ranges.data());
     cap[k] = nq + 1;
+    if (m->has_tr && method == 2) { tptr[k] = m->tr_rows; any_tr = true; }
   }
-  const int rc = visocu_match(ctx, (int32_t)n, quads.data(), method, pass, use_prior ? 1 : 0, use_prior ? rptr.data() : 0, 0, refine,
-                              outs.data(), cap.data(), cnt.data(), visob::device_outliers() ? done.data() : 0);
+  const int rc = visocu_match(ctx, (int32_t)n, quads.data(), method, pass, use_prior ? 1 : 0, use_prior ? rptr.data() : 0,
+                              any_tr ? tptr.data() : 0, refine, outs.data(), cap.data(), cnt.data(), visob::device_outliers() ? done.data() : 0);
   if (rc != VISOCU_OK) std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
   for (size_t k = 0; k < n; k++) {
     Matcher* m = seq[active[k]];
@@ -615,9 +618,22 @@ bool MatcherBatch::matchPass(const vector<int32_t>& active, int pass, int32_t me
   return rc == VISOCU_OK;
 }
 
-void MatcherBatch::matchFeatures(int32_t method) {
+void MatcherBatch::matchFeatures(int32_t method, const Matrix* const* tr_delta) {
   if (!ctx) return;
   vector<int32_t> active;
+  // per-sequence motion prediction of quad matching, as Matcher::matchFeatures(2, Tr_delta) does for one sequence; the
+  // sequences share the context and with it the calibration, which is taken from the first sequence that predicts
+  const Matcher* calib = 0;
+  for (size_t s = 0; s < seq.size(); s++) {
+    Matcher* m = seq[s];
+    const Matrix* T = tr_delta ? tr_delta[s] : 0;
+    m->has_tr = T && method == 2 && T->m >= 3 && T->n >= 4;
+    if (!m->has_tr) continue;
+    for (int r = 0; r < 3; r++)
+      for (int c = 0; c < 4; c++) m->tr_rows[4 * r + c] = T->val[r][c];
+    if (!calib) calib = m;
+  }
+  if (calib) visocu_set_intrinsics(ctx, calib->param.f, calib->param.cu, calib->param.cv, calib->param.base);
   const bool fused = Matcher::fusedAvailable(*seq[0], method) && seq.size() <= 128;
   for (size_t s = 0; s < seq.size(); s++) {
     if (!fused) seq[s]->syncCounts();

@@ -139,7 +139,9 @@ public:
   ~MatcherBatch();
   // one image (and optionally one right image) per sequence; dims as for Matcher::pushBack
   void pushBack(const uint8_t* const* I1, const uint8_t* const* I2, uint32_t* dims, bool replace, bool on_device = false);
-  void matchFeatures(int32_t method);
+  // tr_delta (optional, one entry per sequence, null = no prediction): the previous motion of each sequence for the
+  // motion-predicted quad search, as Matcher::matchFeatures(2, Tr_delta).  The sequences share one calibration (setIntrinsics).
+  void matchFeatures(int32_t method, const Matrix* const* tr_delta = nullptr);
   // Pipelined stepping for callers that walk many frames (the sequence runner): stepSubmit pushes one new frame per sequence
   // and enqueues its flow matching against the previous frame - one submission, nothing is waited for -, stepCollect waits
   // for the OLDEST submitted step and puts its matches into the sequences (getMatches, bucketFeatures ... then refer to that

@@ -23,8 +23,9 @@ void VisualOdometry::adoptMatcher(Matcher* external) {
   matcher->seedShuffle(0);     // same state the own matcher had (viso.cpp:35)
 }
 
-bool VisualOdometry::updateMotion() {
-  std::vector<double> tr = estimateMotion(p_matched);
+bool VisualOdometry::updateMotion() { return setMotion(estimateMotion(p_matched)); }
+
+bool VisualOdometry::setMotion(const std::vector<double>& tr) {
   if (tr.size() != 6) return false;
   Tr_delta = transformationVectorToMatrix(tr);
   Tr_valid = true;

@@ -53,6 +53,9 @@ public:
 
 protected:
   bool updateMotion();
+  // the end of updateMotion: a 6-vector (rx, ry, rz, tx, ty, tz) becomes Tr_delta and Tr_valid; any other size is a failed
+  // estimate and leaves both as they are
+  bool setMotion(const std::vector<double>& tr);
   Matrix transformationVectorToMatrix(std::vector<double> tr);
   virtual std::vector<double> estimateMotion(std::vector<Matcher::p_match> p_matched) = 0;
   // num distinct indices out of 0..N-1 by a partial Fisher-Yates shuffle (viso.cpp:86-102).  The reference keeps

@@ -4,6 +4,7 @@
 //   observations ........... viso_stereo.cpp:217-226   residuals and Jacobian ..... viso_stereo.cpp:228-316
 #include "viso_stereo.h"
 
+#include <algorithm>
 #include <cmath>
 
 using std::vector;
@@ -22,9 +23,57 @@ bool VisualOdometryStereo::process(uint8_t* I1, uint8_t* I2, uint32_t* dims, boo
   return updateMotion();
 }
 
+void VisualOdometryStereo::adoptMatcher(Matcher* external) {
+  VisualOdometry::adoptMatcher(external);
+  matcher->setIntrinsics(param.calib.f, param.calib.cu, param.calib.cv, param.base);
+}
+
+// one getRandomSample(N, 3) per RANSAC iteration, whether or not that iteration's fit fails (viso_stereo.cpp:39-40)
+void VisualOdometryStereo::drawSamples(int32_t N) {
+  samples_last.resize((size_t)param.ransac_iters * 3);
+  for (int32_t k = 0; k < param.ransac_iters; k++) {
+    vector<int> s = getRandomSample(N, 3);
+    std::copy(s.begin(), s.end(), samples_last.begin() + (size_t)k * 3);
+  }
+}
+
+bool VisualOdometryStereo::batchPrepare(const visocu_pmatch** matches, int32_t* N, const int32_t** samples) {
+  matcher->bucketFeatures(param.bucket.max_features, param.bucket.bucket_width, param.bucket.bucket_height);
+  p_matched = matcher->getMatches();
+  return prepareEstimate(matches, N, samples);
+}
+
+bool VisualOdometryStereo::batchPrepare(const vector<Matcher::p_match>& p_matched_, const visocu_pmatch** matches, int32_t* N,
+                                        const int32_t** samples) {
+  p_matched = p_matched_;
+  return prepareEstimate(matches, N, samples);
+}
+
+bool VisualOdometryStereo::prepareEstimate(const visocu_pmatch** matches, int32_t* N, const int32_t** samples) {
+  batch_ready = false;
+  if ((int32_t)p_matched.size() < 6) return false;
+  drawSamples((int32_t)p_matched.size());
+  *matches = reinterpret_cast<const visocu_pmatch*>(p_matched.data());
+  *N = (int32_t)p_matched.size();
+  *samples = samples_last.data();
+  batch_ready = true;
+  return true;
+}
+
+// the state estimateMotion + updateMotion leave: the winner's inliers even if the refinement fails, the motion if it converged
+bool VisualOdometryStereo::batchFinish(const double* tr6, int32_t ok, const uint8_t* inlier_mask) {
+  if (!batch_ready) return false;
+  batch_ready = false;
+  inliers.clear();
+  for (size_t i = 0; i < p_matched.size(); i++)
+    if (inlier_mask[i]) inliers.push_back((int32_t)i);
+  return setMotion(ok ? vector<double>(tr6, tr6 + 6) : vector<double>());
+}
+
 vector<double> VisualOdometryStereo::estimateMotion(vector<Matcher::p_match> p_matched) {
   const int32_t N = (int32_t)p_matched.size();
   if (N < 6) return vector<double>();
+  drawSamples(N);
   // previous stereo matches -> 3-D points in the previous left camera frame
   X.resize(N); Y.resize(N); Z.resize(N);
   for (int32_t i = 0; i < N; i++) {
@@ -37,7 +86,7 @@ vector<double> VisualOdometryStereo::estimateMotion(vector<Matcher::p_match> p_m
   inliers.clear();
   // RANSAC over 3-point Gauss-Newton fits
   for (int32_t k = 0; k < param.ransac_iters; k++) {
-    vector<int32_t> active = getRandomSample(N, 3);
+    vector<int32_t> active(samples_last.begin() + (size_t)k * 3, samples_last.begin() + (size_t)k * 3 + 3);
     for (int32_t i = 0; i < 6; i++) tr_curr[i] = 0;
     result res = UPDATED;
     int32_t iter = 0;

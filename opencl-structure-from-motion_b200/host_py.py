@@ -52,7 +52,7 @@ def lib():
         if not os.path.exists(LIB_PATH):
             raise VisocuError(LIB_PATH + ' is missing: run __graft_entry__.build()')
         L = C.CDLL(LIB_PATH)
-        for name in ('visob_matcher_create', 'visob_mono_create', 'visob_mono_matcher', 'visob_runner_create', 'visob_stereo_create', 'visob_recon_create', 'visob_sfm_create',
+        for name in ('visob_matcher_create', 'visob_mono_create', 'visob_mono_matcher', 'visob_runner_create', 'visob_runner_create_stereo', 'visob_stereo_create', 'visob_recon_create', 'visob_sfm_create',
                      'visob_matcher_context'):
             getattr(L, name).restype = C.c_void_p
         L.visob_matcher_gain.restype = C.c_float
@@ -250,6 +250,25 @@ class Stereo:
             lib().visob_stereo_get_inliers(self.h, _p(out), n)
         return out
 
+    def samples(self):
+        """The RANSAC sample table of the last estimate (ransac_iters x 3)."""
+        n = lib().visob_stereo_get_samples(self.h, None, 0)
+        out = np.zeros(n, np.int32)
+        if n:
+            lib().visob_stereo_get_samples(self.h, _p(out), n)
+        return out.reshape(-1, 3)
+
+    def batch_prepare(self, matches):
+        """First half of process_matches for a device estimate: keeps the matches and draws the sample table (samples()).
+        False if there are fewer than 6 matches."""
+        m = np.ascontiguousarray(matches, dtype=P_MATCH)
+        return bool(lib().visob_stereo_batch_prepare(self.h, _p(m), len(m)))
+
+    def batch_finish(self, tr6, ok, mask):
+        """Second half: the results of visocu_stereo_motion for the prepared matches; returns what process_matches returns."""
+        tr6 = np.ascontiguousarray(tr6, np.float64); mask = np.ascontiguousarray(mask, np.uint8)
+        return bool(lib().visob_stereo_batch_finish(self.h, _p(tr6), int(ok), _p(mask)))
+
 
 class Sfm:
     """StructureFromMotion facade (host/sfm.h)."""
@@ -316,12 +335,22 @@ def svd(A):
 
 
 class Runner:
-    """S independent sequences on one GPU driven by `threads` host workers (mode 0: Matcher, 1: mono odometry)."""
+    """S independent sequences on one GPU driven by `threads` host workers (mode 0: Matcher, 1: mono odometry,
+    2: stereo odometry - see Runner.stereo)."""
 
     def __init__(self, device, n_sequences, threads, mode, method, mono_params):
         self.S = n_sequences
         self.mp = mono_params
         self.h = C.c_void_p(lib().visob_runner_create(device, n_sequences, threads, mode, method, C.byref(mono_params)))
+
+    @classmethod
+    def stereo(cls, device, n_sequences, threads, stereo_params):
+        """Stereo odometry runner: one VisualOdometryStereo per sequence; step() / run() take left and right images."""
+        r = cls.__new__(cls)
+        r.S = n_sequences
+        r.mp = stereo_params
+        r.h = C.c_void_p(lib().visob_runner_create_stereo(device, n_sequences, threads, C.byref(stereo_params)))
+        return r
 
     def close(self):
         if getattr(self, 'h', None):
@@ -359,6 +388,14 @@ class Runner:
     def motion(self, seq):
         out = np.zeros((4, 4))
         lib().visob_runner_get_motion(self.h, seq, _p(out))
+        return out
+
+    def inliers(self, seq):
+        """Inlier indices of the sequence's last motion estimate (odometry modes)."""
+        n = lib().visob_runner_get_inliers(self.h, seq, None, 0)
+        out = np.zeros(max(n, 0), np.int32)
+        if n > 0:
+            lib().visob_runner_get_inliers(self.h, seq, _p(out), n)
         return out
 
     def launches(self):

@@ -17,6 +17,12 @@ RANGE = np.dtype([('u_min', 'f4', 4), ('u_max', 'f4', 4), ('v_min', 'f4', 4), ('
 QUAD = np.dtype([('f1p', 'i4'), ('f2p', 'i4'), ('f1c', 'i4'), ('f2c', 'i4')])
 
 
+class StereoMotionParams(C.Structure):
+    """visocu_stereo_params: calibration and RANSAC settings of VisualOdometryStereo::parameters."""
+    _fields_ = [(n, C.c_double) for n in ('f', 'cu', 'cv', 'base', 'inlier_threshold')] + \
+               [('ransac_iters', C.c_int32), ('reweighting', C.c_int32)]
+
+
 class Params(C.Structure):
     """Matcher::parameters (reference matcher.h:42-69): same order, same defaults."""
     _fields_ = [(n, C.c_int32) for n in ('nms_n', 'nms_tau', 'match_binsize', 'match_radius', 'match_disp_tolerance',
@@ -280,3 +286,27 @@ class Context:
                             inliers=np.nonzero(masks[j])[0].astype(np.int32),
                             counts=counts[j] if want_all else None, F_all=Fall[j].reshape(-1, 3, 3) if want_all else None))
         return res
+
+    # ---- stereo odometry
+    def stereo_motion(self, lists, samples, params, want_all=False):
+        """visocu_stereo_motion for a batch of match lists (P_MATCH arrays) and their sample tables (iters x 3).  params: a
+        StereoMotionParams or anything with its fields (host_py.StereoParams).  Returns one dict per job."""
+        nj = len(lists)
+        if not isinstance(params, StereoMotionParams):
+            params = StereoMotionParams(f=params.f, cu=params.cu, cv=params.cv, base=params.base,
+                                        inlier_threshold=params.inlier_threshold, ransac_iters=params.ransac_iters,
+                                        reweighting=int(params.reweighting))
+        ms = [np.ascontiguousarray(m, dtype=P_MATCH) for m in lists]
+        smp = [np.ascontiguousarray(s, np.int32) for s in samples]
+        iters = params.ransac_iters
+        N = np.array([len(m) for m in ms], np.int32)
+        tr = np.zeros((nj, 6)); ok = np.zeros(nj, np.int32); ninl = np.zeros(nj, np.int32); best = np.zeros(nj, np.int32)
+        masks = [np.zeros(len(m), np.uint8) for m in ms]
+        counts = [np.zeros(iters, np.int32) for _ in range(nj)] if want_all else None
+        trall = [np.zeros((iters, 6)) for _ in range(nj)] if want_all else None
+        mk = lambda lst: (C.c_void_p * nj)(*[a.ctypes.data for a in lst]) if lst is not None else None
+        self._ck(lib().visocu_stereo_motion(self.h, nj, mk(ms), _p(N), mk(smp), C.byref(params), _p(tr), _p(ok), mk(masks),
+                                            _p(ninl), _p(best), mk(counts), mk(trall)), 'stereo_motion')
+        return [dict(ok=bool(ok[j]), tr=tr[j].copy(), mask=masks[j], inliers=np.nonzero(masks[j])[0].astype(np.int32),
+                     n_inliers=int(ninl[j]), best_iter=int(best[j]), counts=counts[j] if want_all else None,
+                     tr_all=trall[j] if want_all else None) for j in range(nj)]
