@@ -212,6 +212,34 @@ int  visocu_stereo_motion(visocu_ctx* ctx, int32_t n_jobs, const visocu_pmatch* 
                           uint8_t* const* inlier_mask, int32_t* n_inliers, int32_t* best_iter,
                           int32_t* const* counts, double* const* tr_all);
 
+/* ---- reconstruction: the finished tracks of Reconstruction::update (reconstruction.cpp:50-146), many updates at once ----
+ * One job = the tracks that ended with one update of one Reconstruction (host/reconstruction.h: batchPrepare fills it).
+ * frames: the update's window, oldest first, frames[n_frames - 1] = the newest camera; per frame proj = K * inv[0:3, 0:4],
+ * inv = rows 0..2 of the inverse of fwd (frame -> newest camera), center = fwd[0:3, 3], all row-major.  tracks: obs k was
+ * seen from frame first + k.  cam_road: rows 0..2 of the camera -> road transform of the point types.
+ * Per track, in the host's order and with its semantics: initPoint (null vector of the 4x4 system of the first observation
+ * in frame `first` and the last one in the NEWEST frame, point in float), pointType on that point, refinePoint (Gauss-Newton
+ * over all observations, the point kept in float between updates, the 3x3 normal equations solved as Matrix::solve does,
+ * converged when all three updates are below 1e-5, at most 22 updates), pointDistance to the centre of frame
+ * n_frames - 1 - (n_frames - first) / 2, rayAngle between the first and the newest centre (1000 for a degenerate ray).
+ * status[j][i]: 0 kept, 1 initPoint failed (|w| < 1e-10), 2 point type below point_type, 3 refinePoint failed (c^2 < 1e-10,
+ * singular solve or no convergence), 4 distance >= max_dist, 5 ray angle <= min_angle.  xyz[j][3 i ..]: the point as last
+ * computed - the initial point for status 2, the refined one for 0, 4 and 5, zeros for 1 and 3.  One thread per track in
+ * FP64; the null vector comes from a Jacobi rotation, not the host's SVD, so points agree with the host to rounding.
+ * A null pointer (status[j], xyz[j] and tracks may be null only for a job without tracks), n_frames outside [1, 8],
+ * n_tracks < 0, n_obs outside [2, 6] or first < 0 or first + n_obs > n_frames gives VISOCU_EINVAL before anything is
+ * written.  One upload, one launch and one read-back per call, on the context's current lane; a call whose jobs hold no
+ * tracks launches nothing. */
+typedef struct { double proj[12], inv[12], center[3]; } visocu_recon_frame;
+typedef struct { int32_t first, n_obs; float u[6], v[6]; } visocu_recon_track;
+typedef struct {
+  const visocu_recon_frame* frames; int32_t n_frames;
+  const visocu_recon_track* tracks; int32_t n_tracks;
+  double cam_road[12]; double max_dist, min_angle; int32_t point_type;
+} visocu_recon_job;
+int  visocu_recon_points(visocu_ctx* ctx, int32_t n_jobs, const visocu_recon_job* jobs, int32_t* const* status,
+                         float* const* xyz);
+
 /* ---- pose recovery helpers after RANSAC (SURVEY.md 8f rank 2) ----
  * visocu_triangulate: VisualOdometryMono::triangulateChieral (viso_mono.cpp:394-431) for up to four (R|t) candidates
  * at once.  uv: N x 4 floats (u1p,v1p,u1c,v1c) in pixels; P1: 3x4 projection of the previous camera, P2: n_sol 3x4

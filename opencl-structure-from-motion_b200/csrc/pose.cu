@@ -30,56 +30,16 @@ __global__ void __launch_bounds__(128) k_triangulate(const TriJob* __restrict__ 
     const double* P1 = job.P1;
     const double* P2 = job.P2[sol];
     // J rows (viso_mono.cpp:411-416); g[c][r] = column c of J
-    double g[4][4], v[4][4];
+    double g[4][4];
 #pragma unroll
     for (int c = 0; c < 4; c++) {
       g[c][0] = P1[8 + c] * (double)m.x - P1[c];
       g[c][1] = P1[8 + c] * (double)m.y - P1[4 + c];
       g[c][2] = P2[8 + c] * (double)m.z - P2[c];
       g[c][3] = P2[8 + c] * (double)m.w - P2[4 + c];
-#pragma unroll
-      for (int r = 0; r < 4; r++) v[c][r] = r == c ? 1.0 : 0.0;
     }
-    double total = 0;
-#pragma unroll
-    for (int c = 0; c < 4; c++)
-#pragma unroll
-      for (int k = 0; k < 4; k++) total = fma(g[c][k], g[c][k], total);
-    const double tiny = 1e-28 * total;      // columns this small are numerically null (J has rank 3): leave them alone
-    for (int sweep = 0; sweep < 40; sweep++) {
-      bool rotated = false;
-#pragma unroll
-      for (int p = 0; p < 3; p++)
-#pragma unroll
-        for (int q = p + 1; q < 4; q++) {
-          double alpha = 0, beta = 0, gamma = 0;
-#pragma unroll
-          for (int k = 0; k < 4; k++) { alpha = fma(g[p][k], g[p][k], alpha); beta = fma(g[q][k], g[q][k], beta); gamma = fma(g[p][k], g[q][k], gamma); }
-          if (alpha > tiny && beta > tiny && fabs(gamma) > 1e-15 * sqrt(alpha * beta)) {
-            const double zeta = (beta - alpha) / (2.0 * gamma);
-            const double t = copysign(1.0, zeta) / (fabs(zeta) + sqrt(1.0 + zeta * zeta));
-            const double c = 1.0 / sqrt(1.0 + t * t), s = c * t;
-#pragma unroll
-            for (int k = 0; k < 4; k++) {
-              const double a = g[p][k], b = g[q][k];
-              g[p][k] = c * a - s * b; g[q][k] = s * a + c * b;
-              const double va = v[p][k], vb = v[q][k];
-              v[p][k] = c * va - s * vb; v[q][k] = s * va + c * vb;
-            }
-            rotated = true;
-          }
-        }
-      if (!rotated) break;
-    }
-    double nrm[4];
-#pragma unroll
-    for (int c = 0; c < 4; c++) { nrm[c] = 0; for (int k = 0; k < 4; k++) nrm[c] = fma(g[c][k], g[c][k], nrm[c]); }
-    int js = 0;
-#pragma unroll
-    for (int c = 1; c < 4; c++) if (nrm[c] < nrm[js]) js = c;
     double X[4];
-#pragma unroll
-    for (int r = 0; r < 4; r++) X[r] = js == 0 ? v[0][r] : (js == 1 ? v[1][r] : (js == 2 ? v[2][r] : v[3][r]));
+    jacobi_null_vector4(g, X);
     double* out = job.X + (size_t)sol * 4 * job.N;
 #pragma unroll
     for (int r = 0; r < 4; r++) out[(size_t)r * job.N + i] = X[r];

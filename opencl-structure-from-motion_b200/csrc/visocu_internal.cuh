@@ -169,6 +169,92 @@ int visocu_run_or_replay(visocu_ctx* ctx, visocu_graph& g, uint64_t key, const s
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// Matrix::solve restated (host/matrix.cpp:249-285) for the N x N system A x = b (N <= 8), A and b at stride `s` (element
+// (r, k) of A at A[(N r + k) s]).  The solution replaces b; A is destroyed.  The final column unscrambling of the reference
+// only concerns the inverse left in A, not the solution, and is omitted.  `used` keeps the reference's counters (4 bits per
+// column): with NaN entries no pivot passes the '>=' test and column 0 is chosen again, so a counter can exceed 1.
+template <int N>
+__device__ __forceinline__ bool gj_solve(double* A, double* b, int s, double eps) {
+  unsigned used = 0;
+  for (int step = 0; step < N; step++) {
+    double big = 0;
+    int pr = 0, pc = 0;
+    for (int r = 0; r < N; r++) {
+      if (((used >> (4 * r)) & 15u) == 1u) continue;
+      for (int cc = 0; cc < N; cc++)
+        if (((used >> (4 * cc)) & 15u) == 0u && fabs(A[(N * r + cc) * s]) >= big) { big = fabs(A[(N * r + cc) * s]); pr = r; pc = cc; }
+    }
+    used += 1u << (4 * pc);
+    if (pr != pc) {
+      for (int k = 0; k < N; k++) { const double x = A[(N * pr + k) * s]; A[(N * pr + k) * s] = A[(N * pc + k) * s]; A[(N * pc + k) * s] = x; }
+      const double x = b[pr * s]; b[pr * s] = b[pc * s]; b[pc * s] = x;
+    }
+    if (fabs(A[(N * pc + pc) * s]) < eps) return false;
+    const double piv = 1.0 / A[(N * pc + pc) * s];
+    A[(N * pc + pc) * s] = 1;
+    for (int k = 0; k < N; k++) A[(N * pc + k) * s] *= piv;
+    b[pc * s] *= piv;
+    for (int r = 0; r < N; r++) {
+      if (r == pc) continue;
+      const double f = A[(N * r + pc) * s];
+      A[(N * r + pc) * s] = 0;
+      for (int k = 0; k < N; k++) A[(N * r + k) * s] -= A[(N * pc + k) * s] * f;
+      b[r * s] -= b[pc * s] * f;
+    }
+  }
+  return true;
+}
+
+// Null vector of a 4x4 system of rank 3 (the linear triangulation of two views) by a one-sided Jacobi in registers, in
+// place of Matrix::svd: g[c][r] = column c of the matrix; X receives the right singular vector of the smallest singular
+// value (unit length, sign arbitrary).  g is destroyed.
+__device__ __forceinline__ void jacobi_null_vector4(double (&g)[4][4], double (&X)[4]) {
+  double v[4][4];
+#pragma unroll
+  for (int c = 0; c < 4; c++)
+#pragma unroll
+    for (int r = 0; r < 4; r++) v[c][r] = r == c ? 1.0 : 0.0;
+  double total = 0;
+#pragma unroll
+  for (int c = 0; c < 4; c++)
+#pragma unroll
+    for (int k = 0; k < 4; k++) total = fma(g[c][k], g[c][k], total);
+  const double tiny = 1e-28 * total;      // columns this small are numerically null (J has rank 3): leave them alone
+  for (int sweep = 0; sweep < 40; sweep++) {
+    bool rotated = false;
+#pragma unroll
+    for (int p = 0; p < 3; p++)
+#pragma unroll
+      for (int q = p + 1; q < 4; q++) {
+        double alpha = 0, beta = 0, gamma = 0;
+#pragma unroll
+        for (int k = 0; k < 4; k++) { alpha = fma(g[p][k], g[p][k], alpha); beta = fma(g[q][k], g[q][k], beta); gamma = fma(g[p][k], g[q][k], gamma); }
+        if (alpha > tiny && beta > tiny && fabs(gamma) > 1e-15 * sqrt(alpha * beta)) {
+          const double zeta = (beta - alpha) / (2.0 * gamma);
+          const double t = copysign(1.0, zeta) / (fabs(zeta) + sqrt(1.0 + zeta * zeta));
+          const double c = 1.0 / sqrt(1.0 + t * t), s = c * t;
+#pragma unroll
+          for (int k = 0; k < 4; k++) {
+            const double a = g[p][k], b = g[q][k];
+            g[p][k] = c * a - s * b; g[q][k] = s * a + c * b;
+            const double va = v[p][k], vb = v[q][k];
+            v[p][k] = c * va - s * vb; v[q][k] = s * va + c * vb;
+          }
+          rotated = true;
+        }
+      }
+    if (!rotated) break;
+  }
+  double nrm[4];
+#pragma unroll
+  for (int c = 0; c < 4; c++) { nrm[c] = 0; for (int k = 0; k < 4; k++) nrm[c] = fma(g[c][k], g[c][k], nrm[c]); }
+  int js = 0;
+#pragma unroll
+  for (int c = 1; c < 4; c++) if (nrm[c] < nrm[js]) js = c;
+#pragma unroll
+  for (int r = 0; r < 4; r++) X[r] = js == 0 ? v[0][r] : (js == 1 ? v[1][r] : (js == 2 ? v[2][r] : v[3][r]));
+}
+
 // cells of Matcher::nonMaximumSuppression along one axis: origins n+margin+k(n+1) < len-n-margin (matcher.cpp:344-345)
 __host__ __device__ static inline int viso_cell_count(int len, int n) {
   int s = len - 2 * n - 2 * VISO_MARGIN;

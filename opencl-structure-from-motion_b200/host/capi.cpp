@@ -4,6 +4,8 @@
 #include <atomic>
 #include <chrono>
 #include <cstring>
+#include <iostream>
+#include <memory>
 #include <sstream>
 #include <thread>
 #include <vector>
@@ -219,13 +221,31 @@ VISOB_API int visob_recon_get_points(void* r, float* out3, int cap) {
   for (int i = 0; i < (int)pts.size() && i < cap; i++) { out3[3 * i] = pts[i].x; out3[3 * i + 1] = pts[i].y; out3[3 * i + 2] = pts[i].z; }
   return (int)pts.size();
 }
+// the two halves of Reconstruction::update around the evaluation of its finished tracks (see reconstruction.h); prepare
+// returns the number of tracks to evaluate
+VISOB_API int visob_recon_batch_prepare(void* r, const void* matches, int n, const double* tr16, int point_type, int min_track_length,
+                                        double max_dist, double min_angle) {
+  const Matcher::p_match* m = (const Matcher::p_match*)matches;
+  return ((Reconstruction*)r)->batchPrepare(std::vector<Matcher::p_match>(m, m + n), Matrix(4, 4, tr16), point_type, min_track_length,
+                                            max_dist, min_angle).n_tracks;
+}
+// the prepared job: its scalar fields into *job (frames / tracks pointing into the object), and copies of the frame table
+// and the tracks into `frames` and `tracks` if they are not null
+VISOB_API void visob_recon_batch_job(void* r, visocu_recon_job* job, visocu_recon_frame* frames, visocu_recon_track* tracks) {
+  const visocu_recon_job& j = ((Reconstruction*)r)->batchJob();
+  *job = j;
+  if (frames) memcpy(frames, j.frames, sizeof(visocu_recon_frame) * (size_t)j.n_frames);
+  if (tracks && j.n_tracks) memcpy(tracks, j.tracks, sizeof(visocu_recon_track) * (size_t)j.n_tracks);
+}
+VISOB_API void visob_recon_host_eval(void* r, int32_t* status, float* xyz) { ((Reconstruction*)r)->hostEval(status, xyz); }
+VISOB_API void visob_recon_batch_finish(void* r, const int32_t* status, const float* xyz) { ((Reconstruction*)r)->batchFinish(status, xyz); }
 VISOB_API void* visob_sfm_create(const MonoParamsC* p, const int32_t* dims) {
   StructureFromMotion* s = new StructureFromMotion(to_cpp(p), std::array<uint32_t, 3>{{(uint32_t)dims[0], (uint32_t)dims[1], (uint32_t)dims[2]}}, true);
   s->setVerbose(false);
   return s;
 }
 VISOB_API void visob_sfm_destroy(void* s) { delete (StructureFromMotion*)s; }
-VISOB_API void visob_sfm_update(void* s, uint8_t* img) { ((StructureFromMotion*)s)->update(img); }
+VISOB_API int visob_sfm_update(void* s, uint8_t* img) { return ((StructureFromMotion*)s)->update(img) ? 1 : 0; }
 VISOB_API int visob_sfm_get_points(void* s, float* out3, int cap) {
   const std::vector<Point3d>& pts = ((StructureFromMotion*)s)->getPoints();
   for (int i = 0; i < (int)pts.size() && i < cap; i++) { out3[3 * i] = pts[i].x; out3[3 * i + 1] = pts[i].y; out3[3 * i + 2] = pts[i].z; }
@@ -270,19 +290,67 @@ VISOB_API void visob_svd(const double* A, int m, int n, double* U, double* W, do
 // stage a single batched launch for all of the worker's sequences) and runs their host stages (outlier removal, priors,
 // bucketing) in between; the workers' streams overlap on the GPU.  Odometry modes: one VisualOdometryMono or
 // VisualOdometryStereo per sequence, running on its sequence of the worker's batch; the GPU stages of the motion estimate
-// are one batched call per worker.
+// are one batched call per worker.  Structure-from-motion mode: mono odometry as above, then what StructureFromMotion::update
+// does per sequence, with the finished tracks of all of the worker's sequences evaluated by one device call.
 namespace {
+struct SfmState {                            // what StructureFromMotion keeps besides its odometry object (host/sfm.h)
+  Reconstruction recon;
+  Matrix Tr_total = Matrix::eye(4);
+  bool first = true, replace = false;
+};
 struct Runner {
-  int device, S, threads, mode, method;      // mode 0 = Matcher only, 1 = VisualOdometryMono::process, 2 = VisualOdometryStereo::process
+  int device, S, threads, mode, method;      // mode 0 = Matcher only, 1 = VisualOdometryMono::process, 2 = VisualOdometryStereo::process,
+                                             // 3 = StructureFromMotion::update
   int bucket_max; float bucket_w, bucket_h;
   MonoParamsC params;
   StereoParamsC sparams;
   std::vector<MatcherBatch*> batches;        // one per worker
-  std::vector<MonoAccess*> monos;            // one per sequence (mode 1)
+  std::vector<MonoAccess*> monos;            // one per sequence (modes 1 and 3)
   std::vector<StereoAccess*> stereos;        // one per sequence (mode 2)
+  std::vector<SfmState*> sfms;               // one per sequence (mode 3)
   std::vector<int32_t> last_matches, last_ok;
   Matcher& matcher_of(int seq) { return batches[seq % threads]->sequence(seq / threads); }
 };
+
+// StructureFromMotion::update after the odometry of one frame, for every sequence of worker `tid`: pose accumulation and
+// Reconstruction::batchPrepare for the sequences whose frame is ok, ONE visocu_recon_points for all of them, batchFinish;
+// a failed frame is replaced by the next push.  If the device call fails, the finished tracks of the step are lost and the
+// step reports ok = 0 for those sequences (their pose has already advanced, as the facade's does on a successful frame).
+void runner_sfm(Runner* r, int tid) {
+  std::vector<int> ids;
+  std::vector<visocu_recon_job> jobs;
+  for (int s = tid; s < r->S; s += r->threads) {
+    SfmState& q = *r->sfms[s];
+    MonoAccess& vo = *r->monos[s];
+    if (q.first) { q.first = false; continue; }
+    if (!r->last_ok[s]) { q.replace = true; continue; }
+    q.Tr_total = q.Tr_total * Matrix::inv(vo.getMotion());
+    jobs.push_back(q.recon.batchPrepare(vo.getMatches(), vo.getMotion(), 0, 2, 30, 3));
+    ids.push_back(s);
+    q.replace = false;
+  }
+  if (ids.empty()) return;
+  const int nj = (int)ids.size();
+  std::vector<std::vector<int32_t> > status(nj);
+  std::vector<std::vector<float> > xyz(nj);
+  std::vector<int32_t*> sp(nj);
+  std::vector<float*> xp(nj);
+  for (int j = 0; j < nj; j++) {
+    status[j].resize((size_t)jobs[j].n_tracks); xyz[j].resize(3 * (size_t)jobs[j].n_tracks);
+    sp[j] = status[j].data(); xp[j] = xyz[j].data();
+  }
+  visocu_ctx* ctx = r->batches[tid]->context();
+  visocu_set_lane(ctx, 4);                         // like the odometry calls: matching stays on lane 0
+  const int rc = visocu_recon_points(ctx, nj, jobs.data(), sp.data(), xp.data());
+  visocu_set_lane(ctx, 0);
+  if (rc != VISOCU_OK) {
+    // the finished tracks of this step are lost (batchPrepare has dropped them): the step is reported as failed
+    std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
+    for (int s : ids) r->last_ok[s] = 0;
+    return;
+  }
+  for (int j = 0; j < nj; j++) r->sfms[ids[j]]->recon.batchFinish(sp[j], xp[j]);
+}
 
 // host stages that follow the matching of one frame for every sequence of worker `tid`: bucketing, and for the odometry
 // mode normalisation, sample tables, ONE batched RANSAC call for all of the worker's sequences, pose
@@ -317,7 +385,7 @@ void runner_post(Runner* r, int tid, int bucket, int32_t* n_matches_out, int32_t
       if (rc == VISOCU_OK)
         for (int j = 0; j < nj; j++) r->last_ok[ids[j]] = r->stereos[ids[j]]->batchFinish(&tr[6 * (size_t)j], ok[j], mptr[j]) ? 1 : 0;
     }
-  } else if (r->mode == 1) {
+  } else if (r->mode == 1 || r->mode == 3) {
     std::vector<int> ids;
     std::vector<const float*> uv;
     std::vector<int32_t> N;
@@ -378,6 +446,7 @@ void runner_post(Runner* r, int tid, int bucket, int32_t* n_matches_out, int32_t
       r->last_ok[s] = 1;
     }
   }
+  if (r->mode == 3) runner_sfm(r, tid);
   for (int s = tid; s < r->S; s += r->threads) {
     if (n_matches_out) n_matches_out[s] = r->last_matches[s];
     if (ok_out) ok_out[s] = r->last_ok[s];
@@ -388,14 +457,26 @@ void runner_push(Runner* r, int tid, const uint8_t* const* imgs, const uint8_t* 
   uint32_t d[3] = {(uint32_t)dims[0], (uint32_t)dims[1], (uint32_t)dims[2]};
   std::vector<const uint8_t*> i1, i2;
   for (int s = tid; s < r->S; s += r->threads) { i1.push_back(imgs[s]); if (imgs2) i2.push_back(imgs2[s]); }
+  if (r->mode == 3) {                              // each sequence's replace flag, as StructureFromMotion passes it
+    std::unique_ptr<bool[]> replace(new bool[i1.size()]);
+    size_t k = 0;
+    for (int s = tid; s < r->S; s += r->threads) replace[k++] = r->sfms[s]->replace;
+    r->batches[tid]->pushBack(i1.data(), 0, d, replace.get(), on_device != 0);
+    return;
+  }
   r->batches[tid]->pushBack(i1.data(), imgs2 ? i2.data() : 0, d, false, on_device != 0);
+}
+
+// Steps of mode 3 never take the pipelined path: a step's push needs the previous step's outcome (the replace flag).
+bool runner_pipelined(Runner* r, int tid, const uint8_t* const* imgs2) {
+  return !imgs2 && r->mode != 3 && r->batches[tid]->stepAvailable(r->method);
 }
 
 // one frame for every sequence of worker `tid`, synchronously
 void runner_advance(Runner* r, int tid, const uint8_t* const* imgs, const uint8_t* const* imgs2, const int32_t* dims, int on_device,
                     int bucket, int32_t* n_matches_out, int32_t* ok_out) {
   MatcherBatch* b = r->batches[tid];
-  if (!imgs2 && b->stepAvailable(r->method)) {
+  if (runner_pipelined(r, tid, imgs2)) {
     uint32_t d[3] = {(uint32_t)dims[0], (uint32_t)dims[1], (uint32_t)dims[2]};
     std::vector<const uint8_t*> i1;
     for (int s = tid; s < r->S; s += r->threads) i1.push_back(imgs[s]);
@@ -466,8 +547,24 @@ VISOB_API void* visob_runner_create_stereo(int device, int n_sequences, int thre
   }
   return r;
 }
+// Structure from motion (mode 3): per sequence what StructureFromMotion keeps - a VisualOdometryMono on its sequence of the
+// worker's batch, the accumulated pose, the first-frame and replace flags and a Reconstruction with the facade's calibration
+// and constants (point type 0, min track length 2, 30 m, 3 degrees).  A step pushes every sequence with its replace flag,
+// runs flow matching and the mono odometry stages, and per worker ONE visocu_recon_points for the finished tracks of the
+// sequences whose frame is ok.  Steps are synchronous.
+VISOB_API void* visob_runner_create_sfm(int device, int n_sequences, int threads, const MonoParamsC* p) {
+  Runner* r = (Runner*)visob_runner_create(device, n_sequences, threads, 1, 0, p);
+  r->mode = 3;
+  for (int s = 0; s < n_sequences; s++) {
+    SfmState* q = new SfmState();
+    q->recon.setCalibration(p->f, p->cu, p->cv);
+    r->sfms.push_back(q);
+  }
+  return r;
+}
 VISOB_API void visob_runner_destroy(void* h) {
   Runner* r = (Runner*)h;
+  for (SfmState* q : r->sfms) delete q;
   for (MonoAccess* m : r->monos) delete m;
   for (StereoAccess* m : r->stereos) delete m;
   for (MatcherBatch* b : r->batches) delete b;
@@ -494,7 +591,7 @@ VISOB_API double visob_runner_run(void* h, int n_steps, const uint8_t* const* im
   run_workers(r->threads, [&](int tid) {
     visob::set_device(r->device);
     MatcherBatch* b = r->batches[tid];
-    if (imgs2 || !b->stepAvailable(r->method)) {
+    if (!runner_pipelined(r, tid, imgs2)) {
       for (int k = 0; k < n_steps; k++)
         runner_advance(r, tid, imgs + (size_t)k * r->S, imgs2 ? imgs2 + (size_t)k * r->S : 0, dims, on_device, bucket,
                        n_matches_out ? n_matches_out + (size_t)k * r->S : 0, ok_out ? ok_out + (size_t)k * r->S : 0);
@@ -527,23 +624,38 @@ VISOB_API double visob_runner_run(void* h, int n_steps, const uint8_t* const* im
 VISOB_API int visob_runner_get_matches(void* h, int seq, void* out, int cap) {
   Runner* r = (Runner*)h;
   if (seq < 0 || seq >= r->S) return -1;
-  if (r->mode == 1) return copy_matches(r->monos[seq]->usedMatches(), out, cap);
+  if (r->mode == 1 || r->mode == 3) return copy_matches(r->monos[seq]->usedMatches(), out, cap);
   if (r->mode == 2) return copy_matches(r->stereos[seq]->usedMatches(), out, cap);
   return copy_matches(r->matcher_of(seq).matches(2), out, cap);
 }
 VISOB_API void visob_runner_get_motion(void* h, int seq, double* out16) {
   Runner* r = (Runner*)h;
   if (r->mode == 0 || seq < 0 || seq >= r->S) return;
-  Matrix T = r->mode == 1 ? r->monos[seq]->getMotion() : r->stereos[seq]->getMotion();
+  Matrix T = r->mode == 2 ? r->stereos[seq]->getMotion() : r->monos[seq]->getMotion();
   for (int i = 0; i < 4; i++) for (int j = 0; j < 4; j++) out16[4 * i + j] = T.val[i][j];
 }
 // inlier indices of the last motion estimate (odometry modes); -1 for mode 0 or a bad sequence
 VISOB_API int visob_runner_get_inliers(void* h, int seq, int32_t* out, int cap) {
   Runner* r = (Runner*)h;
   if (r->mode == 0 || seq < 0 || seq >= r->S) return -1;
-  std::vector<int32_t> in = r->mode == 1 ? r->monos[seq]->getInlierIndices() : r->stereos[seq]->getInlierIndices();
+  std::vector<int32_t> in = r->mode == 2 ? r->stereos[seq]->getInlierIndices() : r->monos[seq]->getInlierIndices();
   if (out) memcpy(out, in.data(), sizeof(int32_t) * (size_t)std::min((int)in.size(), cap));
   return (int)in.size();
+}
+// structure-from-motion mode: the sequence's reconstructed points (x, y, z per point; returns the count, -1 for another mode
+// or a bad sequence) and its accumulated pose (first camera -> current camera)
+VISOB_API int visob_runner_get_points(void* h, int seq, float* out3, int cap) {
+  Runner* r = (Runner*)h;
+  if (r->mode != 3 || seq < 0 || seq >= r->S) return -1;
+  const std::vector<Point3d>& pts = r->sfms[seq]->recon.getPoints();
+  for (int i = 0; i < (int)pts.size() && i < cap; i++) { out3[3 * i] = pts[i].x; out3[3 * i + 1] = pts[i].y; out3[3 * i + 2] = pts[i].z; }
+  return (int)pts.size();
+}
+VISOB_API void visob_runner_get_pose(void* h, int seq, double* out16) {
+  Runner* r = (Runner*)h;
+  if (r->mode != 3 || seq < 0 || seq >= r->S) return;
+  const Matrix& T = r->sfms[seq]->Tr_total;
+  for (int i = 0; i < 4; i++) for (int j = 0; j < 4; j++) out16[4 * i + j] = T.val[i][j];
 }
 VISOB_API void visob_runner_transfer_bytes(void* h, uint64_t* h2d, uint64_t* d2h) {
   Runner* r = (Runner*)h;

@@ -13,6 +13,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <iostream>
+#include <memory>
 
 #include "delaunay.h"
 #include "device.h"
@@ -557,6 +558,12 @@ bool MatcherBatch::ensure(int32_t w, int32_t h) {
 }
 
 void MatcherBatch::pushBack(const uint8_t* const* I1, const uint8_t* const* I2, uint32_t* dims, bool replace, bool on_device) {
+  std::unique_ptr<bool[]> flags(new bool[seq.size()]);
+  for (size_t s = 0; s < seq.size(); s++) flags[s] = replace;
+  pushBack(I1, I2, dims, flags.get(), on_device);
+}
+
+void MatcherBatch::pushBack(const uint8_t* const* I1, const uint8_t* const* I2, uint32_t* dims, const bool* replace, bool on_device) {
   visob::StageTimer timer(0);
   if ((int32_t)dims[0] <= 0 || (int32_t)dims[1] <= 0 || dims[2] < dims[0]) {
     std::cerr << "ERROR: Image dimension mismatch!" << std::endl;
@@ -569,7 +576,7 @@ void MatcherBatch::pushBack(const uint8_t* const* I1, const uint8_t* const* I2, 
   for (size_t s = 0; s < S; s++) {
     int32_t f[2];
     const uint8_t* i2 = I2 ? I2[s] : 0;
-    if (!seq[s]->pushPrepare(I1[s], i2, dims, replace, f)) continue;
+    if (!seq[s]->pushPrepare(I1[s], i2, dims, replace[s], f)) continue;
     frames.push_back(f[0]); imgs.push_back(I1[s]); owner.push_back((int32_t)s);
     if (i2) { frames.push_back(f[1]); imgs.push_back(i2); owner.push_back((int32_t)s); }
   }

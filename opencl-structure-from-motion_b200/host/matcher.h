@@ -139,6 +139,8 @@ public:
   ~MatcherBatch();
   // one image (and optionally one right image) per sequence; dims as for Matcher::pushBack
   void pushBack(const uint8_t* const* I1, const uint8_t* const* I2, uint32_t* dims, bool replace, bool on_device = false);
+  // the same with a replace flag per sequence (Matcher::pushBack's replace: the new image takes the place of the current one)
+  void pushBack(const uint8_t* const* I1, const uint8_t* const* I2, uint32_t* dims, const bool* replace, bool on_device);
   // tr_delta (optional, one entry per sequence, null = no prediction): the previous motion of each sequence for the
   // motion-predicted quad search, as Matcher::matchFeatures(2, Tr_delta).  The sequences share one calibration (setIntrinsics).
   void matchFeatures(int32_t method, const Matrix* const* tr_delta = nullptr);

@@ -28,7 +28,8 @@ public:
 
   void setVerbose(bool on) { verbose = on; }     // the reference always prints; tests and batch runs switch it off
 
-  void update(uint8_t* img_data) {
+  // returns whether the odometry of this frame succeeded (an extension: the reference's update returns nothing)
+  bool update(uint8_t* img_data) {
     const bool ok = viso->process(img_data, &dims[0], replace);
     if (is_first_frame) {
       is_first_frame = false;
@@ -46,6 +47,7 @@ public:
       if (verbose) std::cout << "No motion" << std::endl;
       replace = true;
     }
+    return ok;
   }
 
   const std::vector<Point3d>& getPoints() { return reconstruction.getPoints(); }

@@ -4,7 +4,7 @@ import ctypes as C
 import os
 import numpy as np
 
-from visocu_py import Params, P_MATCH, VisocuError
+from visocu_py import Params, P_MATCH, RECON_FRAME, RECON_TRACK, ReconJob, VisocuError
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'libviso_b200.so')
@@ -52,7 +52,7 @@ def lib():
         if not os.path.exists(LIB_PATH):
             raise VisocuError(LIB_PATH + ' is missing: run __graft_entry__.build()')
         L = C.CDLL(LIB_PATH)
-        for name in ('visob_matcher_create', 'visob_mono_create', 'visob_mono_matcher', 'visob_runner_create', 'visob_runner_create_stereo', 'visob_stereo_create', 'visob_recon_create', 'visob_sfm_create',
+        for name in ('visob_matcher_create', 'visob_mono_create', 'visob_mono_matcher', 'visob_runner_create', 'visob_runner_create_stereo', 'visob_runner_create_sfm', 'visob_stereo_create', 'visob_recon_create', 'visob_sfm_create',
                      'visob_matcher_context'):
             getattr(L, name).restype = C.c_void_p
         L.visob_matcher_gain.restype = C.c_float
@@ -270,6 +270,60 @@ class Stereo:
         return bool(lib().visob_stereo_batch_finish(self.h, _p(tr6), int(ok), _p(mask)))
 
 
+class Recon:
+    """Reconstruction (host/reconstruction.h): update() on the host, or its two halves around an evaluation of the finished
+    tracks elsewhere (batch_prepare, batch_job, then host_eval or visocu_py.Context.recon_points, then batch_finish)."""
+
+    def __init__(self, f, cu, cv):
+        self.h = C.c_void_p(lib().visob_recon_create())
+        lib().visob_recon_set_calibration(self.h, C.c_double(f), C.c_double(cu), C.c_double(cv))
+
+    def __del__(self):
+        if getattr(self, 'h', None):
+            lib().visob_recon_destroy(self.h)
+            self.h = None
+
+    def update(self, matches, tr, point_type=1, min_track_length=2, max_dist=30.0, min_angle=2.0):
+        m = np.ascontiguousarray(matches, P_MATCH); tr = np.ascontiguousarray(tr, np.float64)
+        lib().visob_recon_update(self.h, _p(m), len(m), _p(tr), int(point_type), int(min_track_length), C.c_double(max_dist),
+                                 C.c_double(min_angle))
+
+    def batch_prepare(self, matches, tr, point_type=1, min_track_length=2, max_dist=30.0, min_angle=2.0):
+        """update()'s bookkeeping; returns the number of finished tracks to evaluate."""
+        m = np.ascontiguousarray(matches, P_MATCH); tr = np.ascontiguousarray(tr, np.float64)
+        return lib().visob_recon_batch_prepare(self.h, _p(m), len(m), _p(tr), int(point_type), int(min_track_length),
+                                               C.c_double(max_dist), C.c_double(min_angle))
+
+    def batch_job(self):
+        """The prepared job as a dict (frames, tracks, cam_road, max_dist, min_angle, point_type), copied out."""
+        job = ReconJob()
+        lib().visob_recon_batch_job(self.h, C.byref(job), None, None)
+        frames = np.zeros(job.n_frames, RECON_FRAME); tracks = np.zeros(job.n_tracks, RECON_TRACK)
+        lib().visob_recon_batch_job(self.h, C.byref(job), _p(frames), _p(tracks))
+        return dict(frames=frames, tracks=tracks, cam_road=np.array(job.cam_road[:]), max_dist=job.max_dist,
+                    min_angle=job.min_angle, point_type=job.point_type)
+
+    def host_eval(self):
+        """The host functions on the prepared tracks: (status, xyz) with the meaning of visocu_recon_points."""
+        job = ReconJob()
+        lib().visob_recon_batch_job(self.h, C.byref(job), None, None)
+        status = np.zeros(job.n_tracks, np.int32); xyz = np.zeros((job.n_tracks, 3), np.float32)
+        lib().visob_recon_host_eval(self.h, _p(status), _p(xyz))
+        return status, xyz
+
+    def batch_finish(self, status, xyz):
+        """Appends the points of the prepared tracks whose status is 0."""
+        status = np.ascontiguousarray(status, np.int32); xyz = np.ascontiguousarray(xyz, np.float32)
+        lib().visob_recon_batch_finish(self.h, _p(status), _p(xyz))
+
+    def points(self):
+        n = lib().visob_recon_get_points(self.h, None, 0)
+        out = np.zeros((n, 3), np.float32)
+        if n:
+            lib().visob_recon_get_points(self.h, _p(out), n)
+        return out
+
+
 class Sfm:
     """StructureFromMotion facade (host/sfm.h)."""
 
@@ -283,8 +337,9 @@ class Sfm:
             self.h = None
 
     def update(self, img):
+        """One frame; returns whether its odometry succeeded."""
         img = np.ascontiguousarray(img, np.uint8)
-        lib().visob_sfm_update(self.h, _p(img))
+        return bool(lib().visob_sfm_update(self.h, _p(img)))
 
     def points(self):
         n = lib().visob_sfm_get_points(self.h, None, 0)
@@ -336,7 +391,7 @@ def svd(A):
 
 class Runner:
     """S independent sequences on one GPU driven by `threads` host workers (mode 0: Matcher, 1: mono odometry,
-    2: stereo odometry - see Runner.stereo)."""
+    2: stereo odometry - see Runner.stereo, 3: structure from motion - see Runner.sfm)."""
 
     def __init__(self, device, n_sequences, threads, mode, method, mono_params):
         self.S = n_sequences
@@ -350,6 +405,16 @@ class Runner:
         r.S = n_sequences
         r.mp = stereo_params
         r.h = C.c_void_p(lib().visob_runner_create_stereo(device, n_sequences, threads, C.byref(stereo_params)))
+        return r
+
+    @classmethod
+    def sfm(cls, device, n_sequences, threads, mono_params):
+        """Structure-from-motion runner (mode 3): per sequence what the StructureFromMotion facade does (Sfm), with the
+        finished tracks of each worker's sequences reconstructed by one device call per step; steps are synchronous."""
+        r = cls.__new__(cls)
+        r.S = n_sequences
+        r.mp = mono_params
+        r.h = C.c_void_p(lib().visob_runner_create_sfm(device, n_sequences, threads, C.byref(mono_params)))
         return r
 
     def close(self):
@@ -396,6 +461,20 @@ class Runner:
         out = np.zeros(max(n, 0), np.int32)
         if n > 0:
             lib().visob_runner_get_inliers(self.h, seq, _p(out), n)
+        return out
+
+    def points(self, seq):
+        """The sequence's reconstructed points (structure-from-motion mode)."""
+        n = lib().visob_runner_get_points(self.h, seq, None, 0)
+        out = np.zeros((max(n, 0), 3), np.float32)
+        if n > 0:
+            lib().visob_runner_get_points(self.h, seq, _p(out), n)
+        return out
+
+    def pose(self, seq):
+        """The sequence's accumulated pose, first camera -> current camera (structure-from-motion mode)."""
+        out = np.zeros((4, 4))
+        lib().visob_runner_get_pose(self.h, seq, _p(out))
         return out
 
     def launches(self):

@@ -17,6 +17,16 @@ RANGE = np.dtype([('u_min', 'f4', 4), ('u_max', 'f4', 4), ('v_min', 'f4', 4), ('
 QUAD = np.dtype([('f1p', 'i4'), ('f2p', 'i4'), ('f1c', 'i4'), ('f2c', 'i4')])
 
 
+RECON_FRAME = np.dtype([('proj', 'f8', 12), ('inv', 'f8', 12), ('center', 'f8', 3)])        # visocu_recon_frame
+RECON_TRACK = np.dtype([('first', 'i4'), ('n_obs', 'i4'), ('u', 'f4', 6), ('v', 'f4', 6)])   # visocu_recon_track
+
+
+class ReconJob(C.Structure):
+    """visocu_recon_job: the finished tracks of one Reconstruction update and the window they refer to."""
+    _fields_ = [('frames', C.c_void_p), ('n_frames', C.c_int32), ('tracks', C.c_void_p), ('n_tracks', C.c_int32),
+                ('cam_road', C.c_double * 12), ('max_dist', C.c_double), ('min_angle', C.c_double), ('point_type', C.c_int32)]
+
+
 class StereoMotionParams(C.Structure):
     """visocu_stereo_params: calibration and RANSAC settings of VisualOdometryStereo::parameters."""
     _fields_ = [(n, C.c_double) for n in ('f', 'cu', 'cv', 'base', 'inlier_threshold')] + \
@@ -310,3 +320,24 @@ class Context:
         return [dict(ok=bool(ok[j]), tr=tr[j].copy(), mask=masks[j], inliers=np.nonzero(masks[j])[0].astype(np.int32),
                      n_inliers=int(ninl[j]), best_iter=int(best[j]), counts=counts[j] if want_all else None,
                      tr_all=trall[j] if want_all else None) for j in range(nj)]
+
+    # ---- reconstruction
+    def recon_points(self, jobs):
+        """visocu_recon_points for a list of jobs, each a dict with frames (RECON_FRAME array), tracks (RECON_TRACK array),
+        cam_road (12), max_dist, min_angle and point_type (host_py.Recon.batch_job makes them).  Returns one
+        (status int32 array, xyz float32 n x 3 array) per job."""
+        nj = len(jobs)
+        arr = (ReconJob * max(nj, 1))()
+        keep, status, xyz = [], [], []
+        for j, job in enumerate(jobs):
+            fr = np.ascontiguousarray(job['frames'], RECON_FRAME); tr = np.ascontiguousarray(job['tracks'], RECON_TRACK)
+            keep += [fr, tr]
+            a = arr[j]
+            a.frames, a.n_frames, a.tracks, a.n_tracks = fr.ctypes.data, len(fr), tr.ctypes.data, len(tr)
+            a.cam_road[:] = [float(x) for x in np.ravel(job['cam_road'])]
+            a.max_dist, a.min_angle, a.point_type = job['max_dist'], job['min_angle'], int(job['point_type'])
+            status.append(np.zeros(len(tr), np.int32)); xyz.append(np.zeros((len(tr), 3), np.float32))
+        sp = (C.c_void_p * max(nj, 1))(*[x.ctypes.data for x in status])
+        xp = (C.c_void_p * max(nj, 1))(*[x.ctypes.data for x in xyz])
+        self._ck(lib().visocu_recon_points(self.h, nj, arr, sp, xp), 'recon_points')
+        return list(zip(status, xyz))
