@@ -153,11 +153,6 @@ struct StereoParamsC {        // flat mirror of VisualOdometryStereo::parameters
   double f, cu, cv;
   double base; int32_t ransac_iters; double inlier_threshold; int32_t reweighting;
 };
-struct StereoAccess : public VisualOdometryStereo {
-  explicit StereoAccess(VisualOdometryStereo::parameters p) : VisualOdometryStereo(p) {}
-  // what process() hands to the quad matching: the previous motion once there is a valid one
-  const Matrix* predictedMotion() const { return Tr_valid ? &Tr_delta : nullptr; }
-};
 VisualOdometryStereo::parameters to_cpp(const StereoParamsC* p) {
   VisualOdometryStereo::parameters q;
   q.match = p->match;
@@ -167,28 +162,28 @@ VisualOdometryStereo::parameters to_cpp(const StereoParamsC* p) {
   return q;
 }
 }  // namespace
-VISOB_API void* visob_stereo_create(const StereoParamsC* p) { return new StereoAccess(to_cpp(p)); }
-VISOB_API void visob_stereo_destroy(void* v) { delete (StereoAccess*)v; }
+VISOB_API void* visob_stereo_create(const StereoParamsC* p) { return new VisualOdometryStereo(to_cpp(p)); }
+VISOB_API void visob_stereo_destroy(void* v) { delete (VisualOdometryStereo*)v; }
 VISOB_API int visob_stereo_process(void* v, uint8_t* I1, uint8_t* I2, const int32_t* dims, int replace) {
   uint32_t d[3] = {(uint32_t)dims[0], (uint32_t)dims[1], (uint32_t)dims[2]};
-  return ((StereoAccess*)v)->process(I1, I2, d, replace != 0) ? 1 : 0;
+  return ((VisualOdometryStereo*)v)->process(I1, I2, d, replace != 0) ? 1 : 0;
 }
 VISOB_API int visob_stereo_process_matches(void* v, const void* matches, int n) {     // host only: no image, no GPU
   std::vector<Matcher::p_match> pm((const Matcher::p_match*)matches, (const Matcher::p_match*)matches + n);
-  return ((VisualOdometry*)(StereoAccess*)v)->process(pm) ? 1 : 0;
+  return ((VisualOdometry*)(VisualOdometryStereo*)v)->process(pm) ? 1 : 0;
 }
 VISOB_API void visob_stereo_get_motion(void* v, double* out16) {
-  Matrix T = ((StereoAccess*)v)->getMotion();
+  Matrix T = ((VisualOdometryStereo*)v)->getMotion();
   for (int i = 0; i < 4; i++) for (int j = 0; j < 4; j++) out16[4 * i + j] = T.val[i][j];
 }
-VISOB_API int visob_stereo_get_matches(void* v, void* out, int cap) { return copy_matches(((StereoAccess*)v)->usedMatches(), out, cap); }
+VISOB_API int visob_stereo_get_matches(void* v, void* out, int cap) { return copy_matches(((VisualOdometryStereo*)v)->usedMatches(), out, cap); }
 VISOB_API int visob_stereo_get_inliers(void* v, int32_t* out, int cap) {
-  std::vector<int32_t> in = ((StereoAccess*)v)->getInlierIndices();
+  std::vector<int32_t> in = ((VisualOdometryStereo*)v)->getInlierIndices();
   if (out) memcpy(out, in.data(), sizeof(int32_t) * (size_t)std::min((int)in.size(), cap));
   return (int)in.size();
 }
 VISOB_API int visob_stereo_get_samples(void* v, int32_t* out, int cap) {
-  const std::vector<int>& s = ((StereoAccess*)v)->lastSamples();
+  const std::vector<int>& s = ((VisualOdometryStereo*)v)->lastSamples();
   if (out) for (int i = 0; i < std::min((int)s.size(), cap); i++) out[i] = s[i];
   return (int)s.size();
 }
@@ -196,10 +191,10 @@ VISOB_API int visob_stereo_get_samples(void* v, int32_t* out, int cap) {
 VISOB_API int visob_stereo_batch_prepare(void* v, const void* matches, int n) {
   std::vector<Matcher::p_match> pm((const Matcher::p_match*)matches, (const Matcher::p_match*)matches + n);
   const visocu_pmatch* m = 0; int32_t N = 0; const int32_t* smp = 0;
-  return ((StereoAccess*)v)->batchPrepare(pm, &m, &N, &smp) ? 1 : 0;
+  return ((VisualOdometryStereo*)v)->batchPrepare(pm, &m, &N, &smp) ? 1 : 0;
 }
 VISOB_API int visob_stereo_batch_finish(void* v, const double* tr6, int ok, const uint8_t* mask) {
-  return ((StereoAccess*)v)->batchFinish(tr6, ok, mask) ? 1 : 0;
+  return ((VisualOdometryStereo*)v)->batchFinish(tr6, ok, mask) ? 1 : 0;
 }
 VISOB_API void visob_matcher_match_features_tr(void* m, int method, const double* tr16) {
   Matrix T(4, 4, tr16);
@@ -255,6 +250,28 @@ VISOB_API void visob_sfm_get_pose(void* s, double* out16) {
   const Matrix& T = ((StructureFromMotion*)s)->getPose();
   for (int i = 0; i < 4; i++) for (int j = 0; j < 4; j++) out16[4 * i + j] = T.val[i][j];
 }
+// the stereo facade (host/sfm.h), created with verbose output off; _odometry gives its VisualOdometryStereo for the
+// visob_stereo_get_* entries
+VISOB_API void* visob_stereo_sfm_create(const StereoParamsC* p, const int32_t* dims) {
+  StructureFromMotionStereo* s =
+      new StructureFromMotionStereo(to_cpp(p), std::array<uint32_t, 3>{{(uint32_t)dims[0], (uint32_t)dims[1], (uint32_t)dims[2]}});
+  s->setVerbose(false);
+  return s;
+}
+VISOB_API void visob_stereo_sfm_destroy(void* s) { delete (StructureFromMotionStereo*)s; }
+VISOB_API int visob_stereo_sfm_update(void* s, uint8_t* left, uint8_t* right) {
+  return ((StructureFromMotionStereo*)s)->update(left, right) ? 1 : 0;
+}
+VISOB_API int visob_stereo_sfm_get_points(void* s, float* out3, int cap) {
+  const std::vector<Point3d>& pts = ((StructureFromMotionStereo*)s)->getPoints();
+  for (int i = 0; i < (int)pts.size() && i < cap; i++) { out3[3 * i] = pts[i].x; out3[3 * i + 1] = pts[i].y; out3[3 * i + 2] = pts[i].z; }
+  return (int)pts.size();
+}
+VISOB_API void visob_stereo_sfm_get_pose(void* s, double* out16) {
+  const Matrix& T = ((StructureFromMotionStereo*)s)->getPose();
+  for (int i = 0; i < 4; i++) for (int j = 0; j < 4; j++) out16[4 * i + j] = T.val[i][j];
+}
+VISOB_API void* visob_stereo_sfm_odometry(void* s) { return &((StructureFromMotionStereo*)s)->odometry(); }
 
 // ---- host utilities exposed for tests
 VISOB_API int visob_delaunay(const int32_t* x, const int32_t* y, int n, int32_t* tri_out, int cap_tri) {
@@ -290,30 +307,32 @@ VISOB_API void visob_svd(const double* A, int m, int n, double* U, double* W, do
 // stage a single batched launch for all of the worker's sequences) and runs their host stages (outlier removal, priors,
 // bucketing) in between; the workers' streams overlap on the GPU.  Odometry modes: one VisualOdometryMono or
 // VisualOdometryStereo per sequence, running on its sequence of the worker's batch; the GPU stages of the motion estimate
-// are one batched call per worker.  Structure-from-motion mode: mono odometry as above, then what StructureFromMotion::update
-// does per sequence, with the finished tracks of all of the worker's sequences evaluated by one device call.
+// are one batched call per worker.  Structure-from-motion modes: mono (mode 3) or stereo (mode 4) odometry as above, then
+// what StructureFromMotion::update or StructureFromMotionStereo::update does per sequence, with the finished tracks of all
+// of the worker's sequences evaluated by one device call.
 namespace {
-struct SfmState {                            // what StructureFromMotion keeps besides its odometry object (host/sfm.h)
+struct SfmState {                            // what the facades keep besides their odometry object (host/sfm.h)
   Reconstruction recon;
   Matrix Tr_total = Matrix::eye(4);
   bool first = true, replace = false;
 };
 struct Runner {
   int device, S, threads, mode, method;      // mode 0 = Matcher only, 1 = VisualOdometryMono::process, 2 = VisualOdometryStereo::process,
-                                             // 3 = StructureFromMotion::update
+                                             // 3 = StructureFromMotion::update, 4 = StructureFromMotionStereo::update
   int bucket_max; float bucket_w, bucket_h;
   MonoParamsC params;
   StereoParamsC sparams;
   std::vector<MatcherBatch*> batches;        // one per worker
   std::vector<MonoAccess*> monos;            // one per sequence (modes 1 and 3)
-  std::vector<StereoAccess*> stereos;        // one per sequence (mode 2)
-  std::vector<SfmState*> sfms;               // one per sequence (mode 3)
+  std::vector<VisualOdometryStereo*> stereos; // one per sequence (modes 2 and 4)
+  std::vector<SfmState*> sfms;               // one per sequence (modes 3 and 4)
   std::vector<int32_t> last_matches, last_ok;
   Matcher& matcher_of(int seq) { return batches[seq % threads]->sequence(seq / threads); }
 };
 
-// StructureFromMotion::update after the odometry of one frame, for every sequence of worker `tid`: pose accumulation and
-// Reconstruction::batchPrepare for the sequences whose frame is ok, ONE visocu_recon_points for all of them, batchFinish;
+// StructureFromMotion::update (mode 3) or StructureFromMotionStereo::update (mode 4) after the odometry of one frame, for
+// every sequence of worker `tid`: pose accumulation and Reconstruction::batchPrepare for the sequences whose frame is ok,
+// ONE visocu_recon_points for all of them, batchFinish;
 // a failed frame is replaced by the next push.  If the device call fails, the finished tracks of the step are lost and the
 // step reports ok = 0 for those sequences (their pose has already advanced, as the facade's does on a successful frame).
 void runner_sfm(Runner* r, int tid) {
@@ -321,7 +340,7 @@ void runner_sfm(Runner* r, int tid) {
   std::vector<visocu_recon_job> jobs;
   for (int s = tid; s < r->S; s += r->threads) {
     SfmState& q = *r->sfms[s];
-    MonoAccess& vo = *r->monos[s];
+    VisualOdometry& vo = r->mode == 4 ? (VisualOdometry&)*r->stereos[s] : (VisualOdometry&)*r->monos[s];
     if (q.first) { q.first = false; continue; }
     if (!r->last_ok[s]) { q.replace = true; continue; }
     q.Tr_total = q.Tr_total * Matrix::inv(vo.getMotion());
@@ -356,7 +375,7 @@ void runner_sfm(Runner* r, int tid) {
 // mode normalisation, sample tables, ONE batched RANSAC call for all of the worker's sequences, pose
 void runner_post(Runner* r, int tid, int bucket, int32_t* n_matches_out, int32_t* ok_out) {
   MatcherBatch* b = r->batches[tid];
-  if (r->mode == 2) {
+  if (r->mode == 2 || r->mode == 4) {
     // bucketing and sample tables per sequence, then ONE device motion estimate for all of the worker's sequences
     std::vector<int> ids;
     std::vector<const visocu_pmatch*> ml;
@@ -446,7 +465,7 @@ void runner_post(Runner* r, int tid, int bucket, int32_t* n_matches_out, int32_t
       r->last_ok[s] = 1;
     }
   }
-  if (r->mode == 3) runner_sfm(r, tid);
+  if (r->mode == 3 || r->mode == 4) runner_sfm(r, tid);
   for (int s = tid; s < r->S; s += r->threads) {
     if (n_matches_out) n_matches_out[s] = r->last_matches[s];
     if (ok_out) ok_out[s] = r->last_ok[s];
@@ -457,19 +476,19 @@ void runner_push(Runner* r, int tid, const uint8_t* const* imgs, const uint8_t* 
   uint32_t d[3] = {(uint32_t)dims[0], (uint32_t)dims[1], (uint32_t)dims[2]};
   std::vector<const uint8_t*> i1, i2;
   for (int s = tid; s < r->S; s += r->threads) { i1.push_back(imgs[s]); if (imgs2) i2.push_back(imgs2[s]); }
-  if (r->mode == 3) {                              // each sequence's replace flag, as StructureFromMotion passes it
+  if (r->mode == 3 || r->mode == 4) {              // each sequence's replace flag, as the facades pass it
     std::unique_ptr<bool[]> replace(new bool[i1.size()]);
     size_t k = 0;
     for (int s = tid; s < r->S; s += r->threads) replace[k++] = r->sfms[s]->replace;
-    r->batches[tid]->pushBack(i1.data(), 0, d, replace.get(), on_device != 0);
+    r->batches[tid]->pushBack(i1.data(), r->mode == 4 ? i2.data() : 0, d, replace.get(), on_device != 0);
     return;
   }
   r->batches[tid]->pushBack(i1.data(), imgs2 ? i2.data() : 0, d, false, on_device != 0);
 }
 
-// Steps of mode 3 never take the pipelined path: a step's push needs the previous step's outcome (the replace flag).
+// Steps of modes 3 and 4 never take the pipelined path: a step's push needs the previous step's outcome (the replace flag).
 bool runner_pipelined(Runner* r, int tid, const uint8_t* const* imgs2) {
-  return !imgs2 && r->mode != 3 && r->batches[tid]->stepAvailable(r->method);
+  return !imgs2 && r->mode != 3 && r->mode != 4 && r->batches[tid]->stepAvailable(r->method);
 }
 
 // one frame for every sequence of worker `tid`, synchronously
@@ -484,7 +503,7 @@ void runner_advance(Runner* r, int tid, const uint8_t* const* imgs, const uint8_
     if (b->stepSubmit(i1.data(), d, on_device != 0)) b->stepCollect();
   } else {
     runner_push(r, tid, imgs, imgs2, dims, on_device);
-    if (r->mode == 2) {
+    if (r->mode == 2 || r->mode == 4) {
       std::vector<const Matrix*> pred;                 // quad matching with each sequence's motion, as process() does
       for (int s = tid; s < r->S; s += r->threads) pred.push_back(r->stereos[s]->predictedMotion());
       b->matchFeatures(r->method, pred.data());
@@ -541,7 +560,7 @@ VISOB_API void* visob_runner_create_stereo(int device, int n_sequences, int thre
   r->sparams = *p;
   r->bucket_max = p->bucket_max_features; r->bucket_w = (float)p->bucket_width; r->bucket_h = (float)p->bucket_height;
   for (int s = 0; s < n_sequences; s++) {
-    StereoAccess* vo = new StereoAccess(to_cpp(p));
+    VisualOdometryStereo* vo = new VisualOdometryStereo(to_cpp(p));
     vo->adoptMatcher(&r->batches[s % r->threads]->sequence(s / r->threads));
     r->stereos.push_back(vo);
   }
@@ -562,19 +581,35 @@ VISOB_API void* visob_runner_create_sfm(int device, int n_sequences, int threads
   }
   return r;
 }
+// Stereo structure from motion (mode 4): per sequence a VisualOdometryStereo on its sequence of the worker's batch, as in
+// mode 2, and what StructureFromMotionStereo keeps besides it, as in mode 3.  A step pushes the left and right images of
+// every sequence with its replace flag, runs quad matching with each sequence's previous motion, per worker ONE
+// visocu_stereo_motion and then ONE visocu_recon_points.  Steps are synchronous and need right images.
+VISOB_API void* visob_runner_create_stereo_sfm(int device, int n_sequences, int threads, const StereoParamsC* p) {
+  Runner* r = (Runner*)visob_runner_create_stereo(device, n_sequences, threads, p);
+  r->mode = 4;
+  for (int s = 0; s < n_sequences; s++) {
+    SfmState* q = new SfmState();
+    q->recon.setCalibration(p->f, p->cu, p->cv);
+    r->sfms.push_back(q);
+  }
+  return r;
+}
 VISOB_API void visob_runner_destroy(void* h) {
   Runner* r = (Runner*)h;
   for (SfmState* q : r->sfms) delete q;
   for (MonoAccess* m : r->monos) delete m;
-  for (StereoAccess* m : r->stereos) delete m;
+  for (VisualOdometryStereo* m : r->stereos) delete m;
   for (MatcherBatch* b : r->batches) delete b;
   delete r;
 }
 // imgs / imgs2: S pointers (imgs2 may be null for mono / flow).  on_device: pointers are device memory.
-// bucket: apply bucketFeatures after matching (mode 0).  Returns wall seconds spent in the step.
+// bucket: apply bucketFeatures after matching (mode 0).  Returns wall seconds spent in the step; -1 for a mode-4 step
+// without right images (nothing is pushed or written).
 VISOB_API double visob_runner_step(void* h, const uint8_t* const* imgs, const uint8_t* const* imgs2, const int32_t* dims,
                                    int on_device, int bucket, int32_t* n_matches_out, int32_t* ok_out) {
   Runner* r = (Runner*)h;
+  if (r->mode == 4 && !imgs2) return -1.0;
   auto t0 = std::chrono::steady_clock::now();
   run_workers(r->threads, [&](int tid) {
     visob::set_device(r->device);
@@ -583,10 +618,12 @@ VISOB_API double visob_runner_step(void* h, const uint8_t* const* imgs, const ui
   return std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
 }
 // K steps without a barrier between them: worker t walks its sequences (t, t + threads, ...) through all K frames.
-// imgs / imgs2: K x S pointers, step-major.  n_matches_out / ok_out (K x S, optional) receive per-pair results.
+// imgs / imgs2: K x S pointers, step-major.  n_matches_out / ok_out (K x S, optional) receive per-pair results.  -1 as
+// visob_runner_step.
 VISOB_API double visob_runner_run(void* h, int n_steps, const uint8_t* const* imgs, const uint8_t* const* imgs2, const int32_t* dims,
                                   int on_device, int bucket, int32_t* n_matches_out, int32_t* ok_out) {
   Runner* r = (Runner*)h;
+  if (r->mode == 4 && !imgs2) return -1.0;
   auto t0 = std::chrono::steady_clock::now();
   run_workers(r->threads, [&](int tid) {
     visob::set_device(r->device);
@@ -625,35 +662,35 @@ VISOB_API int visob_runner_get_matches(void* h, int seq, void* out, int cap) {
   Runner* r = (Runner*)h;
   if (seq < 0 || seq >= r->S) return -1;
   if (r->mode == 1 || r->mode == 3) return copy_matches(r->monos[seq]->usedMatches(), out, cap);
-  if (r->mode == 2) return copy_matches(r->stereos[seq]->usedMatches(), out, cap);
+  if (r->mode == 2 || r->mode == 4) return copy_matches(r->stereos[seq]->usedMatches(), out, cap);
   return copy_matches(r->matcher_of(seq).matches(2), out, cap);
 }
 VISOB_API void visob_runner_get_motion(void* h, int seq, double* out16) {
   Runner* r = (Runner*)h;
   if (r->mode == 0 || seq < 0 || seq >= r->S) return;
-  Matrix T = r->mode == 2 ? r->stereos[seq]->getMotion() : r->monos[seq]->getMotion();
+  Matrix T = r->mode == 2 || r->mode == 4 ? r->stereos[seq]->getMotion() : r->monos[seq]->getMotion();
   for (int i = 0; i < 4; i++) for (int j = 0; j < 4; j++) out16[4 * i + j] = T.val[i][j];
 }
 // inlier indices of the last motion estimate (odometry modes); -1 for mode 0 or a bad sequence
 VISOB_API int visob_runner_get_inliers(void* h, int seq, int32_t* out, int cap) {
   Runner* r = (Runner*)h;
   if (r->mode == 0 || seq < 0 || seq >= r->S) return -1;
-  std::vector<int32_t> in = r->mode == 2 ? r->stereos[seq]->getInlierIndices() : r->monos[seq]->getInlierIndices();
+  std::vector<int32_t> in = r->mode == 2 || r->mode == 4 ? r->stereos[seq]->getInlierIndices() : r->monos[seq]->getInlierIndices();
   if (out) memcpy(out, in.data(), sizeof(int32_t) * (size_t)std::min((int)in.size(), cap));
   return (int)in.size();
 }
-// structure-from-motion mode: the sequence's reconstructed points (x, y, z per point; returns the count, -1 for another mode
-// or a bad sequence) and its accumulated pose (first camera -> current camera)
+// structure-from-motion modes (3 and 4): the sequence's reconstructed points (x, y, z per point; returns the count, -1 for
+// another mode or a bad sequence) and its accumulated pose (first camera -> current camera)
 VISOB_API int visob_runner_get_points(void* h, int seq, float* out3, int cap) {
   Runner* r = (Runner*)h;
-  if (r->mode != 3 || seq < 0 || seq >= r->S) return -1;
+  if ((r->mode != 3 && r->mode != 4) || seq < 0 || seq >= r->S) return -1;
   const std::vector<Point3d>& pts = r->sfms[seq]->recon.getPoints();
   for (int i = 0; i < (int)pts.size() && i < cap; i++) { out3[3 * i] = pts[i].x; out3[3 * i + 1] = pts[i].y; out3[3 * i + 2] = pts[i].z; }
   return (int)pts.size();
 }
 VISOB_API void visob_runner_get_pose(void* h, int seq, double* out16) {
   Runner* r = (Runner*)h;
-  if (r->mode != 3 || seq < 0 || seq >= r->S) return;
+  if ((r->mode != 3 && r->mode != 4) || seq < 0 || seq >= r->S) return;
   const Matrix& T = r->sfms[seq]->Tr_total;
   for (int i = 0; i < 4; i++) for (int j = 0; j < 4; j++) out16[4 * i + j] = T.val[i][j];
 }

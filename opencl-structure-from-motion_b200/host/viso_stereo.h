@@ -38,6 +38,8 @@ public:
   bool batchFinish(const double* tr6, int32_t ok, const uint8_t* inlier_mask);
   // the sample table of the last estimate (either path)
   const std::vector<int>& lastSamples() const { return samples_last; }
+  // what process() hands to the quad matching: the previous motion once there is a valid one, else null
+  Matrix* predictedMotion() { return Tr_valid ? &Tr_delta : nullptr; }
 
 private:
   enum result { UPDATED, FAILED, CONVERGED };

@@ -53,7 +53,7 @@ def lib():
             raise VisocuError(LIB_PATH + ' is missing: run __graft_entry__.build()')
         L = C.CDLL(LIB_PATH)
         for name in ('visob_matcher_create', 'visob_mono_create', 'visob_mono_matcher', 'visob_runner_create', 'visob_runner_create_stereo', 'visob_runner_create_sfm', 'visob_stereo_create', 'visob_recon_create', 'visob_sfm_create',
-                     'visob_matcher_context'):
+                     'visob_matcher_context', 'visob_runner_create_stereo_sfm', 'visob_stereo_sfm_create', 'visob_stereo_sfm_odometry'):
             getattr(L, name).restype = C.c_void_p
         L.visob_matcher_gain.restype = C.c_float
         L.visob_runner_step.restype = C.c_double
@@ -214,12 +214,15 @@ class Mono:
 
 
 class Stereo:
-    def __init__(self, params):
+    def __init__(self, params, handle=None, owner=None):
+        """handle: an existing VisualOdometryStereo that `owner` keeps alive (StereoSfm.odometry); not destroyed here."""
         self.params = params
-        self.h = C.c_void_p(lib().visob_stereo_create(C.byref(params)))
+        self.owner = owner
+        self.owned = handle is None
+        self.h = C.c_void_p(lib().visob_stereo_create(C.byref(params)) if handle is None else handle)
 
     def __del__(self):
-        if getattr(self, 'h', None):
+        if getattr(self, 'owned', False) and self.h:
             lib().visob_stereo_destroy(self.h)
             self.h = None
 
@@ -354,6 +357,41 @@ class Sfm:
         return out
 
 
+class StereoSfm:
+    """StructureFromMotionStereo facade (host/sfm.h): stereo odometry and reconstruction, both estimated on the GPU."""
+
+    def __init__(self, params, width, height):
+        self.params = params
+        self.dims = np.array([width, height, width], np.int32)
+        self.h = C.c_void_p(lib().visob_stereo_sfm_create(C.byref(params), _p(self.dims)))
+
+    def __del__(self):
+        if getattr(self, 'h', None):
+            lib().visob_stereo_sfm_destroy(self.h)
+            self.h = None
+
+    def update(self, left, right):
+        """One stereo pair; returns whether its odometry (and, after the first frame, its reconstruction) succeeded."""
+        left = np.ascontiguousarray(left, np.uint8); right = np.ascontiguousarray(right, np.uint8)
+        return bool(lib().visob_stereo_sfm_update(self.h, _p(left), _p(right)))
+
+    def points(self):
+        n = lib().visob_stereo_sfm_get_points(self.h, None, 0)
+        out = np.zeros((n, 3), np.float32)
+        if n:
+            lib().visob_stereo_sfm_get_points(self.h, _p(out), n)
+        return out
+
+    def pose(self):
+        out = np.zeros((4, 4))
+        lib().visob_stereo_sfm_get_pose(self.h, _p(out))
+        return out
+
+    def odometry(self):
+        """The facade's VisualOdometryStereo (matches, inliers, motion of the last frame) as a Stereo view."""
+        return Stereo(self.params, handle=lib().visob_stereo_sfm_odometry(self.h), owner=self)
+
+
 def set_pipeline_depth(depth):
     """Steps that Runner.run keeps in flight per sequence (1 = synchronous, default and maximum 3)."""
     lib().visob_set_pipeline_depth(int(depth))
@@ -391,7 +429,8 @@ def svd(A):
 
 class Runner:
     """S independent sequences on one GPU driven by `threads` host workers (mode 0: Matcher, 1: mono odometry,
-    2: stereo odometry - see Runner.stereo, 3: structure from motion - see Runner.sfm)."""
+    2: stereo odometry - see Runner.stereo, 3: structure from motion - see Runner.sfm, 4: stereo structure from motion -
+    see Runner.stereo_sfm)."""
 
     def __init__(self, device, n_sequences, threads, mode, method, mono_params):
         self.S = n_sequences
@@ -415,6 +454,17 @@ class Runner:
         r.S = n_sequences
         r.mp = mono_params
         r.h = C.c_void_p(lib().visob_runner_create_sfm(device, n_sequences, threads, C.byref(mono_params)))
+        return r
+
+    @classmethod
+    def stereo_sfm(cls, device, n_sequences, threads, stereo_params):
+        """Stereo structure-from-motion runner (mode 4): per sequence what the StereoSfm facade does, with one
+        visocu_stereo_motion and one visocu_recon_points per worker and step; step() / run() take left and right images
+        (without right images they return -1 and do nothing) and are synchronous."""
+        r = cls.__new__(cls)
+        r.S = n_sequences
+        r.mp = stereo_params
+        r.h = C.c_void_p(lib().visob_runner_create_stereo_sfm(device, n_sequences, threads, C.byref(stereo_params)))
         return r
 
     def close(self):
@@ -464,7 +514,7 @@ class Runner:
         return out
 
     def points(self, seq):
-        """The sequence's reconstructed points (structure-from-motion mode)."""
+        """The sequence's reconstructed points (structure-from-motion modes)."""
         n = lib().visob_runner_get_points(self.h, seq, None, 0)
         out = np.zeros((max(n, 0), 3), np.float32)
         if n > 0:
@@ -472,7 +522,7 @@ class Runner:
         return out
 
     def pose(self, seq):
-        """The sequence's accumulated pose, first camera -> current camera (structure-from-motion mode)."""
+        """The sequence's accumulated pose, first camera -> current camera (structure-from-motion modes)."""
         out = np.zeros((4, 4))
         lib().visob_runner_get_pose(self.h, seq, _p(out))
         return out
