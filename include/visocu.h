@@ -240,6 +240,32 @@ typedef struct {
 int  visocu_recon_points(visocu_ctx* ctx, int32_t n_jobs, const visocu_recon_job* jobs, int32_t* const* status,
                          float* const* xyz);
 
+/* ---- device point store: Reconstruction's point list (reconstruction.cpp:41, 146) kept in HBM ----
+ * A store holds one sequence's reconstructed points as float x, y, z (n x 3, packed) in device memory of the context that
+ * created it.  The context owns its stores: visocu_destroy frees those still alive.  A store is not tied to a lane; every
+ * call runs on the context's current lane and waits for its work before it returns.  Growth doubles the capacity.
+ * _append copies n host points behind the stored ones; _read copies points first .. first + count - 1 to the host; both
+ * give VISOCU_EINVAL for a range outside the store or a null pointer.  _points gives the device address and the count;
+ * the address stays valid until the next call that changes the store. */
+typedef struct visocu_recon_store visocu_recon_store;
+int  visocu_recon_store_create(visocu_ctx* ctx, int64_t initial_capacity, visocu_recon_store** out);
+int  visocu_recon_store_destroy(visocu_ctx* ctx, visocu_recon_store* store);
+int  visocu_recon_store_append(visocu_ctx* ctx, visocu_recon_store* store, const float* xyz, int64_t n);
+int  visocu_recon_store_read(visocu_ctx* ctx, const visocu_recon_store* store, int64_t first, int64_t count, float* xyz);
+int  visocu_recon_store_points(const visocu_recon_store* store, const float** d_xyz, int64_t* n);
+/* Reconstruction::update's device half for n_jobs stores (one per sequence): per job j, in this order,
+ *   (a) every point of stores[j] becomes rows 0..2 of tr12[j] (12 doubles, row-major) applied to (p, 1), with the bytes of
+ *       the host's affineTransform (host/reconstruction.cpp);
+ *   (b) jobs[j] is evaluated exactly as visocu_recon_points evaluates it;
+ *   (c) the points with status 0 are appended to stores[j] in track order.
+ * n_kept[j] (optional) = points appended.  status / xyz (optional, each null or n_jobs entries) receive what
+ * visocu_recon_points returns.  Every check of visocu_recon_points, a null store or tr12, a store of another context and a
+ * store named twice give VISOCU_EINVAL before anything is enqueued or written.  If a store cannot grow, the move still runs,
+ * nothing is appended to any store and the call returns VISOCU_ECAPACITY.  One upload, at most three launches (move,
+ * evaluation, append; a stage without work launches nothing) and one read-back; the call waits at the end. */
+int  visocu_recon_update(visocu_ctx* ctx, int32_t n_jobs, visocu_recon_store* const* stores, const double* const* tr12,
+                         const visocu_recon_job* jobs, int32_t* n_kept, int32_t* const* status, float* const* xyz);
+
 /* ---- pose recovery helpers after RANSAC (SURVEY.md 8f rank 2) ----
  * visocu_triangulate: VisualOdometryMono::triangulateChieral (viso_mono.cpp:394-431) for up to four (R|t) candidates
  * at once.  uv: N x 4 floats (u1p,v1p,u1c,v1c) in pixels; P1: 3x4 projection of the previous camera, P2: n_sol 3x4

@@ -230,6 +230,7 @@ extern "C" void visocu_destroy(visocu_ctx* ctx) {
             (unsigned long long)ctx->ro_reason[2], (unsigned long long)ctx->ro_reason[3],
             ctx->ro_declined ? (double)ctx->ro_declined_n / (double)ctx->ro_declined : 0.0);
   }
+  visocu_free_recon_stores(ctx);
   for (int l = 0; l < VISO_LANES; l++)
     if (l == ctx->lane || ctx->lanes[l].created) { if (visocu_use_lane(ctx, l) == VISOCU_OK) free_lane_resources(ctx); }
   free_pool(ctx);

@@ -173,65 +173,96 @@ __global__ void __launch_bounds__(RECON_THREADS) k_recon(const ReconJobDev* __re
 
 }  // namespace
 
+// Shared with recon_store.cu (visocu_recon_update): the checks, the upload image and the launch of k_recon.
+int visocu_recon_check(visocu_ctx* ctx, const char* what, int32_t n_jobs, const visocu_recon_job* jobs, int32_t* const* status,
+                       float* const* xyz, size_t* n_tracks_total, size_t* n_frames_total) {
+  size_t n_total = 0, nf = 0;
+  for (int j = 0; j < n_jobs; j++) {
+    const visocu_recon_job& J = jobs[j];
+    if (J.n_frames < 1 || J.n_frames > MAX_FRAMES || !J.frames || J.n_tracks < 0)
+      return visocu_set_error(ctx, VISOCU_EINVAL, "%s job %d: bad frame table or track count", what, j);
+    if (J.n_tracks > 0 && (!J.tracks || (status && !status[j]) || (xyz && !xyz[j])))
+      return visocu_set_error(ctx, VISOCU_EINVAL, "%s job %d: null pointer", what, j);
+    for (int k = 0; k < J.n_tracks; k++) {
+      const visocu_recon_track& t = J.tracks[k];
+      if (t.n_obs < 2 || t.n_obs > MAX_OBS || t.first < 0 || t.first > J.n_frames - t.n_obs)   // no overflow: n_obs <= 6
+        return visocu_set_error(ctx, VISOCU_EINVAL, "%s job %d track %d: observations outside the window", what, j, k);
+    }
+    n_total += (size_t)J.n_tracks;
+    nf += (size_t)J.n_frames;
+  }
+  if (n_total > (size_t)INT32_MAX / 2) return visocu_set_error(ctx, VISOCU_EINVAL, "%s: too many tracks", what);
+  *n_tracks_total = n_total;
+  *n_frames_total = nf;
+  return VISOCU_OK;
+}
+
+// bytes of k_recon's inputs: job descriptors, frame tables, tracks, each part 256-byte aligned
+size_t visocu_recon_stage_bytes(int32_t n_jobs, size_t n_frames_total, size_t n_tracks_total) {
+  const size_t o_frames = align_up(sizeof(ReconJobDev) * n_jobs, 256);
+  const size_t o_tracks = align_up(o_frames + sizeof(visocu_recon_frame) * n_frames_total, 256);
+  return o_tracks + sizeof(visocu_recon_track) * n_tracks_total;
+}
+
+// writes k_recon's inputs into `pin`, the host image of the device bytes at `dev`; job j's results go to out + its first
+// track.  first_track (n_jobs entries, optional) receives each job's first track.
+void visocu_recon_stage(int32_t n_jobs, const visocu_recon_job* jobs, size_t n_frames_total, uint8_t* pin, uint8_t* dev, int4* out,
+                        int32_t* first_track) {
+  const size_t o_frames = align_up(sizeof(ReconJobDev) * n_jobs, 256);
+  const size_t o_tracks = align_up(o_frames + sizeof(visocu_recon_frame) * n_frames_total, 256);
+  ReconJobDev* hj = (ReconJobDev*)pin;
+  size_t fo = 0, to = 0;
+  for (int j = 0; j < n_jobs; j++) {
+    const visocu_recon_job& J = jobs[j];
+    ReconJobDev& d = hj[j];
+    d.frames = (const visocu_recon_frame*)(dev + o_frames) + fo;
+    d.tracks = (const visocu_recon_track*)(dev + o_tracks) + to;
+    d.out = out + to;
+    memcpy(d.cam_road, J.cam_road, sizeof d.cam_road);
+    d.max_dist = J.max_dist; d.min_angle = J.min_angle;
+    d.first_track = (int)to; d.n_tracks = J.n_tracks; d.point_type = J.point_type; d.n_frames = J.n_frames;
+    if (first_track) first_track[j] = (int32_t)to;
+    memcpy(pin + o_frames + sizeof(visocu_recon_frame) * fo, J.frames, sizeof(visocu_recon_frame) * J.n_frames);
+    if (J.n_tracks) memcpy(pin + o_tracks + sizeof(visocu_recon_track) * to, J.tracks, sizeof(visocu_recon_track) * J.n_tracks);
+    fo += (size_t)J.n_frames; to += (size_t)J.n_tracks;
+  }
+}
+
+int visocu_recon_launch(visocu_ctx* ctx, const uint8_t* dev, int32_t n_jobs, size_t n_tracks_total) {
+  k_recon<<<(unsigned)((n_tracks_total + RECON_THREADS - 1) / RECON_THREADS), RECON_THREADS, 0, ctx->stream>>>(
+      (const ReconJobDev*)dev, n_jobs, (int)n_tracks_total);
+  CU_LAUNCH_CHECK(ctx);
+  return VISOCU_OK;
+}
+
 extern "C" int visocu_recon_points(visocu_ctx* ctx, int32_t n_jobs, const visocu_recon_job* jobs, int32_t* const* status,
                                    float* const* xyz) {
   if (!ctx) return VISOCU_EINVAL;
   if (n_jobs < 0 || (n_jobs > 0 && (!jobs || !status || !xyz))) return visocu_set_error(ctx, VISOCU_EINVAL, "bad recon_points arguments");
   // every job is checked before anything is enqueued or written
   size_t n_total = 0, n_frames_total = 0;
-  for (int j = 0; j < n_jobs; j++) {
-    const visocu_recon_job& J = jobs[j];
-    if (J.n_frames < 1 || J.n_frames > MAX_FRAMES || !J.frames || J.n_tracks < 0)
-      return visocu_set_error(ctx, VISOCU_EINVAL, "recon_points job %d: bad frame table or track count", j);
-    if (J.n_tracks > 0 && (!J.tracks || !status[j] || !xyz[j]))
-      return visocu_set_error(ctx, VISOCU_EINVAL, "recon_points job %d: null pointer", j);
-    for (int k = 0; k < J.n_tracks; k++) {
-      const visocu_recon_track& t = J.tracks[k];
-      if (t.n_obs < 2 || t.n_obs > MAX_OBS || t.first < 0 || t.first > J.n_frames - t.n_obs)   // no overflow: n_obs <= 6
-        return visocu_set_error(ctx, VISOCU_EINVAL, "recon_points job %d track %d: observations outside the window", j, k);
-    }
-    n_total += (size_t)J.n_tracks;
-    n_frames_total += (size_t)J.n_frames;
-  }
+  int rc = visocu_recon_check(ctx, "recon_points", n_jobs, jobs, status, xyz, &n_total, &n_frames_total);
+  if (rc) return rc;
   if (n_total == 0) return VISOCU_OK;
-  if (n_total > (size_t)INT32_MAX / 2) return visocu_set_error(ctx, VISOCU_EINVAL, "recon_points: too many tracks");
   CU_TRY(ctx, cudaSetDevice(ctx->device));
   // Upload: job descriptors, frame tables, tracks (ONE copy).  Read-back: 16 bytes per track (ONE copy).
-  const size_t o_frames = align_up(sizeof(ReconJobDev) * n_jobs, 256);
-  const size_t o_tracks = align_up(o_frames + sizeof(visocu_recon_frame) * n_frames_total, 256);
-  const size_t up_bytes = o_tracks + sizeof(visocu_recon_track) * n_total;
+  const size_t up_bytes = visocu_recon_stage_bytes(n_jobs, n_frames_total, n_total);
   const size_t o_out = align_up(up_bytes, 256);
   const size_t back_bytes = 16 * n_total;
-  int rc = visocu_ensure_scratch(ctx, o_out + back_bytes);
-  if (rc) return rc;
+  if ((rc = visocu_ensure_scratch(ctx, o_out + back_bytes))) return rc;
   if ((rc = visocu_ensure_pinned(ctx, o_out + back_bytes))) return rc;
   uint8_t* sb = (uint8_t*)ctx->scratch;
   uint8_t* pin = (uint8_t*)ctx->pinned;
-  ReconJobDev* hj = (ReconJobDev*)pin;
-  size_t fo = 0, to = 0;
-  for (int j = 0; j < n_jobs; j++) {
-    const visocu_recon_job& J = jobs[j];
-    ReconJobDev& d = hj[j];
-    d.frames = (const visocu_recon_frame*)(sb + o_frames) + fo;
-    d.tracks = (const visocu_recon_track*)(sb + o_tracks) + to;
-    d.out = (int4*)(sb + o_out) + to;
-    memcpy(d.cam_road, J.cam_road, sizeof d.cam_road);
-    d.max_dist = J.max_dist; d.min_angle = J.min_angle;
-    d.first_track = (int)to; d.n_tracks = J.n_tracks; d.point_type = J.point_type; d.n_frames = J.n_frames;
-    memcpy(pin + o_frames + sizeof(visocu_recon_frame) * fo, J.frames, sizeof(visocu_recon_frame) * J.n_frames);
-    if (J.n_tracks) memcpy(pin + o_tracks + sizeof(visocu_recon_track) * to, J.tracks, sizeof(visocu_recon_track) * J.n_tracks);
-    fo += (size_t)J.n_frames; to += (size_t)J.n_tracks;
-  }
+  std::vector<int32_t> first((size_t)n_jobs);
+  visocu_recon_stage(n_jobs, jobs, n_frames_total, pin, sb, (int4*)(sb + o_out), first.data());
   CU_COPY(ctx, sb, pin, up_bytes, cudaMemcpyHostToDevice);
-  k_recon<<<(unsigned)((n_total + RECON_THREADS - 1) / RECON_THREADS), RECON_THREADS, 0, ctx->stream>>>((const ReconJobDev*)sb, n_jobs, (int)n_total);
-  CU_LAUNCH_CHECK(ctx);
+  if ((rc = visocu_recon_launch(ctx, sb, n_jobs, n_total))) return rc;
   CU_COPY(ctx, pin + o_out, sb + o_out, back_bytes, cudaMemcpyDeviceToHost);
   CU_TRY(ctx, visocu_stream_wait(ctx));
   const int32_t* res = (const int32_t*)(pin + o_out);
   for (int j = 0; j < n_jobs; j++) {
-    const int first = hj[j].first_track;
     for (int k = 0; k < jobs[j].n_tracks; k++) {
-      const int32_t* r = res + 4 * (size_t)(first + k);
+      const int32_t* r = res + 4 * (size_t)(first[j] + k);
       status[j][k] = r[0];
       memcpy(xyz[j] + 3 * (size_t)k, r + 1, 12);
     }

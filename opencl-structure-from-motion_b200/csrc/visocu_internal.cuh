@@ -132,6 +132,7 @@ struct visocu_ctx {
   uint64_t h_stats[2] = {0, 0};
   uint64_t ro_node_calls = 0, ro_nodes = 0;   // visocu_delaunay_subtrees: large lists, nodes built for them
   uint64_t ro_ns[4] = {0, 0, 0, 0}, ro_jobs = 0, ro_declined = 0, ro_reason[4] = {0, 0, 0, 0}, ro_declined_n = 0;   // device outlier removal: phase times (VISOCU_RO_STATS)
+  std::vector<visocu_recon_store*> stores;   // device point stores alive on this context (csrc/recon_store.cu)
 };
 
 int visocu_set_error(visocu_ctx* ctx, int code, const char* fmt, ...);
@@ -266,3 +267,11 @@ int visocu_launch_features(visocu_ctx* ctx, const SlotList& sl);
 int visocu_make_tensor_map(visocu_ctx* ctx, size_t frame_stride_bytes);
 void visocu_free_tiles(visocu_ctx* ctx);
 int visocu_make_half_image(visocu_ctx* ctx, int frame);
+// k_recon's checks, upload image and launch (csrc/recon.cu), shared by visocu_recon_points and visocu_recon_update
+int visocu_recon_check(visocu_ctx* ctx, const char* what, int32_t n_jobs, const visocu_recon_job* jobs, int32_t* const* status,
+                       float* const* xyz, size_t* n_tracks_total, size_t* n_frames_total);
+size_t visocu_recon_stage_bytes(int32_t n_jobs, size_t n_frames_total, size_t n_tracks_total);
+void visocu_recon_stage(int32_t n_jobs, const visocu_recon_job* jobs, size_t n_frames_total, uint8_t* pin, uint8_t* dev, int4* out,
+                        int32_t* first_track);
+int visocu_recon_launch(visocu_ctx* ctx, const uint8_t* dev, int32_t n_jobs, size_t n_tracks_total);
+void visocu_free_recon_stores(visocu_ctx* ctx);                // visocu_destroy: the stores still alive

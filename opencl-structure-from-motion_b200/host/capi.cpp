@@ -217,12 +217,18 @@ VISOB_API int visob_recon_get_points(void* r, float* out3, int cap) {
   return (int)pts.size();
 }
 // the two halves of Reconstruction::update around the evaluation of its finished tracks (see reconstruction.h); prepare
-// returns the number of tracks to evaluate
+// returns the number of tracks to evaluate; prepare_tracks is prepare without moving the stored points
 VISOB_API int visob_recon_batch_prepare(void* r, const void* matches, int n, const double* tr16, int point_type, int min_track_length,
                                         double max_dist, double min_angle) {
   const Matcher::p_match* m = (const Matcher::p_match*)matches;
   return ((Reconstruction*)r)->batchPrepare(std::vector<Matcher::p_match>(m, m + n), Matrix(4, 4, tr16), point_type, min_track_length,
                                             max_dist, min_angle).n_tracks;
+}
+VISOB_API int visob_recon_batch_prepare_tracks(void* r, const void* matches, int n, const double* tr16, int point_type,
+                                               int min_track_length, double max_dist, double min_angle) {
+  const Matcher::p_match* m = (const Matcher::p_match*)matches;
+  return ((Reconstruction*)r)->batchPrepareTracks(std::vector<Matcher::p_match>(m, m + n), Matrix(4, 4, tr16), point_type,
+                                                  min_track_length, max_dist, min_angle).n_tracks;
 }
 // the prepared job: its scalar fields into *job (frames / tracks pointing into the object), and copies of the frame table
 // and the tracks into `frames` and `tracks` if they are not null
@@ -272,6 +278,7 @@ VISOB_API void visob_stereo_sfm_get_pose(void* s, double* out16) {
   for (int i = 0; i < 4; i++) for (int j = 0; j < 4; j++) out16[4 * i + j] = T.val[i][j];
 }
 VISOB_API void* visob_stereo_sfm_odometry(void* s) { return &((StructureFromMotionStereo*)s)->odometry(); }
+VISOB_API void visob_stereo_sfm_device_points(void* s, const float** d_xyz, int64_t* n) { ((StructureFromMotionStereo*)s)->devicePoints(d_xyz, n); }
 
 // ---- host utilities exposed for tests
 VISOB_API int visob_delaunay(const int32_t* x, const int32_t* y, int n, int32_t* tri_out, int cap_tri) {
@@ -293,6 +300,14 @@ VISOB_API int visob_delaunay_edges(void* ctx, const int32_t* x, const int32_t* y
   if (edges_out) memcpy(edges_out, e.data(), sizeof(int32_t) * 3 * (size_t)std::min(ne, cap_edges));
   return ne;
 }
+// affineTransform (host/reconstruction.cpp) on n points: M16 row-major 4x4, x, y, z floats per point
+VISOB_API void visob_affine_points(const double* M16, const float* in, float* out, int64_t n) {
+  const Matrix M(4, 4, M16);
+  for (int64_t i = 0; i < n; i++) {
+    const Point3d p = affineTransform(M, Point3d(in[3 * i], in[3 * i + 1], in[3 * i + 2]));
+    out[3 * i] = p.x; out[3 * i + 1] = p.y; out[3 * i + 2] = p.z;
+  }
+}
 VISOB_API void visob_svd(const double* A, int m, int n, double* U, double* W, double* V) {
   Matrix M(m, n, A), Um, Wm, Vm;
   M.svd(Um, Wm, Vm);
@@ -312,7 +327,8 @@ VISOB_API void visob_svd(const double* A, int m, int n, double* U, double* W, do
 // of the worker's sequences evaluated by one device call.
 namespace {
 struct SfmState {                            // what the facades keep besides their odometry object (host/sfm.h)
-  Reconstruction recon;
+  Reconstruction recon;                      // track bookkeeping; the points live in `store`
+  visocu_recon_store* store = nullptr;       // on the worker's context, created by the sequence's first step
   Matrix Tr_total = Matrix::eye(4);
   bool first = true, replace = false;
 };
@@ -331,44 +347,46 @@ struct Runner {
 };
 
 // StructureFromMotion::update (mode 3) or StructureFromMotionStereo::update (mode 4) after the odometry of one frame, for
-// every sequence of worker `tid`: pose accumulation and Reconstruction::batchPrepare for the sequences whose frame is ok,
-// ONE visocu_recon_points for all of them, batchFinish;
-// a failed frame is replaced by the next push.  If the device call fails, the finished tracks of the step are lost and the
-// step reports ok = 0 for those sequences (their pose has already advanced, as the facade's does on a successful frame).
+// every sequence of worker `tid`: pose accumulation and Reconstruction::batchPrepareTracks for the sequences whose frame is
+// ok, then ONE visocu_recon_update for all of them, which moves each sequence's stored points with its motion, evaluates
+// the finished tracks and appends the kept points to the sequence's device store; a failed frame is replaced by the next
+// push.  If the device call fails, the finished tracks of the step are lost and the step reports ok = 0 for those
+// sequences (their pose has already advanced, as the facade's does on a successful frame).
 void runner_sfm(Runner* r, int tid) {
+  visocu_ctx* ctx = r->batches[tid]->context();
   std::vector<int> ids;
   std::vector<visocu_recon_job> jobs;
+  std::vector<visocu_recon_store*> stores;
+  std::vector<double> tr;
   for (int s = tid; s < r->S; s += r->threads) {
     SfmState& q = *r->sfms[s];
     VisualOdometry& vo = r->mode == 4 ? (VisualOdometry&)*r->stereos[s] : (VisualOdometry&)*r->monos[s];
-    if (q.first) { q.first = false; continue; }
+    if (q.first) {
+      q.first = false;
+      if (visocu_recon_store_create(ctx, 0, &q.store) != VISOCU_OK) std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
+      continue;
+    }
     if (!r->last_ok[s]) { q.replace = true; continue; }
-    q.Tr_total = q.Tr_total * Matrix::inv(vo.getMotion());
-    jobs.push_back(q.recon.batchPrepare(vo.getMatches(), vo.getMotion(), 0, 2, 30, 3));
+    const Matrix Tr = vo.getMotion();
+    q.Tr_total = q.Tr_total * Matrix::inv(Tr);
+    jobs.push_back(q.recon.batchPrepareTracks(vo.getMatches(), Tr, 0, 2, 30, 3));
+    for (int i = 0; i < 3; i++) for (int k = 0; k < 4; k++) tr.push_back(Tr.val[i][k]);
+    stores.push_back(q.store);
     ids.push_back(s);
     q.replace = false;
   }
   if (ids.empty()) return;
   const int nj = (int)ids.size();
-  std::vector<std::vector<int32_t> > status(nj);
-  std::vector<std::vector<float> > xyz(nj);
-  std::vector<int32_t*> sp(nj);
-  std::vector<float*> xp(nj);
-  for (int j = 0; j < nj; j++) {
-    status[j].resize((size_t)jobs[j].n_tracks); xyz[j].resize(3 * (size_t)jobs[j].n_tracks);
-    sp[j] = status[j].data(); xp[j] = xyz[j].data();
-  }
-  visocu_ctx* ctx = r->batches[tid]->context();
+  std::vector<const double*> trp(nj);
+  for (int j = 0; j < nj; j++) trp[j] = &tr[12 * (size_t)j];
   visocu_set_lane(ctx, 4);                         // like the odometry calls: matching stays on lane 0
-  const int rc = visocu_recon_points(ctx, nj, jobs.data(), sp.data(), xp.data());
+  const int rc = visocu_recon_update(ctx, nj, stores.data(), trp.data(), jobs.data(), 0, 0, 0);
   visocu_set_lane(ctx, 0);
   if (rc != VISOCU_OK) {
-    // the finished tracks of this step are lost (batchPrepare has dropped them): the step is reported as failed
+    // the finished tracks of this step are lost (batchPrepareTracks has dropped them): the step is reported as failed
     std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
     for (int s : ids) r->last_ok[s] = 0;
-    return;
   }
-  for (int j = 0; j < nj; j++) r->sfms[ids[j]]->recon.batchFinish(sp[j], xp[j]);
 }
 
 // host stages that follow the matching of one frame for every sequence of worker `tid`: bucketing, and for the odometry
@@ -569,8 +587,8 @@ VISOB_API void* visob_runner_create_stereo(int device, int n_sequences, int thre
 // Structure from motion (mode 3): per sequence what StructureFromMotion keeps - a VisualOdometryMono on its sequence of the
 // worker's batch, the accumulated pose, the first-frame and replace flags and a Reconstruction with the facade's calibration
 // and constants (point type 0, min track length 2, 30 m, 3 degrees).  A step pushes every sequence with its replace flag,
-// runs flow matching and the mono odometry stages, and per worker ONE visocu_recon_points for the finished tracks of the
-// sequences whose frame is ok.  Steps are synchronous.
+// runs flow matching and the mono odometry stages, and per worker ONE visocu_recon_update for the sequences whose frame is
+// ok.  Each sequence's points stay in a device store on its worker's context.  Steps are synchronous.
 VISOB_API void* visob_runner_create_sfm(int device, int n_sequences, int threads, const MonoParamsC* p) {
   Runner* r = (Runner*)visob_runner_create(device, n_sequences, threads, 1, 0, p);
   r->mode = 3;
@@ -584,7 +602,7 @@ VISOB_API void* visob_runner_create_sfm(int device, int n_sequences, int threads
 // Stereo structure from motion (mode 4): per sequence a VisualOdometryStereo on its sequence of the worker's batch, as in
 // mode 2, and what StructureFromMotionStereo keeps besides it, as in mode 3.  A step pushes the left and right images of
 // every sequence with its replace flag, runs quad matching with each sequence's previous motion, per worker ONE
-// visocu_stereo_motion and then ONE visocu_recon_points.  Steps are synchronous and need right images.
+// visocu_stereo_motion and then ONE visocu_recon_update.  Steps are synchronous and need right images.
 VISOB_API void* visob_runner_create_stereo_sfm(int device, int n_sequences, int threads, const StereoParamsC* p) {
   Runner* r = (Runner*)visob_runner_create_stereo(device, n_sequences, threads, p);
   r->mode = 4;
@@ -597,7 +615,10 @@ VISOB_API void* visob_runner_create_stereo_sfm(int device, int n_sequences, int 
 }
 VISOB_API void visob_runner_destroy(void* h) {
   Runner* r = (Runner*)h;
-  for (SfmState* q : r->sfms) delete q;
+  for (int s = 0; s < (int)r->sfms.size(); s++) {
+    if (r->sfms[s]->store) visocu_recon_store_destroy(r->batches[s % r->threads]->context(), r->sfms[s]->store);
+    delete r->sfms[s];
+  }
   for (MonoAccess* m : r->monos) delete m;
   for (VisualOdometryStereo* m : r->stereos) delete m;
   for (MatcherBatch* b : r->batches) delete b;
@@ -684,9 +705,26 @@ VISOB_API int visob_runner_get_inliers(void* h, int seq, int32_t* out, int cap) 
 VISOB_API int visob_runner_get_points(void* h, int seq, float* out3, int cap) {
   Runner* r = (Runner*)h;
   if ((r->mode != 3 && r->mode != 4) || seq < 0 || seq >= r->S) return -1;
-  const std::vector<Point3d>& pts = r->sfms[seq]->recon.getPoints();
-  for (int i = 0; i < (int)pts.size() && i < cap; i++) { out3[3 * i] = pts[i].x; out3[3 * i + 1] = pts[i].y; out3[3 * i + 2] = pts[i].z; }
-  return (int)pts.size();
+  const visocu_recon_store* store = r->sfms[seq]->store;
+  if (!store) return 0;
+  const float* d = 0; int64_t n = 0;
+  visocu_recon_store_points(store, &d, &n);
+  const int64_t count = std::min<int64_t>(n, std::max(cap, 0));
+  visocu_ctx* ctx = r->batches[seq % r->threads]->context();
+  if (count > 0 && visocu_recon_store_read(ctx, store, 0, count, out3) != VISOCU_OK) {
+    std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
+    return -1;
+  }
+  return (int)n;
+}
+// the same points in device memory of the runner's GPU (x, y, z floats per point), valid until the next step: 0, or -1 for
+// another mode or a bad sequence; null and 0 before the sequence's first step
+VISOB_API int visob_runner_device_points(void* h, int seq, const float** d_xyz, int64_t* n) {
+  Runner* r = (Runner*)h;
+  if ((r->mode != 3 && r->mode != 4) || seq < 0 || seq >= r->S || !d_xyz || !n) return -1;
+  *d_xyz = 0; *n = 0;
+  if (r->sfms[seq]->store) visocu_recon_store_points(r->sfms[seq]->store, d_xyz, n);
+  return 0;
 }
 VISOB_API void visob_runner_get_pose(void* h, int seq, double* out16) {
   Runner* r = (Runner*)h;

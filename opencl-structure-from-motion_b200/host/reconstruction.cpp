@@ -39,6 +39,11 @@ const visocu_recon_job& Reconstruction::batchPrepare(const vector<Matcher::p_mat
                                                      int32_t min_track_length, double max_dist, double min_angle) {
   // everything already reconstructed moves into the new camera frame
   for (Point3d& p : points) p = affineTransform(Tr, p);
+  return batchPrepareTracks(p_matched, Tr, point_type, min_track_length, max_dist, min_angle);
+}
+
+const visocu_recon_job& Reconstruction::batchPrepareTracks(const vector<Matcher::p_match>& p_matched, Matrix Tr, int32_t point_type,
+                                                           int32_t min_track_length, double max_dist, double min_angle) {
   // frames no live track starts in are dropped from the old end; the rest are re-expressed relative to the new frame
   while (!frames.empty() && frames.front().track_count == 0) frames.pop_front();
   for (Frame& f : frames) {

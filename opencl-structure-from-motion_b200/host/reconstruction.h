@@ -5,7 +5,8 @@
 // Cost: every finished track needs a 4x4 SVD and up to 22 Gauss-Newton updates over as many as 6 observations; with
 // 1 000 - 3 000 matches per frame that is milliseconds per update on one core.  update() runs it on the host; callers with
 // many sequences split it: batchPrepare (the bookkeeping), ONE visocu_recon_points for the finished tracks of all of them
-// (include/visocu.h), batchFinish (SURVEY.md 8f rank 4).
+// (include/visocu.h), batchFinish (SURVEY.md 8f rank 4).  Callers that keep the points in device stores use
+// batchPrepareTracks and ONE visocu_recon_update, which also moves the stored points and appends the kept ones.
 // Own layout: frames carry absolute numbers instead of the reference's frames_ago counters and raw pointers; tracks
 // live in a vector that is compacted in order, which preserves the reference's output order of points.
 #ifndef VISOB_RECONSTRUCTION_H
@@ -45,6 +46,10 @@ public:
   const visocu_recon_job& batchPrepare(const std::vector<Matcher::p_match>& p_matched, Matrix Tr, int32_t point_type = 1,
                                        int32_t min_track_length = 2, double max_dist = 30, double min_angle = 2);
   void batchFinish(const int32_t* status, const float* xyz);
+  // batchPrepare without moving the stored points: for callers that keep the points elsewhere (a device store,
+  // visocu_recon_update) and move them there with Tr.  batchPrepare is the move followed by this.
+  const visocu_recon_job& batchPrepareTracks(const std::vector<Matcher::p_match>& p_matched, Matrix Tr, int32_t point_type = 1,
+                                             int32_t min_track_length = 2, double max_dist = 30, double min_angle = 2);
   const visocu_recon_job& batchJob() const { return job; }
   // the host functions (initPoint, pointType, refinePoint, pointDistance, rayAngle) on every track of the prepared job
   void hostEval(int32_t* status, float* xyz) const;

@@ -12,6 +12,8 @@
 #include "viso_stereo.h"
 #include "visocu.h"
 
+static_assert(sizeof(Point3d) == 12, "a device point store holds packed x, y, z floats");
+
 class StructureFromMotion {
   std::unique_ptr<VisualOdometryMono> viso;
   Reconstruction reconstruction;
@@ -60,13 +62,18 @@ public:
 // Extension (not in the reference): structure from motion on a stereo rig.  update() has StructureFromMotion::update's
 // semantics with VisualOdometryStereo in place of the mono odometry, so the motion is metric (from the baseline) instead of
 // scaled by a ground-plane guess.  Unlike StructureFromMotion, it estimates and reconstructs on the GPU: quad matching with
-// the previous motion, then the batch halves of VisualOdometryStereo and Reconstruction around one single-job
-// visocu_stereo_motion and one single-job visocu_recon_points on the matcher's context.  That is what the sequence
-// runner's stereo structure-from-motion mode (visob_runner_create_stereo_sfm) does for each of its sequences.
+// the previous motion, then the batch halves of VisualOdometryStereo around one single-job visocu_stereo_motion, and
+// Reconstruction::batchPrepareTracks with one single-job visocu_recon_update on the matcher's context.  The points live in
+// a device store (visocu_recon_store): they are moved and appended there, and the host never touches the cloud.  That is
+// what the sequence runner's stereo structure-from-motion mode (visob_runner_create_stereo_sfm) does for each of its
+// sequences.
 class StructureFromMotionStereo {
   std::unique_ptr<VisualOdometryStereo> viso;
   VisualOdometryStereo::parameters param;
   Reconstruction reconstruction;
+  visocu_recon_store* store = nullptr;   // the points, on the matcher's context (created by the first reconstruct)
+  std::vector<Point3d> points;           // host mirror of the store, refreshed by getPoints after an update
+  bool points_stale = false;
   bool replace = false;
   bool is_first_frame = true;
   bool verbose = true;
@@ -89,19 +96,24 @@ class StructureFromMotionStereo {
     return viso->batchFinish(tr, ok, mp);
   }
 
-  // Reconstruction::update with the facade's constants, the finished tracks evaluated on the device.  If the device call
-  // fails, the finished tracks of this frame are lost (batchPrepare has dropped them) and the frame is reported as failed.
+  // Reconstruction::update with the facade's constants, on the device: the stored points move with the motion, the
+  // finished tracks are evaluated and the kept points appended.  If the device call fails, the finished tracks of this
+  // frame are lost (batchPrepareTracks has dropped them) and the frame is reported as failed.
   bool reconstruct(visocu_ctx* ctx) {
-    const visocu_recon_job& job = reconstruction.batchPrepare(viso->getMatches(), viso->getMotion(), 0, 2, 30, 3);
-    std::vector<int32_t> status((size_t)job.n_tracks);
-    std::vector<float> xyz(3 * (size_t)job.n_tracks);
-    int32_t* sp = status.data();
-    float* xp = xyz.data();
-    if (visocu_recon_points(ctx, 1, &job, &sp, &xp) != VISOCU_OK) {
+    if (!store && visocu_recon_store_create(ctx, 0, &store) != VISOCU_OK) {
       std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
       return false;
     }
-    reconstruction.batchFinish(sp, xp);
+    const Matrix Tr = viso->getMotion();
+    const visocu_recon_job& job = reconstruction.batchPrepareTracks(viso->getMatches(), Tr, 0, 2, 30, 3);
+    double tr[12];
+    for (int r = 0; r < 3; r++) for (int c = 0; c < 4; c++) tr[4 * r + c] = Tr.val[r][c];
+    const double* trp = tr;
+    points_stale = true;
+    if (visocu_recon_update(ctx, 1, &store, &trp, &job, 0, 0, 0) != VISOCU_OK) {
+      std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
+      return false;
+    }
     return true;
   }
 
@@ -110,6 +122,11 @@ public:
       : viso(new VisualOdometryStereo(params)), param(params), dims(dims_) {
     reconstruction.setCalibration(params.calib.f, params.calib.cu, params.calib.cv);
   }
+  ~StructureFromMotionStereo() {
+    if (store) visocu_recon_store_destroy(viso->getMatcher()->context(), store);
+  }
+  StructureFromMotionStereo(const StructureFromMotionStereo&) = delete;
+  StructureFromMotionStereo& operator=(const StructureFromMotionStereo&) = delete;
 
   void setVerbose(bool on) { verbose = on; }
 
@@ -139,7 +156,27 @@ public:
     return ok;
   }
 
-  const std::vector<Point3d>& getPoints() { return reconstruction.getPoints(); }
+  // points of all finished tracks, in current camera coordinates: a host copy of the device store
+  const std::vector<Point3d>& getPoints() {
+    if (points_stale) {
+      const float* d = 0; int64_t n = 0;
+      visocu_recon_store_points(store, &d, &n);
+      points.resize((size_t)n);
+      visocu_ctx* ctx = viso->getMatcher()->context();
+      if (visocu_recon_store_read(ctx, store, 0, n, (float*)points.data()) != VISOCU_OK) {
+        std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
+        points.clear();
+      }
+      points_stale = false;
+    }
+    return points;
+  }
+  // the same points in device memory (x, y, z floats per point), valid until the next update; null and 0 before the
+  // first reconstruction
+  void devicePoints(const float** d_xyz, int64_t* n) const {
+    *d_xyz = 0; *n = 0;
+    if (store) visocu_recon_store_points(store, d_xyz, n);
+  }
   const Matrix& getPose() const { return Tr_total; }
   VisualOdometryStereo& odometry() { return *viso; }
 };

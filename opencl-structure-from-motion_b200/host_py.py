@@ -297,6 +297,13 @@ class Recon:
         return lib().visob_recon_batch_prepare(self.h, _p(m), len(m), _p(tr), int(point_type), int(min_track_length),
                                                C.c_double(max_dist), C.c_double(min_angle))
 
+    def batch_prepare_tracks(self, matches, tr, point_type=1, min_track_length=2, max_dist=30.0, min_angle=2.0):
+        """batch_prepare without moving the stored points (for points kept in a device store, visocu_py.Context.recon_update);
+        returns the number of finished tracks to evaluate."""
+        m = np.ascontiguousarray(matches, P_MATCH); tr = np.ascontiguousarray(tr, np.float64)
+        return lib().visob_recon_batch_prepare_tracks(self.h, _p(m), len(m), _p(tr), int(point_type), int(min_track_length),
+                                                      C.c_double(max_dist), C.c_double(min_angle))
+
     def batch_job(self):
         """The prepared job as a dict (frames, tracks, cam_road, max_dist, min_angle, point_type), copied out."""
         job = ReconJob()
@@ -390,6 +397,38 @@ class StereoSfm:
     def odometry(self):
         """The facade's VisualOdometryStereo (matches, inliers, motion of the last frame) as a Stereo view."""
         return Stereo(self.params, handle=lib().visob_stereo_sfm_odometry(self.h), owner=self)
+
+    def device_points(self):
+        """(device address, count) of the points in the facade's device store, valid until the next update."""
+        d = C.c_void_p(); n = C.c_int64()
+        lib().visob_stereo_sfm_device_points(self.h, C.byref(d), C.byref(n))
+        return d.value or 0, n.value
+
+    def points_tensor(self):
+        """The points as a float32 CUDA tensor (n x 3) of its own (a copy of the device store)."""
+        return _points_tensor(*self.device_points())
+
+
+class _DevicePoints:
+    """A borrowed view of n x 3 device floats for torch (__cuda_array_interface__)."""
+
+    def __init__(self, ptr, n):
+        self.__cuda_array_interface__ = dict(shape=(n, 3), typestr='<f4', data=(ptr, False), version=3, strides=None)
+
+
+def _points_tensor(ptr, n):
+    import torch
+    if n == 0:
+        return torch.zeros((0, 3), dtype=torch.float32, device='cuda')
+    return torch.as_tensor(_DevicePoints(ptr, n), device='cuda').clone()
+
+
+def affine_points(M, xyz):
+    """Reconstruction's affineTransform (host/reconstruction.cpp) on every point: rows 0..2 of the 4x4 M applied to (p, 1)."""
+    M = np.ascontiguousarray(M, np.float64); a = np.ascontiguousarray(xyz, np.float32).reshape(-1, 3)
+    out = np.zeros_like(a)
+    lib().visob_affine_points(_p(M), _p(a), _p(out), C.c_int64(len(a)))
+    return out
 
 
 def set_pipeline_depth(depth):
@@ -520,6 +559,18 @@ class Runner:
         if n > 0:
             lib().visob_runner_get_points(self.h, seq, _p(out), n)
         return out
+
+    def device_points(self, seq):
+        """(device address, count) of the sequence's points in its device store (structure-from-motion modes), valid
+        until the next step."""
+        d = C.c_void_p(); n = C.c_int64()
+        if lib().visob_runner_device_points(self.h, seq, C.byref(d), C.byref(n)):
+            raise VisocuError('device_points: not a structure-from-motion runner, or no sequence %d' % seq)
+        return d.value or 0, n.value
+
+    def points_tensor(self, seq):
+        """The sequence's points as a float32 CUDA tensor (n x 3) on the runner's device, a copy of its own."""
+        return _points_tensor(*self.device_points(seq))
 
     def pose(self, seq):
         """The sequence's accumulated pose, first camera -> current camera (structure-from-motion modes)."""

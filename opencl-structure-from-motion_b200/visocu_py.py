@@ -322,13 +322,12 @@ class Context:
                      tr_all=trall[j] if want_all else None) for j in range(nj)]
 
     # ---- reconstruction
-    def recon_points(self, jobs):
-        """visocu_recon_points for a list of jobs, each a dict with frames (RECON_FRAME array), tracks (RECON_TRACK array),
-        cam_road (12), max_dist, min_angle and point_type (host_py.Recon.batch_job makes them).  Returns one
-        (status int32 array, xyz float32 n x 3 array) per job."""
+    @staticmethod
+    def _job_array(jobs):
+        """ReconJob array of job dicts (host_py.Recon.batch_job makes them), and the arrays it points into."""
         nj = len(jobs)
         arr = (ReconJob * max(nj, 1))()
-        keep, status, xyz = [], [], []
+        keep = []
         for j, job in enumerate(jobs):
             fr = np.ascontiguousarray(job['frames'], RECON_FRAME); tr = np.ascontiguousarray(job['tracks'], RECON_TRACK)
             keep += [fr, tr]
@@ -336,8 +335,76 @@ class Context:
             a.frames, a.n_frames, a.tracks, a.n_tracks = fr.ctypes.data, len(fr), tr.ctypes.data, len(tr)
             a.cam_road[:] = [float(x) for x in np.ravel(job['cam_road'])]
             a.max_dist, a.min_angle, a.point_type = job['max_dist'], job['min_angle'], int(job['point_type'])
-            status.append(np.zeros(len(tr), np.int32)); xyz.append(np.zeros((len(tr), 3), np.float32))
+        return arr, keep
+
+    def recon_points(self, jobs):
+        """visocu_recon_points for a list of jobs, each a dict with frames (RECON_FRAME array), tracks (RECON_TRACK array),
+        cam_road (12), max_dist, min_angle and point_type (host_py.Recon.batch_job makes them).  Returns one
+        (status int32 array, xyz float32 n x 3 array) per job."""
+        nj = len(jobs)
+        arr, keep = self._job_array(jobs)
+        status = [np.zeros(arr[j].n_tracks, np.int32) for j in range(nj)]
+        xyz = [np.zeros((arr[j].n_tracks, 3), np.float32) for j in range(nj)]
         sp = (C.c_void_p * max(nj, 1))(*[x.ctypes.data for x in status])
         xp = (C.c_void_p * max(nj, 1))(*[x.ctypes.data for x in xyz])
         self._ck(lib().visocu_recon_points(self.h, nj, arr, sp, xp), 'recon_points')
         return list(zip(status, xyz))
+
+    def recon_store(self, initial_capacity=0):
+        """A device point store on this context (visocu_recon_store)."""
+        return ReconStore(self, initial_capacity)
+
+    def recon_update(self, stores, trs, jobs, want_status=False):
+        """visocu_recon_update: per job j, the points of stores[j] move with trs[j] (4x4, or rows 0..2), jobs[j] (a dict
+        as for recon_points) is evaluated and its kept points are appended to stores[j].  Returns the kept counts (int32
+        array), and with want_status also one (status, xyz) per job as recon_points returns them."""
+        nj = len(jobs)
+        arr, keep = self._job_array(jobs)
+        t = [np.ascontiguousarray(np.asarray(x, np.float64)[:3, :4]) for x in trs]
+        tp = (C.c_void_p * max(nj, 1))(*[x.ctypes.data for x in t])
+        sp = (C.c_void_p * max(nj, 1))(*[s.h.value for s in stores])
+        kept = np.zeros(nj, np.int32)
+        status = xyz = None
+        if want_status:
+            status = [np.zeros(arr[j].n_tracks, np.int32) for j in range(nj)]
+            xyz = [np.zeros((arr[j].n_tracks, 3), np.float32) for j in range(nj)]
+        mk = lambda lst: None if lst is None else (C.c_void_p * max(nj, 1))(*[x.ctypes.data for x in lst])
+        self._ck(lib().visocu_recon_update(self.h, nj, sp, tp, arr, _p(kept), mk(status), mk(xyz)), 'recon_update')
+        return (kept, list(zip(status, xyz))) if want_status else kept
+
+
+class ReconStore:
+    """One sequence's reconstructed points (float x, y, z) in device memory of a Context (visocu_recon_store_*)."""
+
+    def __init__(self, ctx, initial_capacity=0):
+        self.ctx = ctx
+        self.h = C.c_void_p()
+        ctx._ck(lib().visocu_recon_store_create(ctx.h, C.c_int64(int(initial_capacity)), C.byref(self.h)), 'recon_store_create')
+
+    def close(self):
+        if self.h.value and self.ctx.h.value:
+            self.ctx._ck(lib().visocu_recon_store_destroy(self.ctx.h, self.h), 'recon_store_destroy')
+        self.h = C.c_void_p()
+
+    def device_pointer(self):
+        """(device address, point count); the address stays valid until the next call that changes the store."""
+        d = C.c_void_p(); n = C.c_int64()
+        if lib().visocu_recon_store_points(self.h, C.byref(d), C.byref(n)):
+            raise VisocuError('recon_store_points: no store')
+        return d.value or 0, n.value
+
+    @property
+    def count(self):
+        return self.device_pointer()[1]
+
+    def append(self, xyz):
+        a = np.ascontiguousarray(xyz, np.float32).reshape(-1, 3)
+        self.ctx._ck(lib().visocu_recon_store_append(self.ctx.h, self.h, _p(a), C.c_int64(len(a))), 'recon_store_append')
+
+    def read(self, first=0, count=None):
+        n = self.count
+        count = n - first if count is None else count
+        out = np.zeros((max(count, 0), 3), np.float32)
+        self.ctx._ck(lib().visocu_recon_store_read(self.ctx.h, self.h, C.c_int64(first), C.c_int64(count), _p(out)),
+                     'recon_store_read')
+        return out
