@@ -95,6 +95,11 @@ int  visocu_get_features(visocu_ctx* ctx, int32_t frame, int32_t pass, int32_t* 
 /* planes for parity checks / getGain: which = 0 du, 1 dv (matching resolution), 2 du_full, 3 dv_full,
  * 4 padded input image, 5 half-resolution image.  dims3 = {w, h, bpl} of that plane. */
 int  visocu_get_plane(visocu_ctx* ctx, int32_t frame, int32_t which, uint8_t* out, size_t cap, int32_t* dims3);
+/* The tile configurations of the fused filter + NMS kernel that visocu_configure built, largest first (at most 3):
+ * out5[5 k .. 5 k + 4] = {kx, ky, ntx, nty, threads} of level k (kx x ky cells of the aligning NMS pass per tile, ntx x nty
+ * tiles per frame, threads per CTA).  *pick = the level a launch of n_launch frames (1..128) runs on.  For tests and
+ * tuning: which tiles run depends on how many frames one push launch carries. */
+int  visocu_tile_levels(const visocu_ctx* ctx, int32_t n_launch, int32_t* n_levels, int32_t* out5, int32_t* pick);
 
 /* ---- filter:: functions (viso/filter.h:78-94), host buffers in and out, same argument order ---- */
 int  visocu_sobel5x5(visocu_ctx* ctx, const uint8_t* in, uint8_t* out_v, uint8_t* out_h, int32_t w, int32_t h);

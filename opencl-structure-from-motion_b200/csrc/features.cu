@@ -574,6 +574,7 @@ k_filter_nms(const __grid_constant__ Geometry g, const FrameDev* frames, const _
     const int fx0 = 2 * x_ilo;                              // full-resolution column of staging byte 0
     const int xr = t.nbox == 2 ? 2 * IS - BW : 0;           // first column of the right box, relative to fx0
     const uint32_t part_bytes = (uint32_t)(t.nbox * BW * SR);   // one staging buffer; two of them alternate
+    const uint32_t part_stride = (part_bytes + 127u) & ~127u;   // TMA destinations are 128-byte aligned
     if (tid == 0) {
       asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(bar));
       asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(bar + 8));
@@ -582,7 +583,7 @@ k_filter_nms(const __grid_constant__ Geometry g, const FrameDev* frames, const _
     __syncthreads();
     // part p goes to buffer p & 1 and signals mbarrier p & 1; the load of part p + 1 is in flight while part p is worked on
     auto load_part = [&](int p) {
-      const uint32_t dst = stage0 + (uint32_t)(p & 1) * part_bytes, b = bar + 8u * (uint32_t)(p & 1);
+      const uint32_t dst = stage0 + (uint32_t)(p & 1) * part_stride, b = bar + 8u * (uint32_t)(p & 1);
       const int fy = 2 * (y_ilo + p * t.HP) - 2;
       asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(b), "r"(part_bytes) : "memory");
       asm volatile(
@@ -597,7 +598,7 @@ k_filter_nms(const __grid_constant__ Geometry g, const FrameDev* frames, const _
     for (int p = 0; p < t.P; p++) {
       const int hr0 = p * t.HP, hr1 = min(hr0 + t.HP, IH);  // half-resolution rows of the image tile formed by this part
       const int fy0 = 2 * (y_ilo + hr0) - 2;                // first staged full-resolution row
-      const uint32_t stage = stage0 + (uint32_t)(p & 1) * part_bytes;
+      const uint32_t stage = stage0 + (uint32_t)(p & 1) * part_stride;
       const uint32_t right = stage + (uint32_t)(BW * SR) - (uint32_t)xr;
       mbar_wait_or_trap(bar + 8u * (uint32_t)(p & 1), (uint32_t)((p >> 1) & 1));
       // full-resolution Sobel rows of this part
@@ -1035,11 +1036,14 @@ bool make_tile_cfg(const Geometry& g, int kx, int ky, int threads, bool fused, T
     t.nbox = 2 * t.IS > 256 ? 2 : 1;
     t.BW = t.nbox == 2 ? 256 : 2 * t.IS;
     const int rows_fit = (int)(t.f_bytes / (unsigned)(2 * t.nbox * t.BW));     // two staging buffers
-    int hp = std::min((rows_fit - 4) / 2, 126);
-    if (hp < 4) return false;
+    // at least 4 half-resolution rows per part: the response plane area of a small tile is enlarged to hold them
+    const int hp = std::max(std::min((rows_fit - 4) / 2, 126), 4);
     t.P = (t.IH + hp - 1) / hp;
     t.HP = (t.IH + t.P - 1) / t.P;
     t.SR = 2 * t.HP + 4;
+    // the second buffer starts on the next 128-byte boundary (a TMA destination must be 128-byte aligned)
+    t.f_bytes = std::max(t.f_bytes, 2 * (unsigned)align_up((size_t)t.nbox * t.BW * t.SR, 128));
+    t.smem = t.img_bytes + t.f_bytes + 16 + 32 + (unsigned)t.max_cells * 4 + 16;
     int nwF_max = 1;
     for (int a = 0; a < t.ntx; a++) {
       AxisTile& X = xt[a];
@@ -1160,6 +1164,27 @@ int visocu_make_half_image(visocu_ctx* ctx, int frame) {
   return VISOCU_OK;
 }
 
+// the largest tiles that still give a launch of n frames about one CTA per SM; else the smallest
+static int pick_tile_level(const visocu_ctx* ctx, int n) {
+  for (int c = 0; c < ctx->n_tiles; c++) {
+    TileCfg t; memcpy(&t, ctx->tiles[c].cfg, sizeof t);
+    if ((long long)t.ntx * t.nty * n >= ctx->sm_count) return c;
+  }
+  return ctx->n_tiles - 1;
+}
+
+extern "C" int visocu_tile_levels(const visocu_ctx* ctx, int32_t n_launch, int32_t* n_levels, int32_t* out5, int32_t* pick) {
+  if (!ctx || !ctx->configured || n_launch < 1 || n_launch > VISO_MAX_BATCH) return VISOCU_EINVAL;
+  if (n_levels) *n_levels = ctx->n_tiles;
+  for (int c = 0; c < ctx->n_tiles && out5; c++) {
+    TileCfg t; memcpy(&t, ctx->tiles[c].cfg, sizeof t);
+    const int32_t v[5] = {t.kx, t.ky, t.ntx, t.nty, t.threads};
+    memcpy(out5 + 5 * c, v, sizeof v);
+  }
+  if (pick) *pick = pick_tile_level(ctx, n_launch);
+  return VISOCU_OK;
+}
+
 int visocu_launch_features(visocu_ctx* ctx, const SlotList& sl) {
   const Geometry& g = ctx->g;
   cudaStream_t st = ctx->stream;
@@ -1172,12 +1197,7 @@ int visocu_launch_features(visocu_ctx* ctx, const SlotList& sl) {
     CU_LAUNCH_CHECK(ctx);
   }
   {
-    // the largest tiles that still give the launch about one CTA per SM; else the smallest
-    int pick = ctx->n_tiles - 1;
-    for (int c = 0; c < ctx->n_tiles; c++) {
-      TileCfg t; memcpy(&t, ctx->tiles[c].cfg, sizeof t);
-      if ((long long)t.ntx * t.nty * sl.n >= ctx->sm_count) { pick = c; break; }
-    }
+    const int pick = pick_tile_level(ctx, sl.n);
     TileCfg t; memcpy(&t, ctx->tiles[pick].cfg, sizeof t);
     // opt in to large dynamic shared memory once per device (the attribute belongs to the function on a device, not
     // to a context: several contexts with different tile shapes share it)

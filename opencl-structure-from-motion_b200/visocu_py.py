@@ -181,6 +181,14 @@ class Context:
         self._ck(lib().visocu_get_plane(self.h, frame, which, _p(out), C.c_size_t(out.nbytes), _p(dims)), 'get_plane')
         return out, (w, h, bpl)
 
+    def tile_levels(self, n_launch=1):
+        """(levels, pick): the fused filter + NMS kernel's tile configurations, largest first, as dicts (kx, ky, ntx, nty,
+        threads), and the level a push launch of n_launch frames runs on."""
+        n = C.c_int32(); out = np.zeros(15, np.int32); pick = C.c_int32()
+        self._ck(lib().visocu_tile_levels(self.h, int(n_launch), C.byref(n), _p(out), C.byref(pick)), 'tile_levels')
+        keys = ('kx', 'ky', 'ntx', 'nty', 'threads')
+        return [dict(zip(keys, out[5 * k:5 * k + 5].tolist())) for k in range(n.value)], pick.value
+
     # ---- filters
     def sobel5x5(self, img):
         img = np.ascontiguousarray(img, np.uint8); h, w = img.shape
