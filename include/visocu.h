@@ -101,6 +101,27 @@ int  visocu_get_plane(visocu_ctx* ctx, int32_t frame, int32_t which, uint8_t* ou
  * tuning: which tiles run depends on how many frames one push launch carries. */
 int  visocu_tile_levels(const visocu_ctx* ctx, int32_t n_launch, int32_t* n_levels, int32_t* out5, int32_t* pick);
 
+/* ---- rectification of raw camera images (not in the reference, which expects undistorted, rectified images) ----
+ * A camera: raw pinhole K = (fx, fy, cx, cy), radial-tangential distortion k1, k2, p1, p2, k3 (OpenCV's and KITTI's model),
+ * the rectifying rotation R (raw camera -> rectified coordinates, row-major) and the rectified projection f, cu, cv.
+ * visocu_set_rectification builds one map per camera for raw images of src_w x src_h and the configured (output) size: the
+ * output pixel (u, v) samples the raw image at the distorted projection of the ray R^T ((u - cu) / f, (v - cv) / f, 1),
+ * in 1/32 pixel and clamped to the raw image (the border is replicated); host/rectify.h states it exactly.  At most 2
+ * cameras; n_cams = 0 removes the maps; visocu_configure removes them as well.  VISOCU_EINVAL, before anything changes, for
+ * a non-finite parameter, fx, fy or f <= 0, src_w or src_h outside [16, 8191] or an output pixel whose rotated ray has
+ * z <= 0; VISOCU_ESTATE on a context that is not configured.
+ * visocu_push_frames_rectified is visocu_push_frames for raw images (bpl_in >= src_w): image k is resampled with map cam[k]
+ * into its frame (bilinear in 1/32 pixel, integer arithmetic: ((32-fx)(32-fy) p00 + fx(32-fy) p01 + (32-fx) fy p10 +
+ * fx fy p11 + 512) >> 10), then the features are computed as for a plain push.  VISOCU_ESTATE without maps, VISOCU_EINVAL
+ * for a camera index out of range or bpl_in < src_w, both before anything is enqueued.
+ * visocu_get_rectify_map copies map `cam` (2 int32 per output pixel, x then y in 1/32 pixel, row-major) to out; cap in
+ * int32 entries. */
+typedef struct { double fx, fy, cx, cy, k1, k2, p1, p2, k3, R[9], f, cu, cv; } visocu_camera;
+int  visocu_set_rectification(visocu_ctx* ctx, int32_t n_cams, const visocu_camera* cams, int32_t src_w, int32_t src_h);
+int  visocu_push_frames_rectified(visocu_ctx* ctx, int32_t n, const int32_t* frames, const uint8_t* const* imgs, const int32_t* cam,
+                                  int32_t bpl_in, int32_t on_device, int32_t* n_sparse, int32_t* n_dense);
+int  visocu_get_rectify_map(visocu_ctx* ctx, int32_t cam, int32_t* out, size_t cap);
+
 /* ---- filter:: functions (viso/filter.h:78-94), host buffers in and out, same argument order ---- */
 int  visocu_sobel5x5(visocu_ctx* ctx, const uint8_t* in, uint8_t* out_v, uint8_t* out_h, int32_t w, int32_t h);
 int  visocu_sobel3x3(visocu_ctx* ctx, const uint8_t* in, uint8_t* out_v, uint8_t* out_h, int32_t w, int32_t h);

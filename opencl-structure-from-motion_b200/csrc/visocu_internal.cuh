@@ -133,6 +133,10 @@ struct visocu_ctx {
   uint64_t ro_node_calls = 0, ro_nodes = 0;   // visocu_delaunay_subtrees: large lists, nodes built for them
   uint64_t ro_ns[4] = {0, 0, 0, 0}, ro_jobs = 0, ro_declined = 0, ro_reason[4] = {0, 0, 0, 0}, ro_declined_n = 0;   // device outlier removal: phase times (VISOCU_RO_STATS)
   std::vector<visocu_recon_store*> stores;   // device point stores alive on this context (csrc/recon_store.cu)
+  // rectification maps (csrc/rectify.cu): per camera 2 int32 per output pixel, on the device and a host copy
+  int rect_n = 0, rect_src_w = 0, rect_src_h = 0;
+  int2* rect_map[2] = {nullptr, nullptr};
+  std::vector<int32_t> rect_host[2];
 };
 
 int visocu_set_error(visocu_ctx* ctx, int code, const char* fmt, ...);
@@ -275,3 +279,7 @@ void visocu_recon_stage(int32_t n_jobs, const visocu_recon_job* jobs, size_t n_f
                         int32_t* first_track);
 int visocu_recon_launch(visocu_ctx* ctx, const uint8_t* dev, int32_t n_jobs, size_t n_tracks_total);
 void visocu_free_recon_stores(visocu_ctx* ctx);                // visocu_destroy: the stores still alive
+// csrc/rectify.cu: the maps go with visocu_configure and visocu_destroy; the gather kernel replaces k_repitch in a push
+struct CamList { int32_t c[VISO_MAX_BATCH]; };
+void visocu_free_rectification(visocu_ctx* ctx);
+void visocu_launch_rectify(visocu_ctx* ctx, const SlotList& sl, const CamList& cams, int bpl_in);

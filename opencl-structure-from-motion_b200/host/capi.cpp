@@ -17,6 +17,7 @@
 #include "viso_mono.h"
 #include "viso_stereo.h"
 #include "reconstruction.h"
+#include "rectify.h"
 #include "sfm.h"
 #include "visocu.h"
 
@@ -280,6 +281,29 @@ VISOB_API void visob_stereo_sfm_get_pose(void* s, double* out16) {
 VISOB_API void* visob_stereo_sfm_odometry(void* s) { return &((StructureFromMotionStereo*)s)->odometry(); }
 VISOB_API void visob_stereo_sfm_device_points(void* s, const float** d_xyz, int64_t* n) { ((StructureFromMotionStereo*)s)->devicePoints(d_xyz, n); }
 
+// ---- rectification (host/rectify.h): setRectification of the classes above, 1 = done, 0 = refused
+VISOB_API int visob_matcher_set_rectification(void* m, const Rectification* r) { return ((Matcher*)m)->setRectification(*r) ? 1 : 0; }
+VISOB_API int visob_mono_set_rectification(void* v, const Rectification* r) { return ((MonoAccess*)v)->setRectification(*r) ? 1 : 0; }
+VISOB_API int visob_stereo_set_rectification(void* v, const Rectification* r) { return ((VisualOdometryStereo*)v)->setRectification(*r) ? 1 : 0; }
+VISOB_API int visob_sfm_set_rectification(void* s, const Rectification* r) { return ((StructureFromMotion*)s)->setRectification(*r) ? 1 : 0; }
+VISOB_API int visob_stereo_sfm_set_rectification(void* s, const Rectification* r) {
+  return ((StructureFromMotionStereo*)s)->setRectification(*r) ? 1 : 0;
+}
+VISOB_API void visob_stereo_rectify(const visocu_camera* cam0, const visocu_camera* cam1, const double* R9, const double* T3, int32_t out_w,
+                                    int32_t out_h, visocu_camera* rect0, visocu_camera* rect1, double* base) {
+  visob::stereoRectify(*cam0, *cam1, R9, T3, out_w, out_h, rect0, rect1, base);
+}
+// the map visocu_set_rectification builds, computed on the host (no device needed): 0, or VISOCU_EINVAL with the reason
+// in why (256 bytes, optional)
+VISOB_API int visob_rectify_map(const visocu_camera* cam, int32_t src_w, int32_t src_h, int32_t out_w, int32_t out_h, int32_t* out,
+                                char* why256) {
+  const char* why = "";
+  const bool ok = visob::rectifyCheck(*cam, src_w, src_h, out_w, out_h, &why) &&
+                  (!out || visob::rectifyMap(*cam, src_w, src_h, out_w, out_h, out, &why));
+  if (why256) snprintf(why256, 256, "%s", ok ? "" : why);
+  return ok ? VISOCU_OK : VISOCU_EINVAL;
+}
+
 // ---- host utilities exposed for tests
 VISOB_API int visob_delaunay(const int32_t* x, const int32_t* y, int n, int32_t* tri_out, int cap_tri) {
   std::vector<int32_t> tri;
@@ -343,6 +367,7 @@ struct Runner {
   std::vector<VisualOdometryStereo*> stereos; // one per sequence (modes 2 and 4)
   std::vector<SfmState*> sfms;               // one per sequence (modes 3 and 4)
   std::vector<int32_t> last_matches, last_ok;
+  bool started = false;                      // a step has run: the rectification is fixed
   Matcher& matcher_of(int seq) { return batches[seq % threads]->sequence(seq / threads); }
 };
 
@@ -627,10 +652,30 @@ VISOB_API void visob_runner_destroy(void* h) {
 // imgs / imgs2: S pointers (imgs2 may be null for mono / flow).  on_device: pointers are device memory.
 // bucket: apply bucketFeatures after matching (mode 0).  Returns wall seconds spent in the step; -1 for a mode-4 step
 // without right images (nothing is pushed or written).
+// Raw camera images for every mode: what setRectification does for each sequence's objects (MatcherBatch, the odometry's
+// calibration, the reconstruction's projection).  Stereo modes (2, 4) need r->n_cams = 2.  1 = done; 0 = refused, with
+// nothing changed: after the first step, or a rectification the mode cannot take.
+VISOB_API int visob_runner_set_rectification(void* h, const Rectification* rc) {
+  Runner* r = (Runner*)h;
+  const bool stereo = r->mode == 2 || r->mode == 4;
+  if (r->started || rc->n_cams < 0 || rc->n_cams > 2 || (stereo && rc->n_cams != 2)) return 0;
+  for (MatcherBatch* b : r->batches) b->setRectification(*rc);
+  for (MonoAccess* m : r->monos) m->setRectification(*rc);
+  for (VisualOdometryStereo* m : r->stereos) m->setRectification(*rc);
+  if (rc->n_cams > 0) {
+    const visocu_camera& c = rc->cams[0];
+    r->params.f = c.f; r->params.cu = c.cu; r->params.cv = c.cv;
+    r->sparams.f = c.f; r->sparams.cu = c.cu; r->sparams.cv = c.cv;
+    if (stereo) r->sparams.base = rc->base;
+    for (SfmState* q : r->sfms) q->recon.setCalibration(c.f, c.cu, c.cv);
+  }
+  return 1;
+}
 VISOB_API double visob_runner_step(void* h, const uint8_t* const* imgs, const uint8_t* const* imgs2, const int32_t* dims,
                                    int on_device, int bucket, int32_t* n_matches_out, int32_t* ok_out) {
   Runner* r = (Runner*)h;
   if (r->mode == 4 && !imgs2) return -1.0;
+  r->started = true;
   auto t0 = std::chrono::steady_clock::now();
   run_workers(r->threads, [&](int tid) {
     visob::set_device(r->device);
@@ -645,6 +690,7 @@ VISOB_API double visob_runner_run(void* h, int n_steps, const uint8_t* const* im
                                   int on_device, int bucket, int32_t* n_matches_out, int32_t* ok_out) {
   Runner* r = (Runner*)h;
   if (r->mode == 4 && !imgs2) return -1.0;
+  r->started = true;
   auto t0 = std::chrono::steady_clock::now();
   run_workers(r->threads, [&](int tid) {
     visob::set_device(r->device);

@@ -63,6 +63,8 @@ Matcher::Matcher(parameters param) : param(param), ctx(0), owns_ctx(true), slot_
   for (int k = 0; k < 4; k++) slot[k] = -1;
   for (int k = 0; k < 8; k++) n_feat[k] = 0;
   for (int k = 0; k < 3; k++) dims_p[k] = dims_c[k] = 0;
+  memset(&rect, 0, sizeof rect);
+  started = false;
   memset(&rnd_data, 0, sizeof rnd_data);
   memset(rnd_state, 0, sizeof rnd_state);
   initstate_r(1, rnd_state, sizeof rnd_state, &rnd_data);     // the state rand() starts from
@@ -121,11 +123,31 @@ bool Matcher::ensureContext(int32_t w, int32_t h) {
       std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
       return false;
     }
+    if (rect.n_cams > 0 && visocu_set_rectification(ctx, rect.n_cams, rect.cams, rect.src_w, rect.src_h) != VISOCU_OK) {
+      std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
+      return false;
+    }
     cfg_w = w; cfg_h = h;
     for (int k = 0; k < 4; k++) slot[k] = -1;        // features of another image size cannot be matched
     for (int k = 0; k < 8; k++) n_feat[k] = 0;
     have_I1p = have_I1c = false;
   }
+  return true;
+}
+
+bool Matcher::setRectification(const Rectification& r) {
+  if (started || r.n_cams < 0 || r.n_cams > 2) return false;
+  rect = r;
+  cfg_w = cfg_h = 0;                                 // the next push configures the context and sets the maps
+  return true;
+}
+
+bool Matcher::rectifiedDims(const uint32_t* dims, uint32_t* out) const {
+  if ((int32_t)dims[0] != rect.src_w || (int32_t)dims[1] != rect.src_h || (int32_t)dims[2] < rect.src_w) {
+    std::cerr << "ERROR: Image dimension mismatch!" << std::endl;
+    return false;
+  }
+  out[0] = (uint32_t)rect.out_w; out[1] = (uint32_t)rect.out_h; out[2] = (uint32_t)rect.out_w;
   return true;
 }
 
@@ -135,14 +157,20 @@ void Matcher::pushBackDevice(const uint8_t* d_I1, const uint8_t* d_I2, uint32_t*
 void Matcher::push(const uint8_t* I1, const uint8_t* I2, uint32_t* dims, bool replace, bool on_device) {
   visob::StageTimer timer(0);
   int32_t frames[2];
-  if (!pushPrepare(I1, I2, dims, replace, frames)) return;
+  uint32_t od[3];
+  const bool rectify = rect.n_cams > 0;
+  if (rectify && !rectifiedDims(dims, od)) return;
+  if (!pushPrepare(I1, I2, rectify ? od : dims, replace, frames)) return;
   const uint8_t* imgs[2] = {I1, I2};
+  const int32_t cams[2] = {0, 1};
   int32_t ns[2] = {-1, -1}, nd[2] = {-1, -1};
   const int nimg = I2 ? 2 : 1;
   // flow matching of a monocular sequence goes through the fused call, which needs no record counts on the host: the
   // push then returns without waiting for the GPU (the counts are fetched lazily if somebody asks, syncCounts)
   const bool lazy = lazyCounts() && !I2;
-  const bool ok = visocu_push_frames(ctx, nimg, frames, imgs, (int32_t)dims[2], on_device ? 1 : 0, lazy ? 0 : ns, lazy ? 0 : nd) == VISOCU_OK;
+  const int32_t bpl = (int32_t)dims[2], where = on_device ? 1 : 0;
+  const bool ok = (rectify ? visocu_push_frames_rectified(ctx, nimg, frames, imgs, cams, bpl, where, lazy ? 0 : ns, lazy ? 0 : nd)
+                           : visocu_push_frames(ctx, nimg, frames, imgs, bpl, where, lazy ? 0 : ns, lazy ? 0 : nd)) == VISOCU_OK;
   if (!ok) std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
   pushFinish(ok, I2 != 0, ns, nd);
 }
@@ -155,6 +183,7 @@ bool Matcher::pushPrepare(const uint8_t* I1, const uint8_t* I2, uint32_t* dims, 
     return false;
   }
   if (!ensureContext(width, height)) return false;
+  started = true;
   if (!replace) {
     // current -> previous: the device frames swap roles, nothing is copied
     std::swap(slot[0], slot[2]);
@@ -532,6 +561,16 @@ void Matcher::removeOutliers(vector<p_match>& p_matched, int32_t method) {
 MatcherBatch::MatcherBatch(Matcher::parameters param, int32_t n_sequences) : k_submit(0), k_collect(0), ctx(0), width(0), height(0) {
   for (int32_t s = 0; s < n_sequences; s++) seq.push_back(new Matcher(param));
   device = visob::current_device();
+  memset(&rect, 0, sizeof rect);
+  started = false;
+}
+
+bool MatcherBatch::setRectification(const Rectification& r) {
+  if (started || r.n_cams < 0 || r.n_cams > 2) return false;
+  for (Matcher* m : seq) m->setRectification(r);     // the sequences check the raw dims and see the rectified ones
+  rect = r;
+  width = height = 0;                                // the next push configures the context and sets the maps
+  return true;
 }
 
 MatcherBatch::~MatcherBatch() {
@@ -552,7 +591,12 @@ bool MatcherBatch::ensure(int32_t w, int32_t h) {
     std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
     return false;
   }
+  if (rect.n_cams > 0 && visocu_set_rectification(ctx, rect.n_cams, rect.cams, rect.src_w, rect.src_h) != VISOCU_OK) {
+    std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
+    return false;
+  }
   width = w; height = h;
+  started = true;
   for (size_t s = 0; s < seq.size(); s++) seq[s]->useSharedContext(ctx, 4 * (int32_t)s, w, h);
   return true;
 }
@@ -565,26 +609,35 @@ void MatcherBatch::pushBack(const uint8_t* const* I1, const uint8_t* const* I2, 
 
 void MatcherBatch::pushBack(const uint8_t* const* I1, const uint8_t* const* I2, uint32_t* dims, const bool* replace, bool on_device) {
   visob::StageTimer timer(0);
-  if ((int32_t)dims[0] <= 0 || (int32_t)dims[1] <= 0 || dims[2] < dims[0]) {
+  uint32_t od[3];
+  const bool rectify = rect.n_cams > 0;
+  if (rectify) {
+    if (!seq[0]->rectifiedDims(dims, od)) return;
+  } else if ((int32_t)dims[0] <= 0 || (int32_t)dims[1] <= 0 || dims[2] < dims[0]) {
     std::cerr << "ERROR: Image dimension mismatch!" << std::endl;
     return;
   }
+  const int32_t bpl = (int32_t)dims[2];
+  if (rectify) dims = od;                            // the sequences see the rectified images
   if (!ensure((int32_t)dims[0], (int32_t)dims[1])) return;
   const size_t S = seq.size();
-  vector<int32_t> frames, owner;
+  vector<int32_t> frames, owner, cams;
   vector<const uint8_t*> imgs;
   for (size_t s = 0; s < S; s++) {
     int32_t f[2];
     const uint8_t* i2 = I2 ? I2[s] : 0;
     if (!seq[s]->pushPrepare(I1[s], i2, dims, replace[s], f)) continue;
-    frames.push_back(f[0]); imgs.push_back(I1[s]); owner.push_back((int32_t)s);
-    if (i2) { frames.push_back(f[1]); imgs.push_back(i2); owner.push_back((int32_t)s); }
+    frames.push_back(f[0]); imgs.push_back(I1[s]); owner.push_back((int32_t)s); cams.push_back(0);
+    if (i2) { frames.push_back(f[1]); imgs.push_back(i2); owner.push_back((int32_t)s); cams.push_back(1); }
   }
   if (frames.empty()) return;
   vector<int32_t> ns(frames.size(), -1), nd(frames.size(), -1);
   const bool lazy = seq[0]->lazyCounts() && !I2;           // see Matcher::push
-  const bool ok = visocu_push_frames(ctx, (int32_t)frames.size(), frames.data(), imgs.data(), (int32_t)dims[2], on_device ? 1 : 0,
-                                     lazy ? 0 : ns.data(), lazy ? 0 : nd.data()) == VISOCU_OK;
+  const int32_t nf = (int32_t)frames.size(), where = on_device ? 1 : 0;
+  const bool ok = (rectify ? visocu_push_frames_rectified(ctx, nf, frames.data(), imgs.data(), cams.data(), bpl, where, lazy ? 0 : ns.data(),
+                                                          lazy ? 0 : nd.data())
+                           : visocu_push_frames(ctx, nf, frames.data(), imgs.data(), bpl, where, lazy ? 0 : ns.data(),
+                                                lazy ? 0 : nd.data())) == VISOCU_OK;
   if (!ok) std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
   for (size_t k = 0; k < frames.size();) {
     const int32_t s = owner[k];
@@ -674,10 +727,16 @@ bool MatcherBatch::stepAvailable(int32_t method) const {
 bool MatcherBatch::stepSubmit(const uint8_t* const* I1, uint32_t* dims, bool on_device) {
   // host images of a step stay valid until the step is collected (the runner's contract): mode 2 of visocu_push_frames
   visob::StageTimer timer(0);
-  if ((int32_t)dims[0] <= 0 || (int32_t)dims[1] <= 0 || dims[2] < dims[0]) {
+  uint32_t od[3];
+  const bool rectify = rect.n_cams > 0;
+  if (rectify) {
+    if (!seq[0]->rectifiedDims(dims, od)) return false;
+  } else if ((int32_t)dims[0] <= 0 || (int32_t)dims[1] <= 0 || dims[2] < dims[0]) {
     std::cerr << "ERROR: Image dimension mismatch!" << std::endl;
     return false;
   }
+  const int32_t bpl = (int32_t)dims[2];
+  if (rectify) dims = od;
   if (!ensure((int32_t)dims[0], (int32_t)dims[1])) return false;
   if (k_submit - k_collect >= 3) return false;                       // the fourth frame of the ring is still being read
   const size_t S = seq.size();
@@ -685,14 +744,16 @@ bool MatcherBatch::stepSubmit(const uint8_t* const* I1, uint32_t* dims, bool on_
   const int lane = (int)(k & 3);
   if (visocu_set_lane(ctx, lane) != VISOCU_OK) { std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl; return false; }
   // frame k of sequence s lives in slot 4 s + (k & 3): four consecutive frames stay alive
-  vector<int32_t> frames(S);
+  vector<int32_t> frames(S), cams(S, 0);
   vector<visocu_quad> quads(S);
   for (size_t s = 0; s < S; s++) {
     frames[s] = 4 * (int32_t)s + lane;
     quads[s] = visocu_quad{4 * (int32_t)s + (int)((k + 3) & 3), -1, frames[s], -1};
     if (!I1[s]) { std::cerr << "ERROR: Image dimension mismatch!" << std::endl; return false; }
   }
-  bool ok = visocu_push_frames(ctx, (int32_t)S, frames.data(), I1, (int32_t)dims[2], on_device ? 1 : 2, 0, 0) == VISOCU_OK;
+  const int32_t where = on_device ? 1 : 2;
+  bool ok = (rectify ? visocu_push_frames_rectified(ctx, (int32_t)S, frames.data(), I1, cams.data(), bpl, where, 0, 0)
+                     : visocu_push_frames(ctx, (int32_t)S, frames.data(), I1, bpl, where, 0, 0)) == VISOCU_OK;
   if (ok && k > 0)
     ok = visocu_match_fused_submit(ctx, (int32_t)S, quads.data(), seq[0]->refineMode(), 0, (int)((k + 3) & 3)) == VISOCU_OK;
   if (!ok) std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;

@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "matrix.h"
+#include "rectify.h"
 #include "visocu.h"
 
 struct visocu_ctx;
@@ -68,6 +69,12 @@ public:
   float getGain(std::vector<int32_t> inliers);
 
   // ---- extensions (not in the reference) ----
+  // Raw camera images: after setRectification(r) with r.n_cams > 0, pushBack and pushBackDevice take images of
+  // r.src_w x r.src_h (bytes per line >= r.src_w) and resample them on the GPU into r.out_w x r.out_h rectified images, the
+  // left one with map 0 and the right one with map 1 (host/rectify.h); everything after the push sees the rectified
+  // images.  r.n_cams = 0 returns to plain pushes.  Allowed before the first push only: afterwards it returns false and
+  // changes nothing (as it does for more than 2 cameras).
+  bool setRectification(const Rectification& r);
   // same as pushBack, but the images already live in device memory of this matcher's GPU
   void pushBackDevice(const uint8_t* d_I1, const uint8_t* d_I2, uint32_t* dims, const bool replace);
   visocu_ctx* context() { return ctx; }
@@ -99,6 +106,8 @@ private:
   void syncCounts();
   int32_t queryCount(int pass, int32_t method) const;
   bool ensureContext(int32_t w, int32_t h);
+  // with rectification: dims must be the raw size (else false, with the reference's message); out = the output dims
+  bool rectifiedDims(const uint32_t* dims, uint32_t* out) const;
   bool fetchImage(int which, std::vector<uint8_t>& out);
   bool matching(int pass, std::vector<p_match>& out, int32_t method, bool use_prior, int refine);
   // both passes of multi-stage flow matching as one submission (visocu_match_fused) for a group of matchers on one context
@@ -114,6 +123,8 @@ private:
   int32_t slot_base;                     // first device frame of this matcher inside its context
   int device;
   int32_t cfg_w, cfg_h;
+  Rectification rect;                    // rect.n_cams = 0: plain pushes
+  bool started;                          // a push has been prepared: the rectification is fixed
   // ring buffer: frame slots of the context.  slot[0] = previous left, [1] = previous right, [2] = current left,
   // [3] = current right (-1 = empty)
   int32_t slot[4];
@@ -154,6 +165,8 @@ public:
   bool stepAvailable(int32_t method) const;
   bool stepSubmit(const uint8_t* const* I1, uint32_t* dims, bool on_device);
   bool stepCollect();
+  // Matcher::setRectification for all sequences (the shared context holds the maps): before the first push or step only
+  bool setRectification(const Rectification& r);
   int32_t stepsInFlight() const { return (int32_t)(k_submit - k_collect); }
   int32_t size() const { return (int32_t)seq.size(); }
   Matcher& sequence(int32_t i) { return *seq[i]; }
@@ -163,6 +176,8 @@ private:
   bool ensure(int32_t w, int32_t h);
   bool matchPass(const std::vector<int32_t>& active, int pass, int32_t method, bool use_prior, int refine);
   int32_t step_dims[3];
+  Rectification rect;
+  bool started;
   int64_t k_submit, k_collect;                          // steps submitted / collected so far (stepSubmit / stepCollect)
   std::vector<Matcher*> seq;
   visocu_ctx* ctx;

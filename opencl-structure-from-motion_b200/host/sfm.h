@@ -32,6 +32,15 @@ public:
 
   void setVerbose(bool on) { verbose = on; }     // the reference always prints; tests and batch runs switch it off
 
+  // extension: raw camera images of r.src_w x r.src_h for update() (VisualOdometryMono::setRectification); the
+  // reconstruction uses the rectified projection.  Before the first frame only, else false and nothing changes.  update()
+  // hands the constructor's dims to the push, so construct the facade with the raw size {src_w, src_h, bytes per line}.
+  bool setRectification(const Rectification& r) {
+    if (!viso->setRectification(r)) return false;
+    if (r.n_cams > 0) reconstruction.setCalibration(r.cams[0].f, r.cams[0].cu, r.cams[0].cv);
+    return true;
+  }
+
   // returns whether the odometry of this frame succeeded (an extension: the reference's update returns nothing)
   bool update(uint8_t* img_data) {
     const bool ok = viso->process(img_data, &dims[0], replace);
@@ -129,6 +138,16 @@ public:
   StructureFromMotionStereo& operator=(const StructureFromMotionStereo&) = delete;
 
   void setVerbose(bool on) { verbose = on; }
+
+  // extension: raw stereo pairs of r.src_w x r.src_h for update() (VisualOdometryStereo::setRectification); odometry and
+  // reconstruction use the rectified projection and r.base.  Before the first frame only, else false and nothing changes.
+  // update() hands the constructor's dims to the push, so construct the facade with the raw size.
+  bool setRectification(const Rectification& r) {
+    if (!viso->setRectification(r)) return false;
+    param.calib.f = r.cams[0].f; param.calib.cu = r.cams[0].cu; param.calib.cv = r.cams[0].cv; param.base = r.base;
+    reconstruction.setCalibration(param.calib.f, param.calib.cu, param.calib.cv);
+    return true;
+  }
 
   // left / right: one rectified stereo pair of dims; returns whether the odometry of this frame succeeded (and, after the
   // first frame, the reconstruction's device call)

@@ -32,6 +32,12 @@ struct MonoTimer {
 using std::vector;
 
 VisualOdometryMono::VisualOdometryMono(parameters param) : VisualOdometry(param), param(param) {}
+
+bool VisualOdometryMono::setRectification(const Rectification& r) {
+  if (!matcher->setRectification(r)) return false;
+  if (r.n_cams > 0) { param.calib.f = r.cams[0].f; param.calib.cu = r.cams[0].cu; param.calib.cv = r.cams[0].cv; }
+  return true;
+}
 VisualOdometryMono::~VisualOdometryMono() {}
 
 bool VisualOdometryMono::process(uint8_t* I, uint32_t* dims, bool replace) {

@@ -24,6 +24,10 @@ public:
   // returns false if the motion is too small or an error occurred; valid after two calls
   bool process(uint8_t* I, uint32_t* dims, bool replace = false);
 
+  // extension: raw camera images (Matcher::setRectification); the calibration becomes the rectified projection of
+  // r.cams[0].  Before the first frame only: afterwards it returns false and changes nothing.
+  bool setRectification(const Rectification& r);
+
   // extensions for tests / the batch runner
   bool processDevice(const uint8_t* d_I, uint32_t* dims, bool replace = false);
   // the second half of process() for callers that pushed and matched through a MatcherBatch: bucketing + motion
@@ -60,7 +64,7 @@ private:
   int32_t triangulateChieral(std::vector<Matcher::p_match>& p_matched, Matrix& K, Matrix& R, Matrix& t, Matrix& X);
 
 protected:
-  const parameters param;
+  parameters param;
   Matrix F_last;
   std::vector<int> samples_last;
   std::vector<float> uv_last;

@@ -23,6 +23,13 @@ bool VisualOdometryStereo::process(uint8_t* I1, uint8_t* I2, uint32_t* dims, boo
   return updateMotion();
 }
 
+bool VisualOdometryStereo::setRectification(const Rectification& r) {
+  if (r.n_cams != 2 || !matcher->setRectification(r)) return false;
+  param.calib.f = r.cams[0].f; param.calib.cu = r.cams[0].cu; param.calib.cv = r.cams[0].cv; param.base = r.base;
+  matcher->setIntrinsics(param.calib.f, param.calib.cu, param.calib.cv, param.base);
+  return true;
+}
+
 void VisualOdometryStereo::adoptMatcher(Matcher* external) {
   VisualOdometry::adoptMatcher(external);
   matcher->setIntrinsics(param.calib.f, param.calib.cu, param.calib.cv, param.base);

@@ -24,6 +24,11 @@ public:
   bool process(uint8_t* I1, uint8_t* I2, uint32_t* dims, bool replace = false);
   using VisualOdometry::process;
 
+  // extension: raw stereo pairs (Matcher::setRectification with r.n_cams = 2); the calibration becomes the rectified
+  // projection and r.base.  Before the first frame only: afterwards, or for r.n_cams != 2, it returns false and changes
+  // nothing.
+  bool setRectification(const Rectification& r);
+
   // extensions for the batch runner and the tests
   // runs on a matcher owned by somebody else (a MatcherBatch sequence), with this object's calibration
   void adoptMatcher(Matcher* external);

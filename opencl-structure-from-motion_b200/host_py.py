@@ -4,7 +4,7 @@ import ctypes as C
 import os
 import numpy as np
 
-from visocu_py import Params, P_MATCH, RECON_FRAME, RECON_TRACK, ReconJob, VisocuError
+from visocu_py import Camera, Params, P_MATCH, RECON_FRAME, RECON_TRACK, ReconJob, VisocuError
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'libviso_b200.so')
@@ -41,6 +41,41 @@ class StereoParams(C.Structure):
         d.update(kw)
         for k, v in d.items():
             setattr(self, k, v)
+
+
+class Rectification(C.Structure):
+    """Rectification (host/rectify.h): n_cams cameras (left, right) for raw src_w x src_h images, rectified to out_w x out_h;
+    base = rectified baseline (stereo odometry)."""
+    _fields_ = [('n_cams', C.c_int32), ('cams', Camera * 2), ('src_w', C.c_int32), ('src_h', C.c_int32),
+                ('out_w', C.c_int32), ('out_h', C.c_int32), ('base', C.c_double)]
+
+    def __init__(self, cams, src_w, src_h, out_w, out_h, base=0.0):
+        super().__init__()
+        self.n_cams = len(cams)
+        for k, c in enumerate(cams):
+            self.cams[k] = c
+        self.src_w, self.src_h, self.out_w, self.out_h, self.base = int(src_w), int(src_h), int(out_w), int(out_h), float(base)
+
+
+def stereo_rectify(cam0, cam1, R, T, out_w, out_h):
+    """Bouguet's rectification of a rig whose camera 1 sees X1 = R X0 + T (host/rectify.h): (rect0, rect1, base), the
+    input cameras with their rectifying rotation and common rectified projection."""
+    R = np.ascontiguousarray(R, np.float64).reshape(9); T = np.ascontiguousarray(T, np.float64).reshape(3)
+    r0, r1, base = Camera(1, 1, 0, 0), Camera(1, 1, 0, 0), C.c_double()
+    lib().visob_stereo_rectify(C.byref(cam0), C.byref(cam1), _p(R), _p(T), int(out_w), int(out_h), C.byref(r0), C.byref(r1),
+                               C.byref(base))
+    return r0, r1, base.value
+
+
+def rectify_map(cam, src_w, src_h, out_w, out_h):
+    """The map visocu_set_rectification builds, computed on the host: (out_h, out_w, 2) int32 in 1/32 pixel; raises
+    VisocuError for what the library rejects."""
+    out = np.zeros((out_h, out_w, 2), np.int32) if out_w > 0 and out_h > 0 else None
+    why = C.create_string_buffer(256)
+    rc = lib().visob_rectify_map(C.byref(cam), int(src_w), int(src_h), int(out_w), int(out_h), _p(out), why)
+    if rc:
+        raise VisocuError('rectify_map: %d %s' % (rc, why.value.decode()))
+    return out
 
 
 _lib = None
@@ -109,6 +144,10 @@ class Matcher:
             lib().visob_matcher_match_features(self.h, method)
         else:
             lib().visob_matcher_match_features_tr(self.h, method, _p(np.ascontiguousarray(tr_delta, np.float64)))
+
+    def set_rectification(self, rect):
+        """Raw images of rect.src_w x rect.src_h from now on; False (nothing changed) after the first push."""
+        return bool(lib().visob_matcher_set_rectification(self.h, C.byref(rect)))
 
     def set_intrinsics(self, f, cu, cv, base):
         lib().visob_matcher_set_intrinsics(self.h, C.c_double(f), C.c_double(cu), C.c_double(cv), C.c_double(base))
@@ -182,6 +221,10 @@ class Mono:
         m = np.ascontiguousarray(matches, dtype=P_MATCH)
         return bool(lib().visob_mono_process_matches(self.h, _p(m), len(m)))
 
+    def set_rectification(self, rect):
+        """Raw images, calibration = rectified projection of camera 0; False (nothing changed) after the first frame."""
+        return bool(lib().visob_mono_set_rectification(self.h, C.byref(rect)))
+
     def motion(self):
         out = np.zeros((4, 4))
         lib().visob_mono_get_motion(self.h, _p(out))
@@ -233,6 +276,10 @@ class Stereo:
     def process_matches(self, matches):
         m = np.ascontiguousarray(matches, dtype=P_MATCH)
         return bool(lib().visob_stereo_process_matches(self.h, _p(m), len(m)))
+
+    def set_rectification(self, rect):
+        """Raw stereo pairs (rect.n_cams = 2), calibration and base from rect; False (nothing changed) after the first frame."""
+        return bool(lib().visob_stereo_set_rectification(self.h, C.byref(rect)))
 
     def motion(self):
         out = np.zeros((4, 4))
@@ -351,6 +398,9 @@ class Sfm:
         img = np.ascontiguousarray(img, np.uint8)
         return bool(lib().visob_sfm_update(self.h, _p(img)))
 
+    def set_rectification(self, rect):
+        return bool(lib().visob_sfm_set_rectification(self.h, C.byref(rect)))
+
     def points(self):
         n = lib().visob_sfm_get_points(self.h, None, 0)
         out = np.zeros((n, 3), np.float32)
@@ -381,6 +431,10 @@ class StereoSfm:
         """One stereo pair; returns whether its odometry (and, after the first frame, its reconstruction) succeeded."""
         left = np.ascontiguousarray(left, np.uint8); right = np.ascontiguousarray(right, np.uint8)
         return bool(lib().visob_stereo_sfm_update(self.h, _p(left), _p(right)))
+
+    def set_rectification(self, rect):
+        """Raw stereo pairs for update(); False (nothing changed) after the first frame."""
+        return bool(lib().visob_stereo_sfm_set_rectification(self.h, C.byref(rect)))
 
     def points(self):
         n = lib().visob_stereo_sfm_get_points(self.h, None, 0)
@@ -512,6 +566,10 @@ class Runner:
             self.h = None
 
     __del__ = close
+
+    def set_rectification(self, rect):
+        """Raw images for step() / run() (dims = the raw size); False (nothing changed) after the first step."""
+        return bool(lib().visob_runner_set_rectification(self.h, C.byref(rect)))
 
     def step(self, ptrs, dims, ptrs2=None, on_device=False, bucket=False):
         S = self.S

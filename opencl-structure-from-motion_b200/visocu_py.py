@@ -50,6 +50,25 @@ class Params(C.Structure):
             setattr(self, k, v)
 
 
+class Camera(C.Structure):
+    """visocu_camera: raw pinhole K, radial-tangential distortion, rectifying rotation R (row-major) and the rectified
+    projection f, cu, cv (host/rectify.h).  Defaults: no distortion, R = I, f = fy, (cu, cv) = (cx, cy)."""
+    _fields_ = [(n, C.c_double) for n in ('fx', 'fy', 'cx', 'cy', 'k1', 'k2', 'p1', 'p2', 'k3')] + \
+               [('R', C.c_double * 9)] + [(n, C.c_double) for n in ('f', 'cu', 'cv')]
+
+    def __init__(self, fx, fy, cx, cy, k1=0.0, k2=0.0, p1=0.0, p2=0.0, k3=0.0, R=None, f=None, cu=None, cv=None):
+        super().__init__()
+        for k, v in dict(fx=fx, fy=fy, cx=cx, cy=cy, k1=k1, k2=k2, p1=p1, p2=p2, k3=k3).items():
+            setattr(self, k, float(v))
+        self.R[:] = [float(x) for x in np.asarray(np.eye(3) if R is None else R, np.float64).reshape(9)]
+        self.f = float(fy if f is None else f)
+        self.cu = float(cx if cu is None else cu)
+        self.cv = float(cy if cv is None else cv)
+
+    def rotation(self):
+        return np.array(self.R[:], np.float64).reshape(3, 3)
+
+
 class VisocuError(RuntimeError):
     pass
 
@@ -164,6 +183,34 @@ class Context:
         self._ck(lib().visocu_push_frames(self.h, n, _p(frames), arr, int(bpl_in), int(on_device),
                                           _p(ns) if want_counts else None, _p(nd) if want_counts else None), 'push_frames')
         return ns, nd
+
+    def set_rectification(self, cams, src_w, src_h):
+        """visocu_set_rectification: maps for raw src_w x src_h images (cams: 0, 1 or 2 Camera)."""
+        arr = (Camera * max(1, len(cams)))(*cams)
+        self._ck(lib().visocu_set_rectification(self.h, len(cams), arr if cams else None, int(src_w), int(src_h)),
+                 'set_rectification')
+
+    def push_frames_rectified(self, frames, cams, imgs=None, ptrs=None, bpl_in=None, on_device=False, want_counts=True):
+        """visocu_push_frames_rectified: raw image k resampled with map cams[k] into frame frames[k]."""
+        frames = np.ascontiguousarray(frames, np.int32)
+        cams = np.ascontiguousarray(cams, np.int32)
+        n = len(frames)
+        if ptrs is None:
+            imgs = [np.ascontiguousarray(i, np.uint8) for i in imgs]
+            ptrs = [i.ctypes.data for i in imgs]
+            bpl_in = imgs[0].shape[1] if bpl_in is None else bpl_in
+        arr = (C.c_void_p * n)(*ptrs)
+        ns = np.zeros(n, np.int32); nd = np.zeros(n, np.int32)
+        self._ck(lib().visocu_push_frames_rectified(self.h, n, _p(frames), arr, _p(cams), int(bpl_in), int(on_device),
+                                                    _p(ns) if want_counts else None, _p(nd) if want_counts else None),
+                 'push_frames_rectified')
+        return ns, nd
+
+    def rectify_map(self, cam, width, height):
+        """The map of camera `cam` for width x height output images: (height, width, 2) int32, x and y in 1/32 pixel."""
+        out = np.zeros((height, width, 2), np.int32)
+        self._ck(lib().visocu_get_rectify_map(self.h, int(cam), _p(out), C.c_size_t(out.size)), 'get_rectify_map')
+        return out
 
     def features(self, frame, pass_):
         n = C.c_int32()
