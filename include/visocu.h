@@ -122,6 +122,29 @@ int  visocu_push_frames_rectified(visocu_ctx* ctx, int32_t n, const int32_t* fra
                                   int32_t bpl_in, int32_t on_device, int32_t* n_sparse, int32_t* n_dense);
 int  visocu_get_rectify_map(visocu_ctx* ctx, int32_t cam, int32_t* out, size_t cap);
 
+/* ---- dense stereo disparity (not in the reference): semi-global matching on the images of pushed frames ----
+ * visocu_disparity computes, for pair k, the disparity map of frame left[k] against frame right[k] from their
+ * full-resolution images as pushed (the rectified bytes after a rectifying push, whatever half_resolution says):
+ * census 9x7 (62 bits, neighbour < centre, coordinates clamped), cost = Hamming distance of cenL(x, y) and cenR(x - d, y)
+ * (62 where x - d < 0), 4 paths (+-x, +-y) or 8 (and the diagonals) of L_r(p, d) = C(p, d) + min(L_r(p-r, d),
+ * L_r(p-r, d+-1) + p1, min_k L_r(p-r, k) + p2) - min_k L_r(p-r, k) (L_r = C at the border), S = the sum of the paths;
+ * d* = the smallest d of min S.  Invalid (-1): uniqueness (some |d - d*| > 1 with 100 S(d*) > uniqueness S(d)) and, when
+ * lr_max_diff >= 0, x - d* < 0 or |dR(x - d*) - d*| > lr_max_diff, dR(x') = the smallest d < min(D, w - x') of
+ * min S(x' + d, y, d).  out[k] receives w x h int16 (row stride w) in 1/16 pixel: 16 d* plus, with subpixel = 1 and
+ * 0 < d* < D - 1, floor((16 (a - c) + den) / (2 den)) for den = a + c - 2 b > 0 (a, b, c = S at d* - 1, d*, d* + 1).
+ * Valid: max_disp D in {64, 128, 256}, paths in {4, 8}, 1 <= p1 < p2 <= 150, 0 <= uniqueness <= 100,
+ * -1 <= lr_max_diff <= D, subpixel in {0, 1}; oracle/sgm_oracle.c states the algorithm in plain C.
+ * out_on_device = 0: out[k] are host memory; 1: device memory of the context's GPU.  The call runs on the current lane,
+ * behind the last push of every lane, and waits for its work.  VISOCU_EINVAL for bad parameters, a frame index out of
+ * range, a null pointer or n_pairs < 0; VISOCU_ESTATE for a frame never pushed or an unconfigured context; both before
+ * anything is enqueued or written.  Per group of at most 128 pairs: 4 launches with 4 paths, 6 with 8, and scratch of
+ * w h (16 + 2 D) bytes per pair (+ 2 w h for host outputs). */
+typedef struct { int32_t max_disp, paths, p1, p2, uniqueness, lr_max_diff, subpixel; } visocu_sgm_params;
+int  visocu_disparity(visocu_ctx* ctx, int32_t n_pairs, const int32_t* left, const int32_t* right,
+                      const visocu_sgm_params* p, int16_t* const* out, int32_t out_on_device);
+/* VISOCU_OK if p is non-null and inside the valid ranges above, else VISOCU_EINVAL (for callers that store parameters) */
+int  visocu_sgm_check(const visocu_sgm_params* p);
+
 /* ---- filter:: functions (viso/filter.h:78-94), host buffers in and out, same argument order ---- */
 int  visocu_sobel5x5(visocu_ctx* ctx, const uint8_t* in, uint8_t* out_v, uint8_t* out_h, int32_t w, int32_t h);
 int  visocu_sobel3x3(visocu_ctx* ctx, const uint8_t* in, uint8_t* out_v, uint8_t* out_h, int32_t w, int32_t h);

@@ -282,6 +282,15 @@ VISOB_API void* visob_stereo_sfm_odometry(void* s) { return &((StructureFromMoti
 VISOB_API void visob_stereo_sfm_device_points(void* s, const float** d_xyz, int64_t* n) { ((StructureFromMotionStereo*)s)->devicePoints(d_xyz, n); }
 
 // ---- rectification (host/rectify.h): setRectification of the classes above, 1 = done, 0 = refused
+// dense disparity of the current stereo pair (Matcher::computeDisparity): 1 = done, 0 = failed (message on cerr)
+VISOB_API int visob_matcher_disparity(void* m, const visocu_sgm_params* p, int16_t* out, int on_device) {
+  return ((Matcher*)m)->computeDisparity(*p, out, on_device != 0) ? 1 : 0;
+}
+VISOB_API int visob_matcher_stereo_pair(void* m, int32_t* frames2, int32_t* wh) { return ((Matcher*)m)->stereoPair(frames2, frames2 + 1, wh, wh + 1) ? 1 : 0; }
+VISOB_API void* visob_stereo_matcher(void* v) { return ((VisualOdometryStereo*)v)->getMatcher(); }
+VISOB_API int visob_stereo_sfm_disparity(void* s, const visocu_sgm_params* p, int16_t* out, int on_device) {
+  return ((StructureFromMotionStereo*)s)->computeDisparity(*p, out, on_device != 0) ? 1 : 0;
+}
 VISOB_API int visob_matcher_set_rectification(void* m, const Rectification* r) { return ((Matcher*)m)->setRectification(*r) ? 1 : 0; }
 VISOB_API int visob_mono_set_rectification(void* v, const Rectification* r) { return ((MonoAccess*)v)->setRectification(*r) ? 1 : 0; }
 VISOB_API int visob_stereo_set_rectification(void* v, const Rectification* r) { return ((VisualOdometryStereo*)v)->setRectification(*r) ? 1 : 0; }
@@ -368,6 +377,12 @@ struct Runner {
   std::vector<SfmState*> sfms;               // one per sequence (modes 3 and 4)
   std::vector<int32_t> last_matches, last_ok;
   bool started = false;                      // a step has run: the rectification is fixed
+  // dense disparity (modes 2 and 4): while disp_on, per sequence a device map of the last step (null: none this step)
+  bool disp_on = false;
+  visocu_sgm_params disp_params{};
+  std::vector<int16_t*> disp_buf;            // runner-owned, w x h int16 on the sequence's worker context
+  std::vector<int32_t> disp_w, disp_h;
+  std::vector<uint8_t> disp_valid;          // bytes, not bits: the workers write their own sequences concurrently
   Matcher& matcher_of(int seq) { return batches[seq % threads]->sequence(seq / threads); }
 };
 
@@ -412,6 +427,34 @@ void runner_sfm(Runner* r, int tid) {
     std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
     for (int s : ids) r->last_ok[s] = 0;
   }
+}
+
+// Dense disparity of every sequence of worker `tid` with a stereo pair this step: ONE visocu_disparity on lane 5, which
+// the odometry and reconstruction calls (lane 4) and the matching (lane 0) do not use, into the runner's device buffers.
+// Only reads the frames: the odometry results of the step are the same with and without it.
+void runner_disparity(Runner* r, int tid) {
+  visocu_ctx* ctx = r->batches[tid]->context();
+  std::vector<int32_t> left, right;
+  std::vector<int16_t*> out;
+  std::vector<int> ids;
+  for (int s = tid; s < r->S; s += r->threads) {
+    r->disp_valid[s] = 0;
+    int32_t l, rt, w, h;
+    if (!ctx || !r->matcher_of(s).stereoPair(&l, &rt, &w, &h)) continue;
+    if (r->disp_buf[s] && (r->disp_w[s] != w || r->disp_h[s] != h)) { visocu_device_free(ctx, r->disp_buf[s]); r->disp_buf[s] = nullptr; }
+    if (!r->disp_buf[s]) {
+      void* p = nullptr;
+      if (visocu_device_alloc(ctx, (size_t)w * h * sizeof(int16_t), &p) != VISOCU_OK) { std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl; continue; }
+      r->disp_buf[s] = (int16_t*)p; r->disp_w[s] = w; r->disp_h[s] = h;
+    }
+    left.push_back(l); right.push_back(rt); out.push_back(r->disp_buf[s]); ids.push_back(s);
+  }
+  if (ids.empty()) return;
+  visocu_set_lane(ctx, 5);
+  const int rc = visocu_disparity(ctx, (int32_t)ids.size(), left.data(), right.data(), &r->disp_params, out.data(), 1);
+  visocu_set_lane(ctx, 0);
+  if (rc != VISOCU_OK) { std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl; return; }
+  for (int s : ids) r->disp_valid[s] = 1;
 }
 
 // host stages that follow the matching of one frame for every sequence of worker `tid`: bucketing, and for the odometry
@@ -509,6 +552,7 @@ void runner_post(Runner* r, int tid, int bucket, int32_t* n_matches_out, int32_t
     }
   }
   if (r->mode == 3 || r->mode == 4) runner_sfm(r, tid);
+  if (r->disp_on) runner_disparity(r, tid);
   for (int s = tid; s < r->S; s += r->threads) {
     if (n_matches_out) n_matches_out[s] = r->last_matches[s];
     if (ok_out) ok_out[s] = r->last_ok[s];
@@ -640,6 +684,8 @@ VISOB_API void* visob_runner_create_stereo_sfm(int device, int n_sequences, int 
 }
 VISOB_API void visob_runner_destroy(void* h) {
   Runner* r = (Runner*)h;
+  for (int s = 0; s < (int)r->disp_buf.size(); s++)
+    if (r->disp_buf[s]) visocu_device_free(r->batches[s % r->threads]->context(), r->disp_buf[s]);
   for (int s = 0; s < (int)r->sfms.size(); s++) {
     if (r->sfms[s]->store) visocu_recon_store_destroy(r->batches[s % r->threads]->context(), r->sfms[s]->store);
     delete r->sfms[s];
@@ -670,6 +716,27 @@ VISOB_API int visob_runner_set_rectification(void* h, const Rectification* rc) {
     for (SfmState* q : r->sfms) q->recon.setCalibration(c.f, c.cu, c.cv);
   }
   return 1;
+}
+// Dense disparity for the stereo modes (2, 4): with p, every following step computes each sequence's disparity map
+// (visocu_disparity, one call per worker) into a device buffer of the runner; null turns it off.  1 = done, 0 = refused
+// (another mode, or parameters outside the ranges of visocu_disparity).
+VISOB_API int visob_runner_set_disparity(void* h, const visocu_sgm_params* p) {
+  Runner* r = (Runner*)h;
+  if (r->mode != 2 && r->mode != 4) return 0;
+  if (!p) { r->disp_on = false; return 1; }
+  if (visocu_sgm_check(p) != VISOCU_OK) return 0;
+  r->disp_params = *p;
+  r->disp_on = true;
+  r->disp_buf.resize(r->S, nullptr); r->disp_w.resize(r->S, 0); r->disp_h.resize(r->S, 0); r->disp_valid.resize(r->S, 0);
+  return 1;
+}
+// the sequence's disparity map of the last step in device memory (w x h int16, 1/16 pixel, -1 = invalid), valid until
+// the next step: 0, or -1 when the feature is off, for another mode, a bad sequence or a step without a map
+VISOB_API int visob_runner_device_disparity(void* h, int seq, const int16_t** d_map, int32_t* w, int32_t* ht) {
+  Runner* r = (Runner*)h;
+  if (!r->disp_on || seq < 0 || seq >= r->S || !d_map || !w || !ht || !r->disp_valid[seq]) return -1;
+  *d_map = r->disp_buf[seq]; *w = r->disp_w[seq]; *ht = r->disp_h[seq];
+  return 0;
 }
 VISOB_API double visob_runner_step(void* h, const uint8_t* const* imgs, const uint8_t* const* imgs2, const int32_t* dims,
                                    int on_device, int bucket, int32_t* n_matches_out, int32_t* ok_out) {

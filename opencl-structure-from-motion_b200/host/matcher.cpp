@@ -218,6 +218,25 @@ void Matcher::pushFinish(bool ok, bool stereo, const int32_t* ns, const int32_t*
   have_I1c = false;
 }
 
+bool Matcher::stereoPair(int32_t* left, int32_t* right, int32_t* w, int32_t* h) const {
+  if (!ctx || slot[2] < 0 || slot[3] < 0) return false;
+  *left = slot[2]; *right = slot[3]; *w = cfg_w; *h = cfg_h;
+  return true;
+}
+
+bool Matcher::computeDisparity(const visocu_sgm_params& p, int16_t* out, bool on_device) {
+  int32_t l, r, w, h;
+  if (!stereoPair(&l, &r, &w, &h)) {
+    std::cerr << "ERROR: computeDisparity needs a stereo pair (the last push was mono or failed)" << std::endl;
+    return false;
+  }
+  if (visocu_disparity(ctx, 1, &l, &r, &p, &out, on_device ? 1 : 0) != VISOCU_OK) {
+    std::cerr << "ERROR: " << visocu_last_error(ctx) << std::endl;
+    return false;
+  }
+  return true;
+}
+
 // padded copy of a left image (previous or current) from the device frame it lives in
 bool Matcher::fetchImage(int which, vector<uint8_t>& out) {
   const int32_t f = slot[which];

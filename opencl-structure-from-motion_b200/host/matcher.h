@@ -75,6 +75,12 @@ public:
   // images.  r.n_cams = 0 returns to plain pushes.  Allowed before the first push only: afterwards it returns false and
   // changes nothing (as it does for more than 2 cameras).
   bool setRectification(const Rectification& r);
+  // Dense disparity of the current stereo pair (left against right image of the last push, visocu_disparity): out
+  // receives w x h int16 in 1/16 pixel (-1 = invalid), row stride w; host memory, or device memory of this matcher's GPU
+  // with on_device.  False, with a message on cerr, after a mono push or when the device call fails.
+  bool computeDisparity(const visocu_sgm_params& p, int16_t* out, bool on_device);
+  // the device frames and the (rectified) size of the current stereo pair; false after a mono push or a failed one
+  bool stereoPair(int32_t* left, int32_t* right, int32_t* w, int32_t* h) const;
   // same as pushBack, but the images already live in device memory of this matcher's GPU
   void pushBackDevice(const uint8_t* d_I1, const uint8_t* d_I2, uint32_t* dims, const bool replace);
   visocu_ctx* context() { return ctx; }

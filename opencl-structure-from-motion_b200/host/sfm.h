@@ -198,5 +198,7 @@ public:
   }
   const Matrix& getPose() const { return Tr_total; }
   VisualOdometryStereo& odometry() { return *viso; }
+  // dense disparity of the last pair (Matcher::computeDisparity)
+  bool computeDisparity(const visocu_sgm_params& p, int16_t* out, bool on_device) { return viso->getMatcher()->computeDisparity(p, out, on_device); }
 };
 #endif

@@ -88,7 +88,8 @@ def lib():
             raise VisocuError(LIB_PATH + ' is missing: run __graft_entry__.build()')
         L = C.CDLL(LIB_PATH)
         for name in ('visob_matcher_create', 'visob_mono_create', 'visob_mono_matcher', 'visob_runner_create', 'visob_runner_create_stereo', 'visob_runner_create_sfm', 'visob_stereo_create', 'visob_recon_create', 'visob_sfm_create',
-                     'visob_matcher_context', 'visob_runner_create_stereo_sfm', 'visob_stereo_sfm_create', 'visob_stereo_sfm_odometry'):
+                     'visob_matcher_context', 'visob_runner_create_stereo_sfm', 'visob_stereo_sfm_create', 'visob_stereo_sfm_odometry',
+                     'visob_stereo_matcher'):
             getattr(L, name).restype = C.c_void_p
         L.visob_matcher_gain.restype = C.c_float
         L.visob_runner_step.restype = C.c_double
@@ -154,6 +155,21 @@ class Matcher:
 
     def bucket(self, max_features, bw, bh):
         lib().visob_matcher_bucket(self.h, max_features, C.c_float(bw), C.c_float(bh))
+
+    def stereo_size(self):
+        """(w, h) of the current stereo pair, or None after a mono push or a failed one."""
+        f = np.zeros(2, np.int32); wh = np.zeros(2, np.int32)
+        return tuple(wh.tolist()) if lib().visob_matcher_stereo_pair(self.h, _p(f), _p(wh)) else None
+
+    def disparity(self, params=None):
+        """Matcher::computeDisparity of the current stereo pair: an (h, w) int16 map in 1/16 pixel (-1 = invalid), or
+        None after a mono push or when the device call fails."""
+        wh = self.stereo_size()
+        if wh is None:
+            return None
+        out = np.zeros((wh[1], wh[0]), np.int16)
+        ok = lib().visob_matcher_disparity(self.h, C.byref(_sgm(params)), _p(out), 0)
+        return out if ok else None
 
     def matches(self, stage=2):
         n = lib().visob_matcher_get_matches(self.h, stage, None, 0)
@@ -307,6 +323,16 @@ class Stereo:
         if n:
             lib().visob_stereo_get_samples(self.h, _p(out), n)
         return out.reshape(-1, 3)
+
+    def matcher(self):
+        """The odometry's Matcher (a view, kept alive by this object)."""
+        m = Matcher(self.params, handle=lib().visob_stereo_matcher(self.h))
+        m.owner = self
+        return m
+
+    def disparity(self, params=None):
+        """Dense disparity of the last stereo pair (Matcher.disparity)."""
+        return self.matcher().disparity(params)
 
     def batch_prepare(self, matches):
         """First half of process_matches for a device estimate: keeps the matches and draws the sample table (samples()).
@@ -462,12 +488,49 @@ class StereoSfm:
         """The points as a float32 CUDA tensor (n x 3) of its own (a copy of the device store)."""
         return _points_tensor(*self.device_points())
 
+    def disparity_tensor(self, params=None):
+        """Dense disparity of the last pair as an (h, w) int16 CUDA tensor, written in place by the device; None after a
+        failed frame."""
+        import torch
+        wh = self.odometry().matcher().stereo_size()
+        if wh is None:
+            return None
+        out = torch.empty((wh[1], wh[0]), dtype=torch.int16, device='cuda')
+        torch.cuda.current_stream(out.device).synchronize()
+        ok = lib().visob_stereo_sfm_disparity(self.h, C.byref(_sgm(params)), C.c_void_p(out.data_ptr()), 1)
+        return out if ok else None
+
 
 class _DevicePoints:
     """A borrowed view of n x 3 device floats for torch (__cuda_array_interface__)."""
 
     def __init__(self, ptr, n):
         self.__cuda_array_interface__ = dict(shape=(n, 3), typestr='<f4', data=(ptr, False), version=3, strides=None)
+
+
+class _DeviceMap:
+    """A borrowed view of an (h, w) int16 device map for torch (__cuda_array_interface__)."""
+
+    def __init__(self, ptr, w, h):
+        self.__cuda_array_interface__ = dict(shape=(h, w), typestr='<i2', data=(ptr, False), version=3, strides=None)
+
+
+def _sgm(params):
+    import visocu_py
+    return visocu_py.SgmParams() if params is None else params
+
+
+def disparity_to_points(disp16, f, cu, cv, base):
+    """The valid pixels (value > 0) of an (h, w) disparity map in 1/16 pixel (numpy or torch) reprojected into the left
+    camera: Z = 16 f base / d, X = (u - cu) Z / f, Y = (v - cv) Z / f.  Returns an (n, 3) float32 torch tensor on the
+    map's device, in row-major pixel order."""
+    import torch
+    d = torch.as_tensor(disp16)
+    v, u = torch.nonzero(d > 0, as_tuple=True)
+    Z = (16.0 * f * base) / d[v, u].to(torch.float32)
+    X = (u.to(torch.float32) - cu) * Z / f
+    Y = (v.to(torch.float32) - cv) * Z / f
+    return torch.stack([X, Y, Z], 1)
 
 
 def _points_tensor(ptr, n):
@@ -625,6 +688,19 @@ class Runner:
         if lib().visob_runner_device_points(self.h, seq, C.byref(d), C.byref(n)):
             raise VisocuError('device_points: not a structure-from-motion runner, or no sequence %d' % seq)
         return d.value or 0, n.value
+
+    def set_disparity(self, params):
+        """Stereo modes: compute every sequence's dense disparity at each following step (SgmParams), or stop (None).
+        False for another mode or parameters out of range."""
+        return bool(lib().visob_runner_set_disparity(self.h, None if params is None else C.byref(params)))
+
+    def disparity_tensor(self, seq):
+        """The sequence's disparity map of the last step as an (h, w) int16 CUDA tensor (a copy), or None without one."""
+        import torch
+        d = C.c_void_p(); w = C.c_int32(); h = C.c_int32()
+        if lib().visob_runner_device_disparity(self.h, seq, C.byref(d), C.byref(w), C.byref(h)):
+            return None
+        return torch.as_tensor(_DeviceMap(d.value, w.value, h.value), device='cuda').clone()
 
     def points_tensor(self, seq):
         """The sequence's points as a float32 CUDA tensor (n x 3) on the runner's device, a copy of its own."""

@@ -110,10 +110,9 @@ def _value_noise(x, y, seed, octaves=4, base=2.0, lacunarity=2.3, gain=0.6):
     return total / np.float32(norm)
 
 
-def corridor_frame(k, width=1241, height=376, seed=1234, f=KITTI_F, cu=KITTI_CU, cv=KITTI_CV,
-                   cam_height=1.6, pitch=-0.08, step=0.8, baseline_x=0.0):
-    """Frame k of a forward drive (0.8 m per frame, yaw 0.01*sin(0.3k)) through a textured corridor.
-    Camera axes: x right, y down, z forward.  Floor y=+cam_height, ceiling y=-4, walls x=+-6."""
+def _corridor_rays(k, width, height, f, cu, cv, cam_height, pitch, step, baseline_x):
+    """Ray cast of corridor_frame: per pixel the surface hit (0 floor, 1 ceiling, 2 / 3 walls), the ray parameter t
+    (capped at 400) and the hit point."""
     scale = width / 1241.0
     f, cu, cv = f * scale, cu * scale, cv * scale
     u = np.arange(width, dtype=np.float32)[None, :]
@@ -142,6 +141,14 @@ def corridor_frame(k, width=1241, height=376, seed=1234, f=KITTI_F, cu=KITTI_CU,
     t = np.min(ts, axis=0)
     t = np.minimum(t, np.float32(400.0))
     px, py, pz = ox + t * dx3, oy + t * dy3, oz + t * dz3
+    return which, t, px, py, pz
+
+
+def corridor_frame(k, width=1241, height=376, seed=1234, f=KITTI_F, cu=KITTI_CU, cv=KITTI_CV,
+                   cam_height=1.6, pitch=-0.08, step=0.8, baseline_x=0.0):
+    """Frame k of a forward drive (0.8 m per frame, yaw 0.01*sin(0.3k)) through a textured corridor.
+    Camera axes: x right, y down, z forward.  Floor y=+cam_height, ceiling y=-4, walls x=+-6."""
+    which, t, px, py, pz = _corridor_rays(k, width, height, f, cu, cv, cam_height, pitch, step, baseline_x)
     img = np.zeros((height, width), dtype=np.float32)
     for s, (a, b) in enumerate([(px, pz), (px, pz), (py, pz), (py, pz)]):
         m = which == s
@@ -150,6 +157,13 @@ def corridor_frame(k, width=1241, height=376, seed=1234, f=KITTI_F, cu=KITTI_CU,
     fade = np.clip(np.float32(1.0) - t / np.float32(120.0), 0.15, 1.0)
     out = np.float32(128.0) + (img - np.float32(0.5)) * np.float32(330.0) * fade
     return np.clip(np.rint(out), 0, 255).astype(np.uint8)
+
+
+def corridor_depth(k, width=1241, height=376, f=KITTI_F, cu=KITTI_CU, cv=KITTI_CV, cam_height=1.6, pitch=-0.08, step=0.8,
+                   baseline_x=0.0):
+    """The ray parameter t of corridor_frame per pixel, (height, width) float32: the depth Z in the camera frame, since
+    every ray has dz = 1 there.  t is capped at 400 where the ray leaves the corridor."""
+    return _corridor_rays(k, width, height, f, cu, cv, cam_height, pitch, step, baseline_x)[1]
 
 
 def corridor_sequence(n_frames, width=1241, height=376, seed=1234, start=0, **kw):

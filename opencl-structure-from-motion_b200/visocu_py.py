@@ -69,6 +69,18 @@ class Camera(C.Structure):
         return np.array(self.R[:], np.float64).reshape(3, 3)
 
 
+class SgmParams(C.Structure):
+    """visocu_sgm_params: semi-global matching settings of visocu_disparity (include/visocu.h)."""
+    _fields_ = [(n, C.c_int32) for n in ('max_disp', 'paths', 'p1', 'p2', 'uniqueness', 'lr_max_diff', 'subpixel')]
+
+    def __init__(self, **kw):
+        super().__init__()
+        d = dict(max_disp=128, paths=8, p1=10, p2=120, uniqueness=95, lr_max_diff=1, subpixel=1)
+        d.update(kw)
+        for k, v in d.items():
+            setattr(self, k, int(v))
+
+
 class VisocuError(RuntimeError):
     pass
 
@@ -99,6 +111,7 @@ class Context:
             raise VisocuError('visocu_create: %d %s' % (rc, lib().visocu_last_error(None).decode()))
         self.params = None
         self.dims = None
+        self.device = device
 
     def close(self):
         if getattr(self, 'h', None) and self.h.value:
@@ -227,6 +240,29 @@ class Context:
         out = np.zeros((h, bpl), np.uint8)
         self._ck(lib().visocu_get_plane(self.h, frame, which, _p(out), C.c_size_t(out.nbytes), _p(dims)), 'get_plane')
         return out, (w, h, bpl)
+
+    def _disparity(self, left, right, params, ptrs, on_device):
+        left = np.ascontiguousarray(left, np.int32); right = np.ascontiguousarray(right, np.int32)
+        n = len(left)
+        params = SgmParams() if params is None else params
+        arr = (C.c_void_p * max(n, 1))(*ptrs)
+        self._ck(lib().visocu_disparity(self.h, n, _p(left), _p(right), C.byref(params), arr, int(on_device)), 'disparity')
+
+    def disparity(self, left, right, params=None):
+        """visocu_disparity of frames left[k] against right[k]: a list of (h, w) int16 maps in 1/16 pixel (-1 = invalid)."""
+        w, h = self.dims
+        outs = [np.zeros((h, w), np.int16) for _ in range(len(left))]
+        self._disparity(left, right, params, [o.ctypes.data for o in outs], 0)
+        return outs
+
+    def disparity_tensor(self, left, right, params=None):
+        """The same maps as one int16 CUDA tensor (n, h, w), written by the kernels in place."""
+        import torch
+        w, h = self.dims
+        out = torch.empty((len(left), h, w), dtype=torch.int16, device='cuda:%d' % self.device)
+        torch.cuda.current_stream(out.device).synchronize()     # the memory may still be in use by torch's stream
+        self._disparity(left, right, params, [out[k].data_ptr() for k in range(len(left))], 1)
+        return out
 
     def tile_levels(self, n_launch=1):
         """(levels, pick): the fused filter + NMS kernel's tile configurations, largest first, as dicts (kx, ky, ntx, nty,
