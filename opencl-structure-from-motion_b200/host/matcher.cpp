@@ -476,6 +476,8 @@ void Matcher::computePriorStatistics(vector<p_match>& p_matched, int32_t method)
   const float bs = (float)param.match_binsize;
   const int32_t ub = (int32_t)ceil((float)dims_c[0] / bs), vb = (int32_t)ceil((float)dims_c[1] / bs);
   const int32_t nbin = ub * vb, stages = method == 2 ? 4 : 2, nd = stages * 2;
+  // nothing pushed yet: no image size, so no bin grid and no ranges
+  if (ub <= 0 || vb <= 0) { ranges.clear(); return; }
   // running min / max of the displacements seen in the 3x3 bin neighbourhood of every match
   vector<float> lo((size_t)nbin * 8, 1000000.f), hi((size_t)nbin * 8, -1000000.f);
   vector<uint8_t> seen(nbin, 0);

@@ -138,17 +138,21 @@ def compute_features(img, params):
                 dims=(w, h, b), dims_m=(wm, hm, bm))
 
 
-def matching(method, m1p, m2p, m1c, m2c, dims_c, params, ranges=None):
-    """params: effective parameters (match_radius already halved for half resolution)."""
+def matching(method, m1p, m2p, m1c, m2c, dims_c, params, ranges=None, tr_delta=None, counts=False):
+    """params: effective parameters (match_radius already halved for half resolution).  tr_delta: Tr_delta (4x4 or
+    3x4, quad matching; the prediction also uses params.f, cu, cv, base).  counts=True also returns (entries of the
+    scanned bins, window candidates) over all hops."""
     arrs = [np.ascontiguousarray(m, np.int32) if m is not None else np.zeros((0, 12), np.int32) for m in (m1p, m2p, m1c, m2c)]
     cap = max(len(a) for a in arrs) + 1
     out = np.zeros(cap, P_MATCH)
     d = np.array(dims_c, np.int32)
     r = np.ascontiguousarray(ranges, np.float32) if ranges is not None else None
+    t = np.ascontiguousarray(np.asarray(tr_delta, np.float64)[:3, :4]) if tr_delta is not None else None
+    c2 = np.zeros(2, np.int64)
     n = lib().vo_matching(method, _p(arrs[0]), len(arrs[0]), _p(arrs[1]), len(arrs[1]), _p(arrs[2]), len(arrs[2]), _p(arrs[3]),
-                          len(arrs[3]), _p(d), C.byref(params), int(ranges is not None), _p(r), _p(out), cap)
+                          len(arrs[3]), _p(d), C.byref(params), int(ranges is not None), _p(r), _p(t), _p(out), cap, _p(c2))
     assert 0 <= n <= cap
-    return out[:n].copy()
+    return (out[:n].copy(), (int(c2[0]), int(c2[1]))) if counts else out[:n].copy()
 
 
 def prior_statistics(matches, method, dims_c, params):
@@ -162,14 +166,27 @@ def prior_statistics(matches, method, dims_c, params):
     return out
 
 
+def _planes(planes):
+    g = lambda k: _p(np.ascontiguousarray(planes[k])) if planes.get(k) is not None else None
+    return [g(k) for k in ('du1p', 'dv1p', 'du2p', 'dv2p', 'du1c', 'dv1c', 'du2c', 'dv2c')]
+
+
 def refine_pixel(matches, method, dims, planes):
     """planes: dict with du1p dv1p du2p dv2p du1c dv1c du2c dv2c (full-resolution planes; missing = None)."""
     m = np.array(matches, dtype=P_MATCH, copy=True)
     d = np.array(dims, np.int32)
-    g = lambda k: _p(np.ascontiguousarray(planes[k])) if planes.get(k) is not None else None
-    lib().vo_refine_pixel(_p(m), len(m), method, _p(d), _p(d), g('du1p'), g('dv1p'), g('du2p'), g('dv2p'), g('du1c'), g('dv1c'),
-                          g('du2c'), g('dv2c'))
+    lib().vo_refine_pixel(_p(m), len(m), method, _p(d), _p(d), *_planes(planes))
     return m
+
+
+def refine_subpixel(matches, method, dims, planes):
+    """parabolicFitting on every match.  Returns (matches with refined coordinates, keep flags, decision margins): the
+    list is not compacted; margin = smallest distance of a float decision to its threshold (+inf: none taken)."""
+    m = np.array(matches, dtype=P_MATCH, copy=True)
+    d = np.array(dims, np.int32)
+    keep = np.zeros(len(m), np.uint8); margin = np.zeros(len(m), np.float64)
+    lib().vo_refine_subpixel(_p(m), len(m), method, _p(d), _p(d), *_planes(planes), _p(keep), _p(margin))
+    return m, keep.astype(bool), margin
 
 
 def normalize(matches):

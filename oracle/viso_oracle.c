@@ -8,7 +8,9 @@
  * Parity status: PINNED.  tests/test_oracle_vs_ref.py checks every function against the unmodified reference compiled
  * into oracle/_ref/libvisoref*.so (integer stages bit-exact, FP64 stages to the tolerance stated there), and
  * tests/test_oracle_golden.py checks it against the committed fixtures in tests/golden/ (generated from oracle/_ref by
- * tests/golden/make_golden.py).
+ * tests/golden/make_golden.py).  Stereo matching, the motion-predicted quad search and sub-pixel refinement have no
+ * counterpart in the reference shim: tests/test_oracle_vs_ref.py pins them against the reference results stored for
+ * tests/test_gpu_host_layer.py instead (integer results bit-exact, sub-pixel coordinates to 1e-4).
  *
  * FP64 note: the SVD here is a one-sided Jacobi iteration, not the reference's Numerical-Recipes svdcmp
  * (matrix.cpp:586-814); singular values and the null vectors used by the 8-point algorithm agree to rounding, which is
@@ -261,9 +263,14 @@ static binlist make_bins(const int32_t* m, int n, const vo_params* p, int ub, in
 
 static int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
 
-/* matcher.cpp:892-963 (without the motion-predicted cost term, i.e. u_ = v_ = -1) */
+/* Work counters of one vo_matching call: entries of the bins a hop scans, and candidates that pass its window test
+ * (what visocu_match_stats reports for the device). */
+typedef struct { int64_t scanned, candidates; } counters;
+
+/* matcher.cpp:892-963.  (up, vp): predicted position of the match (matcher.cpp:948-953), or u_ = v_ = -1 for none:
+ * then every candidate in the window costs SAD + 4 * distance to it, in double precision. */
 static int find_match(const int32_t* m1, int i1, const int32_t* m2, const binlist* k2, int ub, int vb, int stat_bin, int stage,
-                      int flow, int use_prior, const vo_range* ranges, const vo_params* p) {
+                      int flow, int use_prior, const vo_range* ranges, const vo_params* p, double up, double vp, counters* cnt) {
   int min_ind = 0;
   double min_cost = 10000000;
   const int u1 = m1[12 * i1], v1 = m1[12 * i1 + 1], c = m1[12 * i1 + 3];
@@ -279,14 +286,22 @@ static int find_match(const int32_t* m1, int i1, const int32_t* m2, const binlis
   const float bs = (float)p->match_binsize;
   const int ub0 = clampi((int)floorf(u_min / bs), 0, ub - 1), ub1 = clampi((int)floorf(u_max / bs), 0, ub - 1);
   const int vb0 = clampi((int)floorf(v_min / bs), 0, vb - 1), vb1 = clampi((int)floorf(v_max / bs), 0, vb - 1);
+  const int predicted = up >= 0 && vp >= 0;
   for (int ubin = ub0; ubin <= ub1; ubin++)
     for (int vbin = vb0; vbin <= vb1; vbin++) {
       const int k = (c * vb + vbin) * ub + ubin;
+      cnt->scanned += k2->start[k + 1] - k2->start[k];
       for (int e = k2->start[k]; e < k2->start[k + 1]; e++) {
         const int i2 = k2->idx[e];
         const int u2 = m2[12 * i2], v2 = m2[12 * i2 + 1];
         if (u2 >= u_min && u2 <= u_max && v2 >= v_min && v2 <= v_max) {
+          cnt->candidates++;
           double cost = (double)vo_sad((const uint8_t*)(m1 + 12 * i1 + 4), (const uint8_t*)(m2 + 12 * i2 + 4), 32);
+          if (predicted) {
+            const double du = (double)u2 - up, dv = (double)v2 - vp;
+            const double dist = sqrt(du * du + dv * dv);
+            cost = cost + 4 * dist;
+          }
           if (cost < min_cost) { min_ind = i2; min_cost = cost; }
         }
       }
@@ -294,48 +309,75 @@ static int find_match(const int32_t* m1, int i1, const int32_t* m2, const binlis
   return min_ind;
 }
 
-/* matcher.cpp:965-1205, methods 0 (flow) and 2 (quad), Tr_delta = NULL */
+static int stat_bin_of(const vo_params* p, int u, int v, int ub, int vb) {
+  const float bs = (float)p->match_binsize;
+  int ubin = (int)floorf((float)u / bs), vbin = (int)floorf((float)v / bs);
+  if (ubin > ub - 1) ubin = ub - 1;
+  if (vbin > vb - 1) vbin = vb - 1;
+  return vbin * ub + ubin;
+}
+
+/* matcher.cpp:965-1205: methods 0 (flow), 1 (stereo) and 2 (quad, with the motion-predicted search of
+ * matcher.cpp:1112-1138 if tr_delta, rows 0..2 of Tr_delta, is given).  Nothing is matched if a set the method needs is
+ * empty (matchFeatures returns early, matcher.cpp:190-212).  counts2 (optional): scanned entries, window candidates. */
 int vo_matching(int method, const int32_t* m1p, int n1p, const int32_t* m2p, int n2p, const int32_t* m1c, int n1c,
                 const int32_t* m2c, int n2c, const int32_t dims_c[3], const vo_params* p, int use_prior,
-                const vo_range* ranges, vo_match* out, int cap) {
+                const vo_range* ranges, const double* tr_delta, vo_match* out, int cap, int64_t* counts2) {
   const int ub = (int)ceilf((float)dims_c[0] / (float)p->match_binsize), vb = (int)ceilf((float)dims_c[1] / (float)p->match_binsize);
   int count = 0;
-  const float bs = (float)p->match_binsize;
-  if (method == 0) {
-    binlist k1p = make_bins(m1p, n1p, p, ub, vb), k1c = make_bins(m1c, n1c, p, ub, vb);
+  counters cnt = {0, 0};
+  if (counts2) { counts2[0] = 0; counts2[1] = 0; }
+  if (method < 0 || method > 2) return -1;
+  if (((method != 1) && n1p == 0) || (method == 2 && n2p == 0) || n1c == 0 || (method != 0 && n2c == 0)) return 0;
+  if (method == 0 || method == 1) {
+    /* flow: current left -> previous left -> back; stereo: current left -> current right -> back (matcher.cpp:1045-1084) */
+    const int32_t* mo = method == 0 ? m1p : m2c;
+    const int no = method == 0 ? n1p : n2c;
+    binlist ko = make_bins(mo, no, p, ub, vb), k1c = make_bins(m1c, n1c, p, ub, vb);
     uint8_t* M = (uint8_t*)calloc((size_t)dims_c[0] * dims_c[1], 1);
     for (int i1c = 0; i1c < n1c; i1c++) {
       const int u1c = m1c[12 * i1c], v1c = m1c[12 * i1c + 1];
-      int ubin = (int)floorf((float)u1c / bs), vbin = (int)floorf((float)v1c / bs);
-      if (ubin > ub - 1) ubin = ub - 1;
-      if (vbin > vb - 1) vbin = vb - 1;
-      const int stat = vbin * ub + ubin;
-      const int i1p = find_match(m1c, i1c, m1p, &k1p, ub, vb, stat, 0, 1, use_prior, ranges, p);
-      const int back = find_match(m1p, i1p, m1c, &k1c, ub, vb, stat, 1, 1, use_prior, ranges, p);
+      const int stat = stat_bin_of(p, u1c, v1c, ub, vb);
+      const int flow = method == 0;
+      const int io = find_match(m1c, i1c, mo, &ko, ub, vb, stat, 0, flow, use_prior, ranges, p, -1, -1, &cnt);
+      const int back = find_match(mo, io, m1c, &k1c, ub, vb, stat, 1, flow, use_prior, ranges, p, -1, -1, &cnt);
       if (back != i1c) continue;
+      if (method == 1 && !(u1c >= mo[12 * io])) continue;       /* positive disparity, tested before the pixel rule */
       uint8_t* taken = M + (size_t)v1c * dims_c[0] + u1c;
       if (*taken) continue;
       *taken = 1;
       if (count < cap) {
-        vo_match m = {(float)m1p[12 * i1p], (float)m1p[12 * i1p + 1], i1p, -1, -1, -1, (float)u1c, (float)v1c, i1c, -1, -1, -1};
-        out[count] = m;
+        const vo_match f = {(float)mo[12 * io], (float)mo[12 * io + 1], io, -1, -1, -1, (float)u1c, (float)v1c, i1c, -1, -1, -1};
+        const vo_match s = {-1, -1, -1, -1, -1, -1, (float)u1c, (float)v1c, i1c, (float)mo[12 * io], (float)mo[12 * io + 1], io};
+        out[count] = method == 0 ? f : s;
       }
       count++;
     }
-    free(M); free(k1p.start); free(k1p.idx); free(k1c.start); free(k1c.idx);
-  } else if (method == 2) {
+    free(M); free(ko.start); free(ko.idx); free(k1c.start); free(k1c.idx);
+  } else {
     binlist k1p = make_bins(m1p, n1p, p, ub, vb), k2p = make_bins(m2p, n2p, p, ub, vb);
     binlist k1c = make_bins(m1c, n1c, p, ub, vb), k2c = make_bins(m2c, n2c, p, ub, vb);
     for (int i1p = 0; i1p < n1p; i1p++) {
       const int u1p = m1p[12 * i1p], v1p = m1p[12 * i1p + 1];
-      int ubin = (int)floorf((float)u1p / bs), vbin = (int)floorf((float)v1p / bs);
-      if (ubin > ub - 1) ubin = ub - 1;
-      if (vbin > vb - 1) vbin = vb - 1;
-      const int stat = vbin * ub + ubin;
-      const int i2p = find_match(m1p, i1p, m2p, &k2p, ub, vb, stat, 0, 0, use_prior, ranges, p);
-      const int i2c = find_match(m2p, i2p, m2c, &k2c, ub, vb, stat, 1, 1, use_prior, ranges, p);
-      const int i1c = find_match(m2c, i2c, m1c, &k1c, ub, vb, stat, 2, 0, use_prior, ranges, p);
-      const int back = find_match(m1c, i1c, m1p, &k1p, ub, vb, stat, 3, 1, use_prior, ranges, p);
+      const int stat = stat_bin_of(p, u1p, v1p, ub, vb);
+      const int i2p = find_match(m1p, i1p, m2p, &k2p, ub, vb, stat, 0, 0, use_prior, ranges, p, -1, -1, &cnt);
+      double up = -1, vp = -1, u1pd = -1, v1pd = -1;
+      if (tr_delta) {
+        /* the previous stereo match triangulated, moved by Tr_delta, projected into the current right image */
+        const double* t = tr_delta;
+        u1pd = u1p; v1pd = v1p;
+        double d = u1pd - (double)m2p[12 * i2p];
+        if (d < 1) d = 1;
+        const double x1p = (u1pd - p->cu) * p->base / d, y1p = (v1pd - p->cv) * p->base / d, z1p = p->f * p->base / d;
+        const double x2c = t[0] * x1p + t[1] * y1p + t[2] * z1p + t[3] - p->base;
+        const double y2c = t[4] * x1p + t[5] * y1p + t[6] * z1p + t[7];
+        const double z2c = t[8] * x1p + t[9] * y1p + t[10] * z1p + t[11];
+        up = p->f * x2c / z2c + p->cu;
+        vp = p->f * y2c / z2c + p->cv;
+      }
+      const int i2c = find_match(m2p, i2p, m2c, &k2c, ub, vb, stat, 1, 1, use_prior, ranges, p, up, vp, &cnt);
+      const int i1c = find_match(m2c, i2c, m1c, &k1c, ub, vb, stat, 2, 0, use_prior, ranges, p, -1, -1, &cnt);
+      const int back = find_match(m1c, i1c, m1p, &k1p, ub, vb, stat, 3, 1, use_prior, ranges, p, u1pd, v1pd, &cnt);
       if (back != i1p) continue;
       const int u2p = m2p[12 * i2p], v2p = m2p[12 * i2p + 1], u2c = m2c[12 * i2c], v2c = m2c[12 * i2c + 1];
       const int u1c = m1c[12 * i1c], v1c = m1c[12 * i1c + 1];
@@ -348,13 +390,12 @@ int vo_matching(int method, const int32_t* m1p, int n1p, const int32_t* m2p, int
     }
     free(k1p.start); free(k1p.idx); free(k2p.start); free(k2p.idx);
     free(k1c.start); free(k1c.idx); free(k2c.start); free(k2c.idx);
-  } else {
-    return -1;
   }
+  if (counts2) { counts2[0] = cnt.scanned; counts2[1] = cnt.candidates; }
   return count;
 }
 
-/* matcher.cpp:734-868.  Only the first 2 (flow) or 4 (quad) stage entries of every range are defined. */
+/* matcher.cpp:734-868.  Only the first 2 (flow, stereo) or 4 (quad) stage entries of every range are defined. */
 int vo_prior_statistics(const vo_match* pm, int n, int method, const int32_t dims_c[3], const vo_params* p, vo_range* ranges) {
   const float bs = (float)p->match_binsize;
   const int ub = (int)ceilf((float)dims_c[0] / bs), vb = (int)ceilf((float)dims_c[1] / bs);
@@ -368,6 +409,9 @@ int vo_prior_statistics(const vo_match* pm, int n, int method, const int32_t dim
     float d[8] = {0, 0, 0, 0, 0, 0, 0, 0}, ru, rv;
     if (method == 0) {
       d[0] = m->u1p - m->u1c; d[1] = m->v1p - m->v1c; d[2] = m->u1c - m->u1p; d[3] = m->v1c - m->v1p;
+      ru = m->u1c; rv = m->v1c;
+    } else if (method == 1) {
+      d[0] = m->u2c - m->u1c; d[2] = m->u1c - m->u2c;
       ru = m->u1c; rv = m->v1c;
     } else {
       d[0] = m->u2p - m->u1p; d[2] = m->u2c - m->u2p; d[3] = m->v2c - m->v2p; d[4] = m->u1c - m->u2c;
@@ -417,17 +461,113 @@ static void relocate(const uint8_t* du1, const uint8_t* dv1, const uint8_t* du2,
   *v2 += (float)(best / 5) - 2.0f;
 }
 
-/* Matcher::refinement with refinement == 1, matcher.cpp:1498-1585 (methods 0 and 2) */
+/* Matcher::refinement with refinement == 1, matcher.cpp:1498-1585.  The reference descriptor is always the one at
+ * (u1c, v1c); the relocated points are (u1p, v1p) in the previous left image (flow, quad), (u2c, v2c) in the current
+ * right image (stereo, quad) and (u2p, v2p) in the previous right image (quad). */
 void vo_refine_pixel(vo_match* pm, int n, int method, const int32_t dims_p[3], const int32_t dims_c[3], const uint8_t* du1p,
                      const uint8_t* dv1p, const uint8_t* du2p, const uint8_t* dv2p, const uint8_t* du1c, const uint8_t* dv1c,
                      const uint8_t* du2c, const uint8_t* dv2c) {
   for (int k = 0; k < n; k++) {
     vo_match* m = pm + k;
-    relocate(du1c, dv1c, du1p, dv1p, dims_c, dims_p, m->u1c, m->v1c, &m->u1p, &m->v1p);
-    if (method == 2) {
-      relocate(du1c, dv1c, du2c, dv2c, dims_c, dims_c, m->u1c, m->v1c, &m->u2c, &m->v2c);
-      relocate(du1c, dv1c, du2p, dv2p, dims_c, dims_p, m->u1c, m->v1c, &m->u2p, &m->v2p);
+    if (method == 0 || method == 2) relocate(du1c, dv1c, du1p, dv1p, dims_c, dims_p, m->u1c, m->v1c, &m->u1p, &m->v1p);
+    if (method == 1 || method == 2) relocate(du1c, dv1c, du2c, dv2c, dims_c, dims_c, m->u1c, m->v1c, &m->u2c, &m->v2c);
+    if (method == 2) relocate(du1c, dv1c, du2p, dv2p, dims_c, dims_p, m->u1c, m->v1c, &m->u2p, &m->v2p);
+  }
+}
+
+/* Solves the 6x6 system M x = r in place (Gauss-Jordan elimination with partial pivoting, double precision).
+ * Returns 0 if a pivot vanishes. */
+static int solve6(double M[6][6], double r[6]) {
+  for (int c = 0; c < 6; c++) {
+    int piv = c;
+    for (int i = c + 1; i < 6; i++) if (fabs(M[i][c]) > fabs(M[piv][c])) piv = i;
+    if (fabs(M[piv][c]) < 1e-20) return 0;
+    for (int k = 0; k < 6; k++) { const double t = M[c][k]; M[c][k] = M[piv][k]; M[piv][k] = t; }
+    { const double t = r[c]; r[c] = r[piv]; r[piv] = t; }
+    const double d = M[c][c];
+    for (int k = 0; k < 6; k++) M[c][k] /= d;
+    r[c] /= d;
+    for (int i = 0; i < 6; i++) {
+      if (i == c) continue;
+      const double f = M[i][c];
+      for (int k = 0; k < 6; k++) M[i][k] -= f * M[c][k];
+      r[i] -= f * r[c];
     }
+  }
+  return 1;
+}
+
+static double min2(double a, double b) { return a < b ? a : b; }
+
+/* parabolicFitting, matcher.cpp:1379-1454: 16-byte descriptor costs on the 7x7 positions around (u2, v2), first
+ * minimum, a minimum on the border drops the match, least-squares paraboloid c = b0 j^2 + b1 i^2 + b2 i j + b3 j + b4 i
+ * + b5 through the 3x3 costs around it (normal equations solved per match, as the reference's Matrix::solve does),
+ * then the float offsets and their rejections.  *margin receives the smallest distance of a float decision of this fit
+ * to its threshold (1 - |ddu|, 1 - |ddv|, |divisor|, |b2|; +inf if no float decision was taken).  Returns 0 if the
+ * match is dropped. */
+static int parabolic(const uint8_t* du1, const uint8_t* dv1, const uint8_t* du2, const uint8_t* dv2, const int32_t d1[3],
+                     const int32_t d2[3], float u1, float v1, float* u2, float* v2, double* margin) {
+  *margin = INFINITY;
+  if (*u2 - 3 < MARGIN || *u2 + 3 > d2[0] - 1 - MARGIN || *v2 - 3 < MARGIN || *v2 + 3 > d2[1] - 1 - MARGIN) return 0;
+  uint8_t ref[16], cand[16];
+  vo_small_descriptor(du1, dv1, d1[2], (int)u1, (int)v1, ref);
+  int cost[49];
+  for (int dv = 0; dv < 7; dv++)
+    for (int du = 0; du < 7; du++) {
+      vo_small_descriptor(du2, dv2, d2[2], (int)*u2 + du - 3, (int)*v2 + dv - 3, cand);
+      cost[dv * 7 + du] = vo_sad(ref, cand, 16);
+    }
+  int min_ind = 0;
+  for (int i = 1; i < 49; i++) if (cost[i] < cost[min_ind]) min_ind = i;
+  const int du = min_ind % 7, dv = min_ind / 7;
+  if (du == 0 || du == 6 || dv == 0 || dv == 6) return 0;
+  double AtA[6][6] = {{0}}, b[6] = {0, 0, 0, 0, 0, 0};
+  for (int i = -1; i <= 1; i++)
+    for (int j = -1; j <= 1; j++) {
+      const double row[6] = {j * j, i * i, i * j, j, i, 1};
+      const double c = cost[(dv + i) * 7 + (du + j)];
+      for (int r = 0; r < 6; r++) {
+        for (int q = 0; q < 6; q++) AtA[r][q] += row[r] * row[q];
+        b[r] += row[r] * c;
+      }
+    }
+  if (!solve6(AtA, b)) return 0;
+  const float divisor = (float)(b[2] * b[2] - 4.0 * b[0] * b[1]);
+  *margin = min2(fabs(divisor), fabs(b[2]));
+  if (fabsf(divisor) < 1e-8 || fabs(b[2]) < 1e-8) return 0;
+  const float ddv = (float)((2.0 * b[0] * b[4] - b[2] * b[3]) / divisor);
+  const float ddu = (float)(-(b[4] + 2.0 * b[1] * ddv) / b[2]);
+  *margin = min2(*margin, min2(fabs(1.0 - fabsf(ddu)), fabs(1.0 - fabsf(ddv))));
+  if (fabsf(ddu) >= 1.0f || fabsf(ddv) >= 1.0f) return 0;
+  *u2 += (float)du - 3.0 + ddu;
+  *v2 += (float)dv - 3.0 + ddv;
+  return 1;
+}
+
+/* Matcher::refinement with refinement == 2, matcher.cpp:1498-1585: the same hops as vo_refine_pixel with
+ * parabolicFitting; the first fit that fails drops the match (keep[k] = 0, the list itself is not compacted).
+ * margin[k] (optional): the smallest decision margin over the fits run for match k. */
+void vo_refine_subpixel(vo_match* pm, int n, int method, const int32_t dims_p[3], const int32_t dims_c[3], const uint8_t* du1p,
+                        const uint8_t* dv1p, const uint8_t* du2p, const uint8_t* dv2p, const uint8_t* du1c, const uint8_t* dv1c,
+                        const uint8_t* du2c, const uint8_t* dv2c, uint8_t* keep, double* margin) {
+  for (int k = 0; k < n; k++) {
+    vo_match* m = pm + k;
+    double mg = INFINITY, g;
+    int ok = 1;
+    if (method == 0 || method == 2) {
+      ok = parabolic(du1c, dv1c, du1p, dv1p, dims_c, dims_p, m->u1c, m->v1c, &m->u1p, &m->v1p, &g);
+      mg = min2(mg, g);
+    }
+    if (ok && (method == 1 || method == 2)) {
+      ok = parabolic(du1c, dv1c, du2c, dv2c, dims_c, dims_c, m->u1c, m->v1c, &m->u2c, &m->v2c, &g);
+      mg = min2(mg, g);
+    }
+    if (ok && method == 2) {
+      ok = parabolic(du1c, dv1c, du2p, dv2p, dims_c, dims_p, m->u1c, m->v1c, &m->u2p, &m->v2p, &g);
+      mg = min2(mg, g);
+    }
+    keep[k] = (uint8_t)ok;
+    if (margin) margin[k] = mg;
   }
 }
 

@@ -42,14 +42,20 @@ int  vo_sad(const uint8_t* a, const uint8_t* b, int nbytes);
 int  vo_compute_features(const uint8_t* Ipad, const int32_t dims[3], const vo_params* p,
                          uint8_t* du, uint8_t* dv, uint8_t* du_full, uint8_t* dv_full,
                          int32_t* rec1, int cap1, int32_t* n1, int32_t* rec2, int cap2, int32_t* n2);
+/* method 0 flow, 1 stereo, 2 quad; tr_delta (quad only, may be NULL): rows 0..2 of Tr_delta, 12 doubles, with
+ * p->f, cu, cv, base.  counts2 (may be NULL): entries of the scanned bins and window candidates over all hops. */
 int  vo_matching(int method, const int32_t* m1p, int n1p, const int32_t* m2p, int n2p,
                  const int32_t* m1c, int n1c, const int32_t* m2c, int n2c,
                  const int32_t dims_c[3], const vo_params* p, int use_prior, const vo_range* ranges,
-                 vo_match* out, int cap);
+                 const double* tr_delta, vo_match* out, int cap, int64_t* counts2);
 int  vo_prior_statistics(const vo_match* pm, int n, int method, const int32_t dims_c[3], const vo_params* p, vo_range* ranges);
 void vo_refine_pixel(vo_match* pm, int n, int method, const int32_t dims_p[3], const int32_t dims_c[3],
                      const uint8_t* du1p, const uint8_t* dv1p, const uint8_t* du2p, const uint8_t* dv2p,
                      const uint8_t* du1c, const uint8_t* dv1c, const uint8_t* du2c, const uint8_t* dv2c);
+void vo_refine_subpixel(vo_match* pm, int n, int method, const int32_t dims_p[3], const int32_t dims_c[3],
+                        const uint8_t* du1p, const uint8_t* dv1p, const uint8_t* du2p, const uint8_t* dv2p,
+                        const uint8_t* du1c, const uint8_t* dv1c, const uint8_t* du2c, const uint8_t* dv2c,
+                        uint8_t* keep, double* margin);
 /* RANSAC pieces (FP64).  Compiled with -ffp-contract=off: bit-comparable to oracle/_ref/libvisoref_nofma.so */
 void vo_svd(double* a, int m, int n, double* w, double* v);
 int  vo_normalize(vo_match* pm, int n, double* Tp9, double* Tc9);

@@ -207,3 +207,12 @@ def test_stereo_odometry_from_matches(reference):
         Tr = reference.value('motion%d' % step)
         assert np.abs(Tr - Th).max() < 1e-9
         assert abs(Th[2, 3] + 0.8) < 0.05
+
+
+def test_prior_statistics_before_any_push():
+    """Matcher::computePriorStatistics on a matcher that has seen no image has no image size to lay its bin grid over:
+    it gives no ranges (it used to index a grid of zero bins)."""
+    m = np.zeros(3, H.P_MATCH)
+    m['u1p'], m['v1p'], m['u1c'], m['v1c'], m['u2c'], m['v2c'] = [10, 20, 30], 5, [12, 21, 33], 6, [4, 9, 20], 6
+    for method in (0, 1, 2):
+        assert H.Matcher(V.Params()).prior(m, method).shape == (0, 16)

@@ -1,11 +1,14 @@
 """CPU tests: pin the plain-C restatement (oracle/viso_oracle.c) against the outputs of the unmodified reference on the
 same seeded inputs (SURVEY.md 8c: the reference holds no golden vectors for this path; its outputs are stored under
-tests/golden/reference, see oracle/refgold.py).  Integer stages bit-exact, FP64 stages to the stated tolerance.  Needs no GPU."""
+tests/golden/reference, see oracle/refgold.py).  Integer stages bit-exact, FP64 stages to the stated tolerance.  Needs no GPU.
+Stereo matching, motion-predicted quad matching and sub-pixel refinement are pinned against the results stored for
+tests/test_gpu_host_layer.py (same inputs, the whole Matcher chain)."""
 import numpy as np
 import pytest
 
 import synth
 import pyref
+import refgold
 import pyoracle as O
 import visocu_py as V
 import host_py as H
@@ -101,6 +104,86 @@ def test_quad_matching(reference):
     planes = dict(du1p=f[0]['du'], dv1p=f[0]['dv'], du2p=f[1]['du'], dv2p=f[1]['dv'], du1c=f[2]['du'], dv1c=f[2]['dv'],
                   du2c=f[3]['du'], dv2c=f[3]['dv'])
     reference.same('refined2', O.refine_pixel(got2, 2, f[0]['dims'], planes))
+
+
+# ------------------------------------------------------------------------------------------------------------------------
+# Stereo matching, motion-predicted quad matching and sub-pixel refinement have no counterpart in the reference shim: the
+# oracle's restatement is pinned against the reference results stored for the host-layer GPU tests instead, on the same
+# inputs.  The chain is the Matcher's: pass 0, removeOutliers (the host layer's, pinned by tests/test_host_cpu.py), prior
+# statistics, pass 1 with them, refinement, removeOutliers.
+def _host_layer(case):
+    return refgold.Reference('test_gpu_host_layer', case)
+
+
+def oracle_chain(method, imgs, kw, tr_delta=None):
+    """(survivors of pass 0, survivors of pass 1) of Matcher::matchFeatures(method) on imgs = (1p, 2p, 1c, 2c), None for
+    an image the method does not use; kw: Matcher parameters (match_radius as given to the constructor)."""
+    op = O.Params(**kw)
+    eff = op.effective()
+    f = [None if i is None else O.compute_features(i, op) for i in imgs]
+    dims = next(x for x in f if x is not None)['dims']
+    recs = lambda r: [None if x is None else x[r] for x in f]
+    hm = H.Matcher(V.Params(**kw))
+    kept1 = hm.remove_outliers(O.matching(method, *recs('rec1'), dims, eff, tr_delta=tr_delta), method)
+    ranges = O.prior_statistics(kept1, method, dims, eff)
+    raw2 = O.matching(method, *recs('rec2'), dims, eff, ranges=ranges, tr_delta=tr_delta)
+    planes = {}
+    for name, x in zip(('1p', '2p', '1c', '2c'), f):
+        if x is not None:
+            planes['du' + name] = x['du_full'] if op.half_resolution else x['du']
+            planes['dv' + name] = x['dv_full'] if op.half_resolution else x['dv']
+    if op.refinement == 2:
+        raw2, keep, _ = O.refine_subpixel(raw2, method, dims, planes)
+        raw2 = raw2[keep]
+    elif op.refinement == 1:
+        raw2 = O.refine_pixel(raw2, method, dims, planes)
+    return kept1, hm.remove_outliers(raw2, method)
+
+
+def test_stereo_matching_priors_refinement():
+    """Method 1 (matcher.cpp:1045-1084): matching, its prior statistics and pixel refinement of (u2c, v2c), bit-exact
+    against both modes of test_matcher_stereo_method1."""
+    lp, rpv, lc, rc = synth.blob_quad(1244, 376, seed=47)
+    ref = _host_layer('test_matcher_stereo_method1')
+    for mode, kw in (('fullres', dict(half_resolution=0)), ('defaults', dict())):
+        kept1, kept2 = oracle_chain(1, (None, None, lc, rc), kw)
+        assert len(kept2) > 1000 and np.all(kept2['u1c'] >= kept2['u2c'])
+        ref.same(mode + '_matches1', kept1)
+        ref.same(mode + '_matches2', kept2)
+
+
+def test_quad_matching_with_motion_prediction():
+    """Tr_delta-predicted quad matching (matcher.cpp:1112-1138, cost SAD + 4 * distance in double precision), bit-exact
+    against test_quad_matching_with_motion_prediction (reference built with -ffp-contract=off)."""
+    lp, rpv, lc, rc = synth.blob_quad(1242, 376, seed=53, shift=(3, 1), disparity=12)
+    Tr = np.eye(4); Tr[0, 3] = 0.02; Tr[2, 3] = -0.3; Tr[0, 2] = 0.01; Tr[2, 0] = -0.01
+    kw = dict(nms_n=2, half_resolution=0, f=645.2, cu=635.9, cv=194.1, base=0.54)
+    kept1, kept2 = oracle_chain(2, (lp, rpv, lc, rc), kw, tr_delta=Tr)
+    assert len(kept2) > 500
+    _host_layer('test_quad_matching_with_motion_prediction').same('matches2', kept2)
+    # the prediction changes the result: without it the list differs
+    assert kept2.tobytes() != oracle_chain(2, (lp, rpv, lc, rc), kw)[1].tobytes()
+
+
+def test_subpixel_refinement():
+    """parabolicFitting (matcher.cpp:1379-1454) with a least-squares solve per match: integer fields and the kept set
+    bit-exact against test_matcher_subpixel_refinement, the stored coordinate samples within 1e-4 pixel."""
+    ref = _host_layer('test_matcher_subpixel_refinement')
+    sample = lambda n: np.sort(np.random.default_rng(0).choice(n, min(n, 512), replace=False))
+    a, b = synth.blob_pair(1242, 376, seed=49)
+    _, got = oracle_chain(0, (a, None, b, None), dict(nms_n=4, refinement=2, half_resolution=0))
+    assert len(got) > 1000
+    ref.same('flow_integer', np.stack([got[f] for f in ('i1p', 'i1c', 'u1c', 'v1c')], 1))
+    rows = sample(len(got))
+    for f in ('u1p', 'v1p'):
+        assert np.abs(got[f][rows] - ref.value('flow_' + f)).max() < 1e-4
+    lp, rpv, lc, rc = synth.blob_quad(1242, 376, seed=51)
+    _, got = oracle_chain(2, (lp, rpv, lc, rc), dict(nms_n=2, refinement=2, half_resolution=0))
+    assert len(got) > 500
+    ref.same('quad_integer', np.stack([got[f] for f in ('i1p', 'i2p', 'i1c', 'i2c', 'u1c', 'v1c')], 1))
+    rows = sample(len(got))
+    for f in ('u1p', 'v1p', 'u2p', 'v2p', 'u2c', 'v2c'):
+        assert np.abs(got[f][rows] - ref.value('quad_' + f)).max() < 1e-4
 
 
 def _unit(F):
