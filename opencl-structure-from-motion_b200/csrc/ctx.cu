@@ -291,6 +291,12 @@ extern "C" int visocu_configure(visocu_ctx* ctx, const visocu_params* p, int32_t
   free_pool(ctx);
   ctx->param = *p;
   ctx->ro_bound[0] = ctx->ro_bound[1] = -1;
+  // outlier kernel shape (experiments and tests): VISOCU_RO_THREADS=256|512|1024 threads per list, VISOCU_RO_WARP=0 one
+  // thread per top-level merge.  Read per configure, so that one process can run every variant.
+  ctx->ro_threads = 0;
+  if (const char* e = getenv("VISOCU_RO_THREADS")) { const int t = atoi(e); if (t == 256 || t == 512 || t == 1024) ctx->ro_threads = t; }
+  ctx->ro_warp = 1;
+  if (const char* e = getenv("VISOCU_RO_WARP")) if (e[0] == '0') ctx->ro_warp = 0;
   Geometry& g = ctx->g;
   g.w = width; g.h = height; g.bpl = viso_bpl(width);
   g.half = p->half_resolution ? 1 : 0;

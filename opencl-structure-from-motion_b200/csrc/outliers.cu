@@ -686,9 +686,8 @@ int visocu_launch_remove_outliers(visocu_ctx* ctx, const RoJob* jobs_dev, int n_
     }
   }
   // one or two lists (a stand-alone Matcher): the shortest chain; batches: the smaller footprint
-  static const int forced = [] { const char* e = getenv("VISOCU_RO_THREADS"); return e ? atoi(e) : 0; }();
-  const int threads = forced ? forced : (n_jobs <= 2 ? 1024 : 512);
-  static const int warp = [] { const char* e = getenv("VISOCU_RO_WARP"); return (e && e[0] == '0') ? 0 : 1; }();
+  const int threads = ctx->ro_threads ? ctx->ro_threads : (n_jobs <= 2 ? 1024 : 512);
+  const int warp = ctx->ro_warp;
   const float ft = (float)ctx->param.outlier_flow_tolerance, dt = (float)ctx->param.outlier_disp_tolerance;
   if (threads >= 1024) k_remove_outliers<1024><<<n_jobs, 1024, smem, stream>>>(jobs_dev, method, ft, dt, (int)smem, warp);
   else if (threads >= 512) k_remove_outliers<512><<<n_jobs, 512, smem, stream>>>(jobs_dev, method, ft, dt, (int)smem, warp);
@@ -888,7 +887,11 @@ bool ro_resolve_duplicates(const uint32_t* keys, int n_records, uint8_t* rep) {
     if (right < len - 2) stack.push_back(std::make_pair(lo + right + 1, len - right - 1));    // taken second
     if (left > 1) stack.push_back(std::make_pair(lo, left));                                   // taken first
   }
-  for (int i = 0; i < n_records; i++) rep[i] = 0;
+  // A record without a key (position outside 0..65535, e.g. a negative coordinate) stays a vertex, so that the kernel's
+  // range check sees it and hands the list to the host, which triangulates any coordinates.  Left out, it would collect
+  // no votes and be dropped with status 0.  Records the sub-pixel refinement dropped have no key either, but they never
+  // reach the kernel's list.
+  for (int i = 0; i < n_records; i++) rep[i] = keys[i] == 0xFFFFFFFFu ? 1 : 0;
   for (int i = 0; i < n; i++)
     if (i == 0 || (el[i] >> 32) != (el[i - 1] >> 32)) rep[rec[(size_t)(el[i] & 0xFFFFFFFFu)]] = 1;
   return true;

@@ -89,6 +89,8 @@ struct visocu_ctx {
   std::vector<visocu_quad> fused_jobs;
   int ro_bound_seen[2] = {0, 0};
   int ro_bound[2] = {-1, -1};        // longest match list seen per pass (shared-memory size of the outlier kernel in lazy mode)
+  int ro_threads = 0;                // outlier kernel: threads per list, 0 = by batch size (VISOCU_RO_THREADS, read by visocu_configure)
+  int ro_warp = 1;                   // outlier kernel: a warp per top-level merge; 0 = one thread (VISOCU_RO_WARP)
   const uint8_t** src_table = nullptr; const uint8_t** src_table_pin = nullptr;
   cudaEvent_t ev_push = nullptr;
   visocu_graph g_push, g_match;

@@ -75,19 +75,31 @@ def test_device_outlier_removal_declines_what_it_cannot_do(reference, rctx):
         reference.same('collinear', got[3])
 
 
-def test_device_nodes_of_large_triangulations(rctx):
+def test_device_nodes_of_large_triangulations(rctx, monkeypatch):
     """visocu_delaunay_subtrees through host/delaunay.cpp: a triangulation of more points than the device kernel holds is cut
-    into nodes that the device builds; the edge list (hence every vote of removeOutliers) equals the all-host one."""
+    into nodes that the device builds; the edge list (hence every vote of removeOutliers) equals the all-host one.  The
+    nodes are built under every kernel shape (VISOCU_RO_THREADS x VISOCU_RO_WARP, read when the context is configured),
+    then under the default one, which the context keeps for the tests after this one."""
     import host_py as H
     rng = np.random.default_rng(41)
+    norm = lambda e: np.unique(np.concatenate([np.sort(e[:, :2], 1), e[:, 2:]], 1), axis=0)
+    sets = []
     for n, w, h, grid in ((6500, 1241, 376, 1), (20000, 3840, 2160, 2), (87000, 3840, 2160, 2), (60000, 3840, 2160, 1), (9000, 8000, 200, 1)):
         cells = rng.choice((w // grid) * (h // grid), size=n, replace=False)
         x = ((cells % (w // grid)) * grid + 2).astype(np.int32); y = ((cells // (w // grid)) * grid + 3).astype(np.int32)
         e_host, nodes0 = H.delaunay_edges(x, y)
-        e_dev, nodes = H.delaunay_edges(x, y, rctx)
-        assert nodes0 == 0 and nodes >= 2, (n, nodes)
-        norm = lambda e: np.unique(np.concatenate([np.sort(e[:, :2], 1), e[:, 2:]], 1), axis=0)
-        assert len(e_dev) == len(e_host) and np.array_equal(norm(e_host), norm(e_dev)), (n, w, h, grid)
+        assert nodes0 == 0
+        sets.append((x, y, norm(e_host), (n, w, h, grid)))
+    for variant in [(t, wm) for t in (1024, 512, 256) for wm in ('1', '0')] + [None]:
+        if variant is None:
+            monkeypatch.delenv('VISOCU_RO_THREADS', raising=False); monkeypatch.delenv('VISOCU_RO_WARP', raising=False)
+        else:
+            monkeypatch.setenv('VISOCU_RO_THREADS', str(variant[0])); monkeypatch.setenv('VISOCU_RO_WARP', variant[1])
+        rctx.configure(V.Params(half_resolution=0), 1241, 376, 4)
+        for x, y, want, what in sets:
+            e_dev, nodes = H.delaunay_edges(x, y, rctx)
+            assert nodes >= 2, (variant, what, nodes)
+            assert len(e_dev) == len(want) and np.array_equal(want, norm(e_dev)), (variant, what)
 
 
 def test_large_lists_vote_with_device_nodes(reference):
