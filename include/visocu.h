@@ -137,13 +137,38 @@ int  visocu_get_rectify_map(visocu_ctx* ctx, int32_t cam, int32_t* out, size_t c
  * out_on_device = 0: out[k] are host memory; 1: device memory of the context's GPU.  The call runs on the current lane,
  * behind the last push of every lane, and waits for its work.  VISOCU_EINVAL for bad parameters, a frame index out of
  * range, a null pointer or n_pairs < 0; VISOCU_ESTATE for a frame never pushed or an unconfigured context; both before
- * anything is enqueued or written.  Per group of at most 128 pairs: 4 launches with 4 paths, 6 with 8, and scratch of
- * w h (16 + 2 D) bytes per pair (+ 2 w h for host outputs). */
-typedef struct { int32_t max_disp, paths, p1, p2, uniqueness, lr_max_diff, subpixel; } visocu_sgm_params;
+ * anything is enqueued or written.  Per group of at most 128 pairs: 4 launches with 4 paths, 6 with 8, plus those of the
+ * post-filters below, and scratch of w h (16 + 2 D) bytes per pair (+ 2 w h for host outputs); the filters use the S part
+ * of it, which is dead once the maps are selected.
+ *
+ * Post-filters of each finished map (after uniqueness, left-right check and sub-pixel offset), in this order:
+ *   1. median = 1, masked 3x3 median, out of place (it reads the unfiltered map): a valid pixel (v >= 0) takes the lower
+ *      median of the valid values of its 3x3 window clipped to the image, itself included (sorted, the n valid values'
+ *      entry (n - 1) / 2); an invalid pixel (-1) stays -1.
+ *   2. speckle_size > 0, speckle removal: two valid 4-neighbours p, q are connected when |v_p - v_q| <= 16 speckle_range
+ *      (whole pixels, the map is in 1/16 pixel); every pixel of a connected component of at most speckle_size pixels
+ *      becomes -1.  Invalid pixels connect nothing.
+ * Valid: median in {0, 1}, speckle_size >= 0 (0 = off), 0 <= speckle_range <= D.  With all three 0 the maps are those of
+ * SGM alone.  Launches per group added by the filters: 2 for the median alone (k_disp_median3, k_speckle_apply), 4 for
+ * speckle removal alone (k_speckle_local, k_speckle_merge, k_speckle_count, k_speckle_apply), 5 for both. */
+typedef struct {
+  int32_t max_disp, paths, p1, p2, uniqueness, lr_max_diff, subpixel;
+  int32_t median, speckle_size, speckle_range;      /* post-filters; zero-initialise them for SGM alone */
+} visocu_sgm_params;
 int  visocu_disparity(visocu_ctx* ctx, int32_t n_pairs, const int32_t* left, const int32_t* right,
                       const visocu_sgm_params* p, int16_t* const* out, int32_t out_on_device);
 /* VISOCU_OK if p is non-null and inside the valid ranges above, else VISOCU_EINVAL (for callers that store parameters) */
 int  visocu_sgm_check(const visocu_sgm_params* p);
+/* The post-filters of visocu_disparity, in place, on n_maps maps of w x h int16 (row stride w, 1/16 pixel, -1 = invalid),
+ * whatever the context's frame geometry: the same kernels visocu_disparity runs, for callers that re-filter maps with
+ * other settings.  on_device = 0: maps[k] are host memory; 1: device memory of the context's GPU.  Valid: w, h >= 1,
+ * w h <= VISOCU_DISP_FILTER_MAX_PIXELS, median in {0, 1}, speckle_size >= 0, 0 <= speckle_range <= 256.  The call runs on
+ * the current lane and waits for its work; it needs no configured context.  VISOCU_EINVAL for a bad argument, a null
+ * pointer or n_maps < 0, before anything is enqueued or written.  Per group of at most 128 maps: the launches above and
+ * scratch of 10 w h bytes per map (+ 2 w h for host maps). */
+#define VISOCU_DISP_FILTER_MAX_PIXELS (1 << 24)
+int  visocu_disparity_filter(visocu_ctx* ctx, int32_t n_maps, int16_t* const* maps, int32_t w, int32_t h, int32_t on_device,
+                             int32_t median, int32_t speckle_size, int32_t speckle_range);
 
 /* ---- filter:: functions (viso/filter.h:78-94), host buffers in and out, same argument order ---- */
 int  visocu_sobel5x5(visocu_ctx* ctx, const uint8_t* in, uint8_t* out_v, uint8_t* out_h, int32_t w, int32_t h);

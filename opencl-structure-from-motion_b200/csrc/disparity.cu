@@ -4,7 +4,8 @@
 // pass over S.  oracle/sgm_oracle.c states the same algorithm in plain C; the device is bit-identical to it.
 //
 // Launches per group of at most VISO_MAX_BATCH pairs: k_census, k_sgm_rows, k_sgm_cols, [k_sgm_diag, k_sgm_antidiag],
-// k_sgm_select.  Scratch per pair: census 2 w h 8 B, S w h D 2 B (and w h 2 B of output for host destinations).
+// k_sgm_select, then the post-filters of csrc/disparity_filter.cu when they are on, in S, which is dead by then.
+// Scratch per pair: census 2 w h 8 B, S w h D 2 B (and w h 2 B of output for host destinations).
 #include "visocu_internal.cuh"
 
 namespace {
@@ -210,7 +211,7 @@ int launch_group(visocu_ctx* ctx, const PairList& pl, int nb, const visocu_sgm_p
   if (smem > 48 * 1024) CU_TRY(ctx, cudaFuncSetAttribute(k_sgm_select<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k_sgm_select<K><<<dim3(g.h, nb), 256, smem, st>>>(S, g, p, ol);
   CU_LAUNCH_CHECK(ctx);
-  return VISOCU_OK;
+  return visocu_disp_filter_group(ctx, nb, ol.p, g.w, g.h, p.median, p.speckle_size, p.speckle_range, S);
 }
 
 }  // namespace
@@ -220,7 +221,8 @@ extern "C" int visocu_sgm_check(const visocu_sgm_params* p) {
   const int D = p->max_disp;
   const bool ok = (D == 64 || D == 128 || D == 256) && (p->paths == 4 || p->paths == 8) && p->p1 >= 1 && p->p1 < p->p2 && p->p2 <= 150 &&
                   p->uniqueness >= 0 && p->uniqueness <= 100 && p->lr_max_diff >= -1 && p->lr_max_diff <= D &&
-                  (p->subpixel == 0 || p->subpixel == 1);
+                  (p->subpixel == 0 || p->subpixel == 1) && (p->median == 0 || p->median == 1) && p->speckle_size >= 0 &&
+                  p->speckle_range >= 0 && p->speckle_range <= D;
   return ok ? VISOCU_OK : VISOCU_EINVAL;
 }
 
@@ -231,7 +233,8 @@ extern "C" int visocu_disparity(visocu_ctx* ctx, int32_t n_pairs, const int32_t*
   const int D = p->max_disp;
   if (visocu_sgm_check(p) != VISOCU_OK)
     return visocu_set_error(ctx, VISOCU_EINVAL, "disparity parameters out of range (max_disp %d, paths %d, p1 %d, p2 %d, uniqueness %d, "
-                            "lr_max_diff %d, subpixel %d)", D, p->paths, p->p1, p->p2, p->uniqueness, p->lr_max_diff, p->subpixel);
+                            "lr_max_diff %d, subpixel %d, median %d, speckle_size %d, speckle_range %d)", D, p->paths, p->p1, p->p2,
+                            p->uniqueness, p->lr_max_diff, p->subpixel, p->median, p->speckle_size, p->speckle_range);
   if (n_pairs < 0) return visocu_set_error(ctx, VISOCU_EINVAL, "n_pairs %d < 0", n_pairs);
   if (out_on_device != 0 && out_on_device != 1) return visocu_set_error(ctx, VISOCU_EINVAL, "out_on_device must be 0 or 1");
   if (n_pairs > 0 && (!left || !right || !out)) return visocu_set_error(ctx, VISOCU_EINVAL, "null pair or output list");

@@ -149,6 +149,11 @@ void visocu_drop_graphs(visocu_ctx* ctx);
 void visocu_drop_lane_graphs(visocu_ctx* ctx);               // of the current lane
 int visocu_use_lane(visocu_ctx* ctx, int lane);                  // swap the lane's resources into the working fields
 int visocu_ensure_scratch(visocu_ctx* ctx, size_t bytes);
+// csrc/disparity_filter.cu: the post-filters of include/visocu.h on nb <= VISO_MAX_BATCH device maps of w x h, enqueued on
+// the current lane (nothing when median and speckle_size are 0); scratch of visocu_disp_filter_scratch(nb, w h) bytes
+size_t visocu_disp_filter_scratch(int n_maps, size_t plane);
+int visocu_disp_filter_group(visocu_ctx* ctx, int nb, int16_t* const* maps, int w, int h, int median, int speckle_size,
+                             int speckle_range, void* scratch);
 int visocu_ensure_pinned(visocu_ctx* ctx, size_t bytes);
 int visocu_run_or_replay(visocu_ctx* ctx, visocu_graph& g, uint64_t key, const std::function<int()>& enqueue);
 

@@ -70,12 +70,15 @@ class Camera(C.Structure):
 
 
 class SgmParams(C.Structure):
-    """visocu_sgm_params: semi-global matching settings of visocu_disparity (include/visocu.h)."""
-    _fields_ = [(n, C.c_int32) for n in ('max_disp', 'paths', 'p1', 'p2', 'uniqueness', 'lr_max_diff', 'subpixel')]
+    """visocu_sgm_params: semi-global matching settings of visocu_disparity (include/visocu.h), and its post-filters
+    (median, speckle_size, speckle_range), off by default."""
+    _fields_ = [(n, C.c_int32) for n in ('max_disp', 'paths', 'p1', 'p2', 'uniqueness', 'lr_max_diff', 'subpixel',
+                                         'median', 'speckle_size', 'speckle_range')]
 
     def __init__(self, **kw):
         super().__init__()
-        d = dict(max_disp=128, paths=8, p1=10, p2=120, uniqueness=95, lr_max_diff=1, subpixel=1)
+        d = dict(max_disp=128, paths=8, p1=10, p2=120, uniqueness=95, lr_max_diff=1, subpixel=1, median=0, speckle_size=0,
+                 speckle_range=0)
         d.update(kw)
         for k, v in d.items():
             setattr(self, k, int(v))
@@ -263,6 +266,28 @@ class Context:
         torch.cuda.current_stream(out.device).synchronize()     # the memory may still be in use by torch's stream
         self._disparity(left, right, params, [out[k].data_ptr() for k in range(len(left))], 1)
         return out
+
+    def disparity_filter(self, maps, median=0, speckle_size=0, speckle_range=0):
+        """visocu_disparity_filter in place: the post-filters of visocu_disparity on a list of (h, w) int16 numpy maps
+        (C-contiguous, all of one shape) or on an int16 CUDA tensor of shape (n, h, w).  Returns maps."""
+        if hasattr(maps, 'data_ptr'):
+            import torch
+            assert maps.dtype == torch.int16 and maps.dim() == 3 and maps.is_cuda and maps.is_contiguous()
+            n, h, w = maps.shape
+            torch.cuda.current_stream(maps.device).synchronize()    # the maps may still be written by torch's stream
+            ptrs, on_device = [maps[k].data_ptr() for k in range(n)], 1
+        else:
+            for m in maps:
+                if m.dtype != np.int16 or m.ndim != 2 or not m.flags.c_contiguous or not m.flags.writeable or \
+                        m.shape != maps[0].shape:
+                    raise ValueError('disparity_filter: maps must be writable C-contiguous (h, w) int16 arrays of one shape')
+            n = len(maps)
+            h, w = maps[0].shape if n else (1, 1)
+            ptrs, on_device = [m.ctypes.data for m in maps], 0
+        arr = (C.c_void_p * max(n, 1))(*ptrs)
+        self._ck(lib().visocu_disparity_filter(self.h, n, arr, int(w), int(h), on_device, int(median), int(speckle_size),
+                                               int(speckle_range)), 'disparity_filter')
+        return maps
 
     def tile_levels(self, n_launch=1):
         """(levels, pick): the fused filter + NMS kernel's tile configurations, largest first, as dicts (kx, ky, ntx, nty,
